@@ -27,7 +27,7 @@ Differences from the reference, all deliberate (DESIGN.md "Boundary"):
   of an earlier call) is read as the state those labels describe and the run
   resumes from it; the reference re-seeds such a map from label 0 only
   (VRG:44) and then dies with a ValueError at VRG:111 once its outer band list
-  runs empty (tests/test_oracle_golden.py::test_reference_dies_on_its_own_output);
+  runs empty;
 * an empty seed set or a seed without boundary raises ``ValueError`` (the
   reference dies with ``IndexError`` at VRG:88);
 * ``segmented`` rows come back in C order (the reference's row order is the

@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--intensity f64_dense]
     python bench.py --impl reference ...      # CPU arm: the oracle port on the host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's outputs as DIR/*.npy (dump_outputs)
 
 One "step" is one complete variational region growing run (level scan + init
 branch + every iteration to convergence) on the synthetic vessel-forest phantom
@@ -51,6 +52,8 @@ METRIC = "VRG Gvoxel-updates/s at 880x880x640, 1/2/4/8 B200; % of HBM roofline"
 CPU_SAMPLE_PLANES = 128
 ORACLE_MAX_VOXELS = 1.2e9  # whole-volume oracle parity up to here (C4: 1.07e9); larger volumes: one-GPU replica
 HALO = 2
+DUMP_SAMPLE = 1 << 21  # voxels whose labels --dump-outputs writes
+DUMP_SEED = 20240601
 
 
 def measured_peak():
@@ -313,6 +316,14 @@ class Ctx:
         self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
         return float(t.item())
 
+    def sum_f64(self, a):
+        """Element-wise sum of a float64 array over all ranks (the array itself when alone)."""
+        if self.dist is None:
+            return a
+        t = self.torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).cuda()
+        self.dist.all_reduce(t)
+        return t.cpu().numpy()
+
     def gather_i64(self, values):
         """All ranks' int64 vectors (same length), as a (world, n) array on every rank."""
         t = self.torch.tensor([int(v) - 2 ** 64 if int(v) >= 2 ** 63 else int(v) for v in values], dtype=self.torch.int64,
@@ -332,8 +343,33 @@ def trace_hash(trace):
     return hashlib.sha256(np.ascontiguousarray(trace, dtype=np.int64).tobytes()).hexdigest()[:16]
 
 
-def bench_volume(ctx, shape, seed, intensity, steps, warmup, want_e2e, want_parity, sample_clocks=False):
-    """Times the whole-volume run of `shape` over ctx.world z-slabs; returns the measurements of one JSON line."""
+def dump_outputs(ctx, eng, trace, shape, z0, z1, out_dir):
+    """Writes what the run left in `eng` as .npy files under out_dir (rank 0), at most about 25 MB whatever the volume:
+    labels_sample (float32) = the labels at labels_sample_index (float64 flat voxel indices, the same ones every run),
+    label_counts_per_plane (float64, Z x 5) = how many voxels of each plane carry label 0..4, and
+    trace (float64, rows of n_flips, n_in, n_out per iteration)."""
+    plane = shape[1] * shape[2]
+    nvox = shape[0] * plane
+    idx = np.unique(np.random.default_rng(DUMP_SEED).integers(0, nvox, size=min(nvox, DUMP_SAMPLE)))
+    lab = eng.labels()  # own planes [z0, z1)
+    mine = (idx >= z0 * plane) & (idx < z1 * plane)
+    sample = np.zeros(idx.size)
+    sample[mine] = lab.reshape(-1)[idx[mine] - z0 * plane]
+    counts = np.zeros((shape[0], 5))
+    for k in range(5):
+        counts[z0:z1, k] = (lab == k).sum(axis=(1, 2))
+    sample, counts = ctx.sum_f64(sample), ctx.sum_f64(counts)
+    if ctx.rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "labels_sample.npy"), sample.astype(np.float32))
+        np.save(os.path.join(out_dir, "labels_sample_index.npy"), idx.astype(np.float64))
+        np.save(os.path.join(out_dir, "label_counts_per_plane.npy"), counts)
+        np.save(os.path.join(out_dir, "trace.npy"), np.asarray(trace, dtype=np.float64))
+
+
+def bench_volume(ctx, shape, seed, intensity, steps, warmup, want_e2e, want_parity, sample_clocks=False, dump_dir=None):
+    """Times the whole-volume run of `shape` over ctx.world z-slabs; returns the measurements of one JSON line.
+    With `dump_dir`, the outputs of the last timed step are written there (dump_outputs)."""
     import torch
     from arterynetwork_b200 import _native as nat
     from arterynetwork_b200.distributed import DistributedVRG, GpuSlabEngine, slab_bounds
@@ -386,6 +422,8 @@ def bench_volume(ctx, shape, seed, intensity, steps, warmup, want_e2e, want_pari
         res = eng.poll()
         launches = res["kernel_launches"] - l0
         out["clocks"] = sampler.stop() if sampler else None
+        if dump_dir:
+            dump_outputs(ctx, eng, drv.trace() if drv is not None else eng.trace(), shape, z0, z1, dump_dir)
         # per-launch time of the sweep: one extra step with CUDA events around every sweep launch (plain stream launches);
         # the same step gives the phases of the tail kernel (device clock) and a host-side split of the step
         eng.profile(True)
@@ -550,7 +588,7 @@ def run_ours(args):
     shape = workload_shape(args, world)
     nvox = shape[0] * shape[1] * shape[2]
     prim = bench_volume(ctx, shape, args.seed, args.intensity, args.steps, args.warmup, want_e2e=True,
-                        want_parity=not args.no_parity, sample_clocks=True)
+                        want_parity=not args.no_parity, sample_clocks=True, dump_dir=args.dump_outputs)
     prim["steps"] = args.steps
     modes = None
     if world == 1 and not args.quick:
@@ -646,8 +684,14 @@ def main():
                          "named volume's planes, i.e. the volume grows with N (c5: 2048x2048x128 per GPU)")
     ap.add_argument("--quick", action="store_true", help="primary measurement only (no secondary modes, weak slab, drop-in timing)")
     ap.add_argument("--no-parity", action="store_true", help="skip the whole-volume oracle comparison")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the GPU path's outputs; the reference arm has none")
         return run_reference_arm(args)
     return run_ours(args)
 

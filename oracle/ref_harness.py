@@ -14,8 +14,7 @@ compare against:
 
 ``/root/reference`` exists only in the build container, so nothing in the
 ``-m gpu`` tests, ``smoke()`` or ``bench.py`` may import this module.  It is
-used by ``tests/golden/make_golden.py`` (which writes the committed fixtures)
-and by the container-only tests marked ``needs_reference``.
+used by ``tests/golden/make_golden.py``, which writes the committed fixtures.
 """
 from __future__ import annotations
 

@@ -33,6 +33,44 @@ def test_reference_arm_is_silent_on_other_ranks():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_bad_arguments_are_refused():
+    for extra in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "x"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                             timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and out.stdout == "", (extra, out.stderr[-500:])
+
+
+def test_dump_outputs_writes_a_fixed_sample_the_plane_counts_and_the_trace(tmp_path):
+    shape = (6, 7, 9)
+    labels = np.random.default_rng(1).integers(0, 5, size=shape, dtype=np.uint8)
+    trace = np.array([[-1, 8, 370], [3, 11, 367]])
+
+    class Ctx:
+        rank = 0
+
+        @staticmethod
+        def sum_f64(a):
+            return a
+
+    class Eng:
+        @staticmethod
+        def labels():
+            return labels.copy()
+
+    for d in ("a", "b"):
+        bench.dump_outputs(Ctx, Eng, trace, shape, 0, shape[0], str(tmp_path / d))
+    a = {n: np.load(str(tmp_path / "a" / (n + ".npy"))) for n in ("labels_sample", "labels_sample_index", "label_counts_per_plane", "trace")}
+    for n, v in a.items():
+        assert v.dtype in (np.float32, np.float64)
+        assert np.array_equal(v, np.load(str(tmp_path / "b" / (n + ".npy"))))
+    idx = a["labels_sample_index"].astype(np.int64)
+    assert np.array_equal(a["labels_sample"], labels.ravel()[idx])
+    assert np.array_equal(a["label_counts_per_plane"], [[np.count_nonzero(p == k) for k in range(5)] for p in labels])
+    assert np.array_equal(a["trace"], trace)
+    # the two sample files stay the same size on every workload, far below 64 MB
+    assert bench.DUMP_SAMPLE * (4 + 8) + bench.WORKLOADS["c5"][0] * 5 * 8 < 32 * 2 ** 20
+
+
 def test_cpu_sample_is_bounded_and_holds_seeds():
     for name in ("c2", "c3", "c5"):
         shape = bench.WORKLOADS[name]

@@ -545,3 +545,26 @@ def test_staged_upload_of_a_large_pageable_volume():
         res = eng.run()
         lab = eng.labels()
         assert (lab <= 1).sum() == res["n_in"] and res["n_in"] >= 4 * 12 * 300
+
+
+def test_bench_dump_outputs_equal_the_oracle(tmp_path):
+    """bench.py --dump-outputs writes what its last timed step computed: on config C1 the sampled labels, the label counts of
+    every plane and the trace equal oracle/vrg_oracle.c's on the same phantom."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    import bench
+    from oracle.c_oracle import vrg_oracle_c
+    out = subprocess.run([sys.executable, os.path.join(bench.ROOT, "bench.py"), "--workload", "c1", "--quick", "--steps", "2",
+                          "--warmup", "1", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+    assert line["steps"] == 2 and line["parity"]["oracle"] is True
+    h_data, h_vm = bench.host_phantom_via_device(bench.WORKLOADS["c1"], 0, 0)
+    ref = vrg_oracle_c(h_data, h_vm, max_segment_size=10 ** 15)
+    dump = {n: np.load(str(tmp_path / (n + ".npy"))) for n in ("labels_sample", "labels_sample_index", "label_counts_per_plane", "trace")}
+    assert np.array_equal(dump["labels_sample"], ref["labels"].ravel()[dump["labels_sample_index"].astype(np.int64)])
+    assert np.array_equal(dump["label_counts_per_plane"], [[np.count_nonzero(p == k) for k in range(5)] for p in ref["labels"]])
+    assert np.array_equal(dump["trace"], ref["trace"])

@@ -160,14 +160,3 @@ def test_label_hash_c_equals_numpy_and_adds_over_slabs():
     lab[0, 0, 0], lab[0, 0, 1] = 0, 1
     assert hash_labels(swapped) != hash_labels(lab)
 
-
-@pytest.mark.needs_reference
-def test_reference_dies_on_its_own_output():
-    """Feeding a returned valueMap back in (labels 1 / 2 present): the reference re-seeds from label 0 alone (VRG:44), turns
-    the old inner band into its outer band, never lists the old outer band again (VRG:143: `!= 2`), and dies at VRG:111 once
-    the outer list runs empty.  The drop-in instead resumes from the state the labels describe (tested on the GPU)."""
-    from oracle.ref_harness import run_reference
-    g = load_golden("sphere")
-    with pytest.raises((ValueError, IndexError)):
-        run_reference(g["data"], g["labels"].astype(np.int64), H=g["H"], max_segment_size=g["max_segment_size"],
-                      check_drift=False, record_band=False)
