@@ -18,6 +18,7 @@ INTENSITY_MODES = {"f64_dense": 0, "f64_band": 1, "index": 2, "continuous": 3}
 HALO = 2
 MAX_LEVELS = 65536
 P2P_HANDLE_BYTES = 192
+DTYPE_U8, DTYPE_I8, DTYPE_I16, DTYPE_I32, DTYPE_I64, DTYPE_F32, DTYPE_F64 = range(7)  # vrg_dtype
 BUF_SEG, BUF_EXCL, BUF_FLIPS, BUF_CANCELLED, BUF_LOCAL_STATS, BUF_GLOBAL_STATS, BUF_CTRL = range(7)
 ST_N_IN, ST_N_OUT, ST_N_EXCL, ST_N_FLIPS, ST_N_BAND, ST_BAD_LABEL, ST_NONFINITE, ST_TIME_UP = range(8)
 ST_Q_CANCELLED, ST_Q_ADD_INSIDE, ST_Q_REM_OUTSIDE, ST_Q_REPROMOTED = 8, 9, 10, 11
@@ -59,6 +60,7 @@ _SIGS = {
     "vrg_upload_device": [vp, vp, vp],
     "vrg_upload_value_map": [vp, vp],
     "vrg_attach_device": [vp, vp, vp],
+    "vrg_attach_device_typed": [vp, vp, vp, ctypes.c_int32],
     "vrg_scan_levels": [vp, ctypes.POINTER(i64)],
     "vrg_get_levels": [vp, vp, i64],
     "vrg_set_levels": [vp, vp, i64],
@@ -92,6 +94,8 @@ _SIGS = {
     "vrg_download_labels": [vp, vp],
     "vrg_download_segmented_map": [vp, vp],
     "vrg_labels_device": [vp, vp],
+    "vrg_labels_device_typed": [vp, vp, ctypes.c_int32, ctypes.c_int32],
+    "vrg_segmented_device": [vp, vp, i64, ctypes.POINTER(i64)],
     "vrg_download_segmented": [vp, vp, i64, ctypes.POINTER(i64)],
     "vrg_get_trace": [vp, vp, i64, ctypes.POINTER(i64)],
     "vrg_get_table": [vp, vp, vp, i64],

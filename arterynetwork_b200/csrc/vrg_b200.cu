@@ -7,6 +7,8 @@
 #include "vrg_parzen.cuh"
 #include "vrg_scratch.cuh"
 
+#include <cub/cub.cuh>
+
 #include <algorithm>
 #include <chrono>
 #include <cmath>
@@ -73,7 +75,8 @@ struct vrg_handle {
     bool no_ahead = false;  // A/B switch VRG_NO_AHEAD: vrg_run looks at a batch's status before it queues the next one
     bool no_wide = false;  // A/B switch VRG_NO_WIDE: rows of 31 / 32 words stay two 16-word segments in the dense sweep
     bool dense_attr_set = false, force_ldg = false, hist_attr_set = false, attached = false;
-    const uint8_t *vm_base = nullptr;  // valueMap as indexed by local plane (own buffer or attached)
+    const void *vm_base = nullptr;  // valueMap as indexed by local plane (own uint8 buffer, or attached in its own dtype)
+    int vm_dtype = VRG_DTYPE_U8;
     // optional per-kernel timing (CUDA events on the launch stream), see vrg_profile
     bool prof = false;
     std::vector<cudaEvent_t> ev;   // 4 events per enqueued iteration: decide begin/end, cancel begin/end
@@ -269,7 +272,7 @@ int vrg_create(const vrg_config *cfg, vrg_handle **out) {
 int vrg_destroy(vrg_handle *h) {
     if (!h) return VRG_OK;
     cudaSetDevice(h->cfg.device);
-    if (h->stream) cudaStreamSynchronize(h->stream);
+    cudaStreamSynchronize(h->stream);  // also a caller's stream set by vrg_set_stream, the legacy default one (NULL) included
     for (void *big : {(void *)h->d_data, (void *)h->d_vm, (void *)h->d_index, (void *)h->d_labels})
         if (big) cudaFreeAsync(big, h->stream);
     if (h->stream) cudaStreamSynchronize(h->stream);
@@ -329,6 +332,7 @@ static int upload_impl(vrg_handle *h, const double *data, const uint8_t *vm, cud
     h->attached = false;
     p.data = h->d_data;
     h->vm_base = h->d_vm;
+    h->vm_dtype = VRG_DTYPE_U8;
     if (data) {
         CK(cudaMemcpyAsync(h->d_data + off, data, n * sizeof(double), kind, h->stream));
         h->have_data = true;
@@ -390,6 +394,7 @@ int vrg_upload(vrg_handle *h, const double *d, const uint8_t *vm) {
     { int rc_ = ensure_input_buffers(h); if (rc_ != VRG_OK) return rc_; }
     p.data = h->d_data;
     h->vm_base = h->d_vm;
+    h->vm_dtype = VRG_DTYPE_U8;
     const size_t off = (size_t)p.valid_lo * p.plane_vox, n = (size_t)(p.valid_hi - p.valid_lo) * p.plane_vox;
     { int rc_ = staged_h2d(h, h->d_data + off, d, n * sizeof(double)); if (rc_ != VRG_OK) return rc_; }
     { int rc_ = staged_h2d(h, h->d_vm + off, vm, n); if (rc_ != VRG_OK) return rc_; }
@@ -403,14 +408,31 @@ int vrg_upload_device(vrg_handle *h, const double *d, const uint8_t *vm) {
     if (!d && !vm) return fail(VRG_ERR_ARG, "null buffer");
     return upload_impl(h, d, vm, cudaMemcpyDeviceToDevice);
 }
+static size_t dtype_size(int dtype) {
+    switch (dtype) {
+        case VRG_DTYPE_U8: case VRG_DTYPE_I8: return 1;
+        case VRG_DTYPE_I16: return 2;
+        case VRG_DTYPE_I32: case VRG_DTYPE_F32: return 4;
+        case VRG_DTYPE_I64: case VRG_DTYPE_F64: return 8;
+        default: return 0;
+    }
+}
 // Zero-copy: run on the caller's device-resident extended slab (read-only; must stay alive until the run ends).
 int vrg_attach_device(vrg_handle *h, const double *data_dev, const uint8_t *vm_dev) {
+    return vrg_attach_device_typed(h, data_dev, vm_dev, VRG_DTYPE_U8);
+}
+// same, with the valueMap in any vrg_dtype: vrg_init reads it as it is (no conversion pass)
+int vrg_attach_device_typed(vrg_handle *h, const double *data_dev, const void *vm_dev, int32_t vm_dtype) {
     if (!h || !data_dev || !vm_dev) return fail(VRG_ERR_ARG, "null argument");
+    const size_t es = dtype_size(vm_dtype);
+    if (!es) return fail(VRG_ERR_ARG, "unknown valueMap dtype %d", (int)vm_dtype);
+    if ((uintptr_t)vm_dev % es) return fail(VRG_ERR_ARG, "valueMap buffer not aligned to its element size");
     CK(cudaSetDevice(h->cfg.device));
     Params &p = h->p;
     const long long off = (long long)p.valid_lo * p.plane_vox;  // kernels index by local plane; only valid planes are read
     p.data = (const double *)((uintptr_t)data_dev - (uintptr_t)off * sizeof(double));
-    h->vm_base = (const uint8_t *)((uintptr_t)vm_dev - (uintptr_t)off);
+    h->vm_base = (const void *)((uintptr_t)vm_dev - (uintptr_t)off * es);
+    h->vm_dtype = vm_dtype;
     h->attached = true;
     h->have_data = true;
     h->have_levels = false;
@@ -637,6 +659,20 @@ static int cont_alloc(vrg_handle *h) {
     return VRG_OK;
 }
 
+// bit-planes from the valueMap, read in its own dtype (vrg_attach_device_typed)
+static void launch_init_planes(vrg_handle *h) {
+    const Params &p = h->p;
+    switch (h->vm_dtype) {
+        case VRG_DTYPE_I8: k_init_planes<int8_t><<<h->grid, BLOCK, 0, h->stream>>>(p, (const int8_t *)h->vm_base, h->d_E); break;
+        case VRG_DTYPE_I16: k_init_planes<int16_t><<<h->grid, BLOCK, 0, h->stream>>>(p, (const int16_t *)h->vm_base, h->d_E); break;
+        case VRG_DTYPE_I32: k_init_planes<int32_t><<<h->grid, BLOCK, 0, h->stream>>>(p, (const int32_t *)h->vm_base, h->d_E); break;
+        case VRG_DTYPE_I64: k_init_planes<int64_t><<<h->grid, BLOCK, 0, h->stream>>>(p, (const int64_t *)h->vm_base, h->d_E); break;
+        case VRG_DTYPE_F32: k_init_planes<float><<<h->grid, BLOCK, 0, h->stream>>>(p, (const float *)h->vm_base, h->d_E); break;
+        case VRG_DTYPE_F64: k_init_planes<double><<<h->grid, BLOCK, 0, h->stream>>>(p, (const double *)h->vm_base, h->d_E); break;
+        default: k_init_planes<uint8_t><<<h->grid, BLOCK, 0, h->stream>>>(p, (const uint8_t *)h->vm_base, h->d_E); break;
+    }
+}
+
 // init of the continuous mode: no level table; region sizes by counting, every band voxel gets its full sums
 static int cont_init(vrg_handle *h) {
     Params &p = h->p;
@@ -675,7 +711,7 @@ static int cont_init(vrg_handle *h) {
     CK(cudaMemsetAsync(h->d_C, 0, h->plane_bytes, h->stream));
     CK(cudaMemsetAsync(q.AB, 0, h->plane_bytes, h->stream));
     p.E = h->d_E; p.C = h->d_C;
-    k_init_planes<<<h->grid, BLOCK, 0, h->stream>>>(p, h->vm_base, h->d_E);
+    launch_init_planes(h);
     k_init_bands<<<h->grid, BLOCK, 0, h->stream>>>(p);  // E = Eraw & ~dil26(S), VRG:137
     k_cont_count<<<h->grid, BLOCK, 0, h->stream>>>(p);
     k_cont_band<<<h->grid, BLOCK, 0, h->stream>>>(p, q);
@@ -761,7 +797,7 @@ int vrg_init(vrg_handle *h) {
     memcpy(h->h_ctrl, c, sizeof c);
     CK(cudaMemcpyAsync(h->d_ctrl, h->h_ctrl, sizeof c, cudaMemcpyHostToDevice, h->stream));
     p.E = h->d_E; p.C = h->d_C;
-    k_init_planes<<<h->grid, BLOCK, 0, h->stream>>>(p, h->vm_base, h->d_E);
+    launch_init_planes(h);
     k_init_bands<<<h->grid, BLOCK, 0, h->stream>>>(p);
     { int rc_ = launch_init_hist(h); if (rc_ != VRG_OK) return rc_; }
     h->launches += 3;
@@ -1513,7 +1549,7 @@ int vrg_plane_geometry(vrg_handle *h, int64_t *wpr, int64_t *wpp, int64_t *npl) 
 
 // ---- outputs ----------------------------------------------------------------------------------------
 static int labels_impl(vrg_handle *h, uint8_t *dev_out, int seg_only) {
-    k_labels<<<h->grid, BLOCK, 0, h->stream>>>(h->p, dev_out, seg_only);
+    k_labels<uint8_t><<<h->grid, BLOCK, 0, h->stream>>>(h->p, dev_out, seg_only);
     h->launches++;
     CK(cudaGetLastError());
     return VRG_OK;
@@ -1522,6 +1558,27 @@ int vrg_labels_device(vrg_handle *h, uint8_t *out) {
     NEED_INIT();
     if (!out) return fail(VRG_ERR_ARG, "null buffer");
     return labels_impl(h, out, 0);
+}
+// labels 0..4 (or the 0/1 segmented map) of the own planes as `dtype`, into a device buffer; on the handle's stream, no sync
+int vrg_labels_device_typed(vrg_handle *h, void *out, int32_t dtype, int32_t seg_only) {
+    NEED_INIT();
+    if (!out) return fail(VRG_ERR_ARG, "null buffer");
+    const size_t es = dtype_size(dtype);
+    if (!es) return fail(VRG_ERR_ARG, "unknown dtype %d", (int)dtype);
+    if ((uintptr_t)out % es) return fail(VRG_ERR_ARG, "output buffer not aligned to its element size");
+    const int so = seg_only ? 1 : 0;
+    switch (dtype) {
+        case VRG_DTYPE_I8: k_labels<int8_t><<<h->grid, BLOCK, 0, h->stream>>>(h->p, (int8_t *)out, so); break;
+        case VRG_DTYPE_I16: k_labels<int16_t><<<h->grid, BLOCK, 0, h->stream>>>(h->p, (int16_t *)out, so); break;
+        case VRG_DTYPE_I32: k_labels<int32_t><<<h->grid, BLOCK, 0, h->stream>>>(h->p, (int32_t *)out, so); break;
+        case VRG_DTYPE_I64: k_labels<int64_t><<<h->grid, BLOCK, 0, h->stream>>>(h->p, (int64_t *)out, so); break;
+        case VRG_DTYPE_F32: k_labels<float><<<h->grid, BLOCK, 0, h->stream>>>(h->p, (float *)out, so); break;
+        case VRG_DTYPE_F64: k_labels<double><<<h->grid, BLOCK, 0, h->stream>>>(h->p, (double *)out, so); break;
+        default: k_labels<uint8_t><<<h->grid, BLOCK, 0, h->stream>>>(h->p, (uint8_t *)out, so); break;
+    }
+    h->launches++;
+    CK(cudaGetLastError());
+    return VRG_OK;
 }
 static int download_impl(vrg_handle *h, uint8_t *out, int seg_only) {
     NEED_INIT();
@@ -1623,6 +1680,41 @@ int vrg_download_segmented(vrg_handle *h, int64_t *coords, int64_t cap, int64_t 
                 }
             }
         }
+    *n_out = n;
+    return VRG_OK;
+}
+
+// the same rows compacted on the device: per-row popcounts, an exclusive scan (CUB), a scatter of the triples.  The count
+// travels to the host (the one synchronisation); rows beyond `cap` are not written.
+int vrg_segmented_device(vrg_handle *h, int64_t *rows_dev, int64_t cap, int64_t *n_out) {
+    NEED_INIT();
+    if (!n_out) return fail(VRG_ERR_ARG, "null argument");
+    const Params &p = h->p;
+    const long long nrows_ll = (long long)h->nz_own * p.Y;
+    if (nrows_ll >= (1LL << 31) - 1) return fail(VRG_ERR_ARG, "too many rows for the device compaction");
+    const int nrows = (int)nrows_ll;
+    size_t tmp_bytes = 0;
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, (const long long *)nullptr, (long long *)nullptr, nrows + 1, h->stream));
+    const size_t cnt_bytes = ((size_t)(nrows + 1) * sizeof(long long) + 255) & ~(size_t)255;
+    char *buf = nullptr;
+    CK(big_alloc(h, (void **)&buf, 2 * cnt_bytes + tmp_bytes));
+    long long *counts = (long long *)buf, *offs = (long long *)(buf + cnt_bytes);
+    cudaError_t e = cudaMemsetAsync(counts + nrows, 0, sizeof(long long), h->stream);
+    if (e == cudaSuccess) {
+        k_seg_count<<<h->grid, BLOCK, 0, h->stream>>>(p, counts, nrows);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cub::DeviceScan::ExclusiveSum(buf + 2 * cnt_bytes, tmp_bytes, counts, offs, nrows + 1, h->stream);
+    if (e == cudaSuccess && rows_dev && cap > 0) {
+        k_seg_scatter<<<h->grid, BLOCK, 0, h->stream>>>(p, offs, nrows, (long long *)rows_dev, (long long)cap, (long long)h->cfg.z_begin);
+        e = cudaGetLastError();
+    }
+    long long n = 0;
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&n, offs + nrows, sizeof n, cudaMemcpyDeviceToHost, h->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    cudaFreeAsync(buf, h->stream);
+    if (e != cudaSuccess) return fail(VRG_ERR_CUDA, "segmented rows on the device: %s", cudaGetErrorString(e));
+    h->launches += 2 + (rows_dev && cap > 0);
     *n_out = n;
     return VRG_OK;
 }

@@ -1091,11 +1091,62 @@ __global__ void k_advance(Params p) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// init branch of update(), VRG:129-145: bit-planes from the uint8 valueMap, one word (32 voxels) per thread.
+// init branch of update(), VRG:129-145: bit-planes from the valueMap, read in the caller's dtype.
 // Seeds are label 0 (VRG:44); a map that already holds band labels (1 inner, 2 outer: the output of an earlier run) is
 // read as the state those labels describe -- segmented = {0, 1}.  (The reference re-seeds such a map from label 0 alone
 // and then dies at VRG:111 once its outer band list runs empty: tests/test_oracle_golden.py keeps that probe.)
-__global__ void __launch_bounds__(BLOCK) k_init_planes(Params p, const uint8_t *__restrict__ vm, uint32_t *eraw) {
+// Anything that is not an integral value in 0..4 (negative, fractional, NaN, above 4) raises ST_BAD_LABEL.
+template <typename T>
+__device__ __forceinline__ bool label_value(T v, int &lab) {
+    if constexpr (std::is_floating_point<T>::value) {
+        const bool ok = v >= T(0) && v <= T(4) && v == floor(v);  // NaN fails every comparison
+        lab = ok ? (int)v : 0;
+        return ok;
+    } else if constexpr (std::is_signed<T>::value) {
+        const bool ok = v >= T(0) && v <= T(4);
+        lab = ok ? (int)v : 0;
+        return ok;
+    } else {
+        lab = v <= T(4) ? (int)v : 0;
+        return v <= T(4);
+    }
+}
+
+// Wider (or signed) types: one warp per row, one lane per voxel -- a 32-voxel word is one coalesced 32-lane load and two
+// ballots; lane j keeps word c0 + j, so that the 32 words of a batch go out as one coalesced warp store.  uint8 (the
+// specialisation below): one word per thread, 16-byte loads and per-byte compares.
+template <typename T>
+__global__ void __launch_bounds__(BLOCK) k_init_planes(Params p, const T *__restrict__ vm, uint32_t *eraw) {
+    const int nrows = (p.valid_hi - p.valid_lo) * p.Y, lane = threadIdx.x & 31;
+    const int nwarps = gridDim.x * WARPS;
+    bool bad = false;
+    for (int r = blockIdx.x * WARPS + (threadIdx.x >> 5); r < nrows; r += nwarps) {
+        const int y = r % p.Y, zl = p.valid_lo + r / p.Y;
+        const T *src = vm + (long long)zl * p.plane_vox + (long long)y * p.X;
+        for (int c0 = 0; c0 < p.XW; c0 += 32) {
+            const int nw = min(32, p.XW - c0);
+            uint32_t my_s = 0, my_e = 0;
+#pragma unroll 4
+            for (int j = 0; j < nw; ++j) {
+                const int x = (c0 + j) * 32 + lane;
+                int lab = 3;
+                if (x < p.X) bad |= !label_value<T>(src[x], lab);
+                const uint32_t s = __ballot_sync(FULL, lab <= 1), e = __ballot_sync(FULL, lab == 4);
+                if (lane == j) { my_s = s; my_e = e; }
+            }
+            if (lane < nw) {
+                const int c = c0 + lane;
+                const long long widx = (long long)zl * p.plane_words + (long long)y * p.WP + c;
+                p.S[widx] = my_s;
+                if (my_s) p.unitmap[unit_index(p, zl, y, c)] = 1;
+                if (eraw) eraw[widx] = my_e;
+            }
+        }
+    }
+    if (bad) p.lstats[2 * p.L + ST_BAD_LABEL] = 1;
+}
+template <>
+__global__ void __launch_bounds__(BLOCK) k_init_planes<uint8_t>(Params p, const uint8_t *__restrict__ vm, uint32_t *eraw) {
     const int nrows = (p.valid_hi - p.valid_lo) * p.Y, lane = threadIdx.x & 31;
     const int nwarps = gridDim.x * WARPS;
     bool bad = false;
@@ -1584,8 +1635,11 @@ __global__ void __launch_bounds__(BLOCK) k_build_index(Params p, const double *_
 }
 
 // ---------------------------------------------------------------------------------------------
-// outputs: canonical labels (VRG:21) or the 0/1 segmented map, one byte per voxel, own planes only
-__global__ void __launch_bounds__(BLOCK) k_labels(Params p, uint8_t *__restrict__ out, int seg_only) {
+// outputs: canonical labels (VRG:21) or the 0/1 segmented map as T, own planes only, straight into a buffer of the caller's
+// dtype.  One-byte types: 4 voxels (bytes) per lane and store; wider types: one voxel per lane, a warp writes the 32 voxels of
+// one word per store (32 * sizeof(T) consecutive bytes).
+template <typename T>
+__global__ void __launch_bounds__(BLOCK) k_labels(Params p, T *__restrict__ out, int seg_only) {
     const int lane = threadIdx.x & 31;
     const int nyb = (p.Y + ROWS_PER_UNIT - 1) / ROWS_PER_UNIT;
     const long long nunits = (long long)(p.own_hi - p.own_lo) * nyb * p.nseg;
@@ -1601,29 +1655,90 @@ __global__ void __launch_bounds__(BLOCK) k_labels(Params p, uint8_t *__restrict_
             const long long widx = (long long)un.zl * p.plane_words + (long long)y * p.WP + c;
             const uint32_t e = (p.E && st.active) ? p.E[widx] : 0u;
             outer &= ~e;
-            // 4 voxels (bytes) per lane and store: a warp writes 128 consecutive voxels = 4 words per step
-            uint8_t *rowout = out + ((long long)(un.zl - p.own_lo) * p.Y + y) * p.X;
-            for (int j0 = 1; j0 <= p.segw; j0 += 4) {
-                if (c0 + j0 >= p.XW) break;
-                const int src = j0 + (lane >> 3);  // lane that holds this lane's word
-                const uint32_t sj = __shfl_sync(FULL, s, src), ij = __shfl_sync(FULL, inner, src);
-                const uint32_t oj = __shfl_sync(FULL, outer, src), ej = __shfl_sync(FULL, e, src);
-                if (src > p.segw) continue;
-                const int x = (c0 + src) * 32 + (lane & 7) * 4;
-                uint32_t pack = 0;
+            if constexpr (sizeof(T) == 1) {
+                // 4 voxels (bytes) per lane and store: a warp writes 128 consecutive voxels = 4 words per step
+                uint8_t *rowout = (uint8_t *)out + ((long long)(un.zl - p.own_lo) * p.Y + y) * p.X;
+                for (int j0 = 1; j0 <= p.segw; j0 += 4) {
+                    if (c0 + j0 >= p.XW) break;
+                    const int src = j0 + (lane >> 3);  // lane that holds this lane's word
+                    const uint32_t sj = __shfl_sync(FULL, s, src), ij = __shfl_sync(FULL, inner, src);
+                    const uint32_t oj = __shfl_sync(FULL, outer, src), ej = __shfl_sync(FULL, e, src);
+                    if (src > p.segw) continue;
+                    const int x = (c0 + src) * 32 + (lane & 7) * 4;
+                    uint32_t pack = 0;
 #pragma unroll
-                for (int b = 0; b < 4; ++b) {
-                    const uint32_t bit = 1u << ((lane & 7) * 4 + b);
-                    uint32_t lab;
-                    if (seg_only) lab = (sj & bit) ? 1u : 0u;
-                    else lab = (sj & bit) ? ((ij & bit) ? 1u : 0u) : ((ej & bit) ? 4u : ((oj & bit) ? 2u : 3u));
-                    pack |= lab << (8 * b);
+                    for (int b = 0; b < 4; ++b) {
+                        const uint32_t bit = 1u << ((lane & 7) * 4 + b);
+                        uint32_t lab;
+                        if (seg_only) lab = (sj & bit) ? 1u : 0u;
+                        else lab = (sj & bit) ? ((ij & bit) ? 1u : 0u) : ((ej & bit) ? 4u : ((oj & bit) ? 2u : 3u));
+                        pack |= lab << (8 * b);
+                    }
+                    if (x + 3 < p.X && ((((uintptr_t)(rowout + x)) & 3) == 0)) *(uint32_t *)(rowout + x) = pack;
+                    else
+                        for (int b = 0; b < 4; ++b)
+                            if (x + b < p.X) rowout[x + b] = (uint8_t)(pack >> (8 * b));
                 }
-                if (x + 3 < p.X && ((((uintptr_t)(rowout + x)) & 3) == 0)) *(uint32_t *)(rowout + x) = pack;
-                else
-                    for (int b = 0; b < 4; ++b)
-                        if (x + b < p.X) rowout[x + b] = (uint8_t)(pack >> (8 * b));
+            } else {
+                T *rowout = out + ((long long)(un.zl - p.own_lo) * p.Y + y) * p.X;
+                const uint32_t bit = 1u << lane;
+                for (int j = 1; j <= p.segw; ++j) {
+                    if (c0 + j >= p.XW) break;
+                    const uint32_t sj = __shfl_sync(FULL, s, j), ij = __shfl_sync(FULL, inner, j);
+                    const uint32_t oj = __shfl_sync(FULL, outer, j), ej = __shfl_sync(FULL, e, j);
+                    int lab;
+                    if (seg_only) lab = (sj & bit) ? 1 : 0;
+                    else lab = (sj & bit) ? ((ij & bit) ? 1 : 0) : ((ej & bit) ? 4 : ((oj & bit) ? 2 : 3));
+                    const int x = (c0 + j) * 32 + lane;
+                    if (x < p.X) rowout[x] = (T)lab;
+                }
             }
+        }
+    }
+}
+
+// segmented rows on the device (vrg_segmented_device): popcount of every own-plane row of S, one warp per row ...
+__global__ void __launch_bounds__(BLOCK) k_seg_count(Params p, long long *__restrict__ counts, int nrows) {
+    const int lane = threadIdx.x & 31;
+    for (int r = blockIdx.x * WARPS + (threadIdx.x >> 5); r < nrows; r += gridDim.x * WARPS) {
+        const uint32_t *row = p.S + (long long)(p.own_lo + r / p.Y) * p.plane_words + (long long)(r % p.Y) * p.WP;
+        long long n = 0;
+        for (int c = lane; c < p.XW; c += 32) n += __popc(row[c]);
+        n = warp_sum(n);
+        if (lane == 0) counts[r] = n;
+    }
+}
+// ... and, behind an exclusive scan of those counts, the (z, y, x) triples of the row's set bits in C order, z_begin added.
+// A warp takes 32 words of the row at a time; a warp scan of their popcounts gives each lane its first output row.
+__global__ void __launch_bounds__(BLOCK) k_seg_scatter(Params p, const long long *__restrict__ offs, int nrows,
+                                                       long long *__restrict__ rows, long long cap, long long z_begin) {
+    const int lane = threadIdx.x & 31;
+    for (int r = blockIdx.x * WARPS + (threadIdx.x >> 5); r < nrows; r += gridDim.x * WARPS) {
+        const int zl = r / p.Y, y = r % p.Y;
+        const uint32_t *row = p.S + (long long)(p.own_lo + zl) * p.plane_words + (long long)y * p.WP;
+        long long base = offs[r];
+        for (int c0 = 0; c0 < p.XW; c0 += 32) {
+            const int c = c0 + lane;
+            uint32_t w = c < p.XW ? row[c] : 0u;
+            const int n = __popc(w);
+            int incl = n;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int t = __shfl_up_sync(FULL, incl, o);
+                if (lane >= o) incl += t;
+            }
+            long long k = base + incl - n;
+            while (w) {
+                const int b = __ffs(w) - 1;
+                w &= w - 1;
+                if (k < cap) {
+                    rows[3 * k] = z_begin + zl;
+                    rows[3 * k + 1] = y;
+                    rows[3 * k + 2] = (long long)c * 32 + b;
+                }
+                ++k;
+            }
+            base += __shfl_sync(FULL, incl, 31);
         }
     }
 }

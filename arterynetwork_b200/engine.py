@@ -92,6 +92,10 @@ class VRGEngine:
         """Zero-copy: run on the caller's device-resident extended slab (fp64 data, uint8 valueMap)."""
         nat.check(self.lib.vrg_attach_device(self._h, nat.vp(data_ptr), nat.vp(value_map_ptr)))
 
+    def attach_device_typed(self, data_ptr: int, value_map_ptr: int, value_map_dtype: int):
+        """Zero-copy like ``attach_device``, the valueMap in its own dtype (``nat.DTYPE_*``): vrg_init reads it as it is."""
+        nat.check(self.lib.vrg_attach_device_typed(self._h, nat.vp(data_ptr), nat.vp(value_map_ptr), int(value_map_dtype)))
+
     # -- levels -----------------------------------------------------------------------------
     def scan_levels(self) -> np.ndarray:
         n = nat.i64(0)
@@ -225,6 +229,18 @@ class VRGEngine:
 
     def labels_device(self, dev_ptr: int):
         nat.check(self.lib.vrg_labels_device(self._h, nat.vp(dev_ptr)))
+
+    def labels_device_typed(self, dev_ptr: int, dtype: int, segmented_only: bool = False):
+        """Own planes' labels 0..4 (or the 0/1 segmented map) as ``dtype`` (``nat.DTYPE_*``) into a device buffer, on the
+        handle's stream (no synchronisation)."""
+        nat.check(self.lib.vrg_labels_device_typed(self._h, nat.vp(dev_ptr), int(dtype), int(bool(segmented_only))))
+
+    def segmented_device(self, rows_ptr, cap: int) -> int:
+        """Rows (z, y, x) of the own planes' segmented voxels, C order, compacted on the device into ``rows_ptr`` (int64,
+        ``cap`` rows; None: count only).  Returns their number; rows beyond ``cap`` are not written."""
+        n = nat.i64(0)
+        nat.check(self.lib.vrg_segmented_device(self._h, nat.vp(rows_ptr or None), int(cap), ctypes.byref(n)))
+        return int(n.value)
 
     def segmented(self, at_most=None) -> np.ndarray:
         """Rows (z, y, x) of the segmented voxels of the own planes, C order.  ``at_most``: an upper bound of their number

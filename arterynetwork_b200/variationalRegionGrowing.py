@@ -7,6 +7,15 @@ B200s through ``libvrg_b200.so``.
     from arterynetwork_b200.variationalRegionGrowing import variationalRegionGrowing
     segmented, segmentedMap, valueMap = variationalRegionGrowing(dataArray, valueMap)
 
+CUDA tensors: when ``valueMap`` is a CUDA tensor (and ``dataArray`` a CUDA tensor on the same device) the call runs on
+that device and torch's current stream and returns tensors -- ``valueMap`` is the same tensor, updated in place and kept
+in its own dtype (uint8, int8, int16, int32, int64, float32 or float64; the kernels read and write the labels in that dtype),
+``segmentedMap`` a new C-contiguous int64 CUDA tensor, ``segmented`` an int64 CUDA tensor (K, ndim) in C order of the
+caller's axes; stdout, ``LAST_RUN`` and the warning as below.  Nothing of volume size crosses PCIe.  C-contiguous tensors
+are used as they are, F-contiguous ones (``torch.from_numpy(nibabel_volume).cuda()``) through their reversed-axes view,
+other strides through a contiguous copy whose labels are copied back; intensities other than float64 are converted once.
+On any error the caller's ``valueMap`` is left bit-unchanged.  ``DEVICES`` and ``LIST_ORDER = True`` take host arrays only.
+
 Module switches (the reference has none; defaults reproduce it):
 
 ``DEVICES``   ``None`` = one GPU (``DEVICE``); a list of CUDA ordinals or ``"all"`` =
@@ -45,6 +54,7 @@ Differences from the reference, all deliberate (DESIGN.md "Boundary"):
 from __future__ import annotations
 
 import itertools
+import sys
 import time
 import warnings
 from concurrent.futures import ThreadPoolExecutor
@@ -206,7 +216,7 @@ def _finish_lines(res, segmented, data3, nz=None):
     if nz is None:
         nz = sum(_pool_map(lambda zz: int(np.count_nonzero(data3[zz[0]:zz[1]])), _chunks(data3.shape[0], HOST_THREADS)))
     if res["exit_reason"] == nat.EXIT_MAX_ITER:  # VRG:118-120
-        print('Segmented points are: \n', segmented)
+        print('Segmented points are: \n', segmented if isinstance(segmented, np.ndarray) else segmented.cpu().numpy())
         print('Max iteration reached! Finished at iteration {}'.format(res["iterations"]))
     else:  # VRG:94-104
         print('Finished at iteration {}{}'.format(res["iterations"], _EXIT_SUFFIX[res["exit_reason"]]))
@@ -238,9 +248,123 @@ def _list_order_run(dataArray, valueMap, H, maxSegmentSize):
     return segmented, segmentedMap, valueMap
 
 
+def _label_dtype_code(torch, dtype):
+    return {torch.uint8: nat.DTYPE_U8, torch.int8: nat.DTYPE_I8, torch.int16: nat.DTYPE_I16, torch.int32: nat.DTYPE_I32,
+            torch.int64: nat.DTYPE_I64, torch.float32: nat.DTYPE_F32, torch.float64: nat.DTYPE_F64}.get(dtype)
+
+
+def _tensor_run(dataArray, valueMap, H, maxSegmentSize):
+    """The call on CUDA tensors: inputs attached where they are (the valueMap in its own dtype), labels written back by the
+    kernels in that dtype, segmentedMap and the segmented rows built on the device.  Nothing of volume size crosses PCIe."""
+    global LAST_RUN
+    import torch
+    if not isinstance(dataArray, torch.Tensor) or not dataArray.is_cuda:
+        raise TypeError("valueMap is a CUDA tensor: dataArray must be a CUDA tensor on the same device, got %s"
+                        % type(dataArray).__name__)
+    if dataArray.device != valueMap.device:
+        raise ValueError("dataArray (%s) and valueMap (%s) are on different devices" % (dataArray.device, valueMap.device))
+    if tuple(dataArray.shape) != tuple(valueMap.shape):
+        raise ValueError("dataArray and valueMap must have the same shape")
+    if LIST_ORDER:
+        raise NotImplementedError("variationalRegionGrowing: LIST_ORDER = True (the strict engine) takes host arrays, not "
+                                  "CUDA tensors")
+    if DEVICES is not None:
+        raise NotImplementedError("variationalRegionGrowing: DEVICES (z-slabs over several GPUs) takes host arrays, not CUDA "
+                                  "tensors; set DEVICES = None to run on the tensors' device")
+    nd = dataArray.dim()
+    if nd > 3 or nd == 0:
+        raise NotImplementedError("variationalRegionGrowing: 1-D to 3-D volumes only, got ndim=%d" % nd)
+    code = _label_dtype_code(torch, valueMap.dtype)
+    if code is None:
+        raise TypeError("valueMap dtype %s: uint8, int8, int16, int32, int64, float32 or float64 only" % valueMap.dtype)
+    if dataArray.is_complex():
+        raise TypeError("dataArray must hold real intensities, got %s" % dataArray.dtype)
+    clock = [time.perf_counter()]
+    host_seconds = {}
+
+    def lap(name):  # wall time per stage; stages that end in a synchronisation include the device work queued before them
+        now = time.perf_counter()
+        host_seconds[name] = host_seconds.get(name, 0.0) + now - clock[0]
+        clock[0] = now
+    dev = valueMap.device
+    rev = tuple(range(nd - 1, -1, -1))
+    # nibabel-style F-ordered volume: used through its reversed-axes view, as _as_zyx does for ndarrays
+    transposed = nd > 1 and not dataArray.is_contiguous() and dataArray.permute(rev).is_contiguous()
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev)
+        d = dataArray.permute(rev) if transposed else dataArray
+        if d.dtype != torch.float64:
+            d = d.to(torch.float64)  # processed as float64 whatever the input dtype, like the host path
+        d3 = d.contiguous().reshape((1,) * (3 - nd) + tuple(d.shape))  # (Z, Y, X), C order
+        vm_zyx = valueMap.permute(rev) if transposed else valueMap
+        work = vm_zyx if vm_zyx.is_contiguous() else vm_zyx.contiguous()  # other strides: a copy, written back on success
+        vm3 = work.reshape(d3.shape)
+        lap("prepare_inputs")
+
+        def run(mode):
+            with VRGEngine(d3.shape, H=H, max_segment_size=maxSegmentSize, iter_max=ITER_MAX, device=dev.index,
+                           intensity=mode, max_seconds=MAX_SECONDS or 0.0) as eng:
+                eng.set_stream(stream.cuda_stream)
+                eng.attach_device_typed(d3.data_ptr(), vm3.data_ptr(), code)
+                lap("create_handle")
+                eng.init()
+                res = eng.run()
+                lap("levels_init_iterations")
+                cap = res["n_in"]
+                rows = torch.empty((cap, 3), dtype=torch.int64, device=dev)
+                n = eng.segmented_device(rows.data_ptr() if cap else None, cap)
+                if n > cap:  # not expected on one GPU (n_in is the count); once more with the right size
+                    rows = torch.empty((n, 3), dtype=torch.int64, device=dev)
+                    eng.segmented_device(rows.data_ptr(), n)
+                rows = rows[:n]
+                lap("segmented_rows")
+                nonzero = eng.count_nonzero()  # np.count_nonzero(dataArray) of VRG:95
+                lap("count_nonzero_on_device")
+                seg3 = torch.empty(d3.shape, dtype=torch.int64, device=dev)
+                eng.labels_device_typed(seg3.data_ptr(), nat.DTYPE_I64, segmented_only=True)
+                # the caller's map is written last, once everything else has succeeded (VRG:137-228: in place)
+                eng.labels_device_typed(vm3.data_ptr(), code)
+                lap("labels_out")
+            lap("destroy_handle")
+            return res, rows, nonzero, seg3
+
+        try:
+            res, rows, nonzero, seg3 = run(INTENSITY)
+        except nat.LevelsError:
+            if d3.numel() > CONTINUOUS_MAX_VOXELS:  # same fallback as the host path
+                raise
+            res, rows, nonzero, seg3 = run("continuous")
+        if work is not vm_zyx:
+            vm_zyx.copy_(work)
+        segmented = rows[:, 3 - nd:]
+        if transposed:
+            segmented = segmented.flip(1)
+            key = segmented[:, 0].clone()
+            for ax in range(1, nd):
+                key = key * dataArray.shape[ax] + segmented[:, ax]
+            segmented = segmented[torch.argsort(key)]  # C order of the user's axes
+            segmentedMap = seg3.reshape(d.shape).permute(rev).contiguous()
+        else:
+            segmented = segmented.contiguous()
+            segmentedMap = seg3.reshape(dataArray.shape)
+        lap("user_layout")
+    LAST_RUN = dict(res)
+    LAST_RUN["host_seconds"] = host_seconds
+    _finish_lines(res, segmented, None, nonzero)
+    lap("print")
+    return segmented, segmentedMap, valueMap
+
+
 def variationalRegionGrowing(dataArray, valueMap, H=2.25, maxSegmentSize=5000):
     """B200 implementation of VRG:10-121.  See the module docstring for the contract."""
     global LAST_RUN
+    torch = sys.modules.get("torch")  # a tensor can only come from an imported torch
+    if torch is not None and isinstance(valueMap, torch.Tensor) and valueMap.is_cuda:
+        out = _tensor_run(dataArray, valueMap, H, maxSegmentSize)
+        _warn_order_dependence(LAST_RUN)
+        return out
+    if torch is not None and isinstance(dataArray, torch.Tensor) and dataArray.is_cuda:
+        raise TypeError("dataArray is a CUDA tensor: valueMap must be a CUDA tensor on the same device too")
     dataArray = np.asarray(dataArray)
     if not isinstance(valueMap, np.ndarray):
         raise TypeError("valueMap must be an ndarray (it is updated in place, as in the reference)")

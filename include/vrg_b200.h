@@ -112,6 +112,15 @@ int vrg_upload_device(vrg_handle *h, const double *data_dev, const uint8_t *valu
 int vrg_upload_value_map(vrg_handle *h, const uint8_t *value_map_host); /* new seeds, same data */
 /* zero-copy: run on the caller's device-resident extended slab (read-only, must outlive the run) */
 int vrg_attach_device(vrg_handle *h, const double *data_dev, const uint8_t *value_map_dev);
+/* element types of a device-resident valueMap (vrg_attach_device_typed) and of the typed label outputs */
+typedef enum {
+    VRG_DTYPE_U8 = 0, VRG_DTYPE_I8 = 1, VRG_DTYPE_I16 = 2, VRG_DTYPE_I32 = 3, VRG_DTYPE_I64 = 4,
+    VRG_DTYPE_F32 = 5, VRG_DTYPE_F64 = 6
+} vrg_dtype;
+/* zero-copy like vrg_attach_device, with the valueMap in any vrg_dtype: vrg_init reads it in that dtype (no conversion
+ * pass); anything but an integral value in 0..4 (negative, fractional, NaN, above 4) makes vrg_init return VRG_ERR_LABEL.
+ * The valueMap pointer must be aligned to its element size (any storage offset of a tensor view is). */
+int vrg_attach_device_typed(vrg_handle *h, const double *data_dev, const void *value_map_dev, int32_t value_map_dtype);
 
 /* distinct intensity levels (the decision table's domain) ------------------- */
 int vrg_scan_levels(vrg_handle *h, int64_t *n_levels);             /* local slab */
@@ -191,6 +200,9 @@ int vrg_enqueue_p2p_stats(vrg_handle *h);           /* statistics all-reduce + t
 int vrg_download_labels(vrg_handle *h, uint8_t *value_map_out);   /* own planes, canonical labels 0..4 */
 int vrg_download_segmented_map(vrg_handle *h, uint8_t *seg_out);  /* own planes, 0/1 */
 int vrg_labels_device(vrg_handle *h, uint8_t *value_map_dev_out); /* same, into a device buffer */
+/* own planes into a device buffer of that vrg_dtype: the canonical labels 0..4, or (segmented_only != 0) the 0/1 segmented map;
+ * enqueued on the handle's stream, no synchronisation */
+int vrg_labels_device_typed(vrg_handle *h, void *out_dev, int32_t dtype, int32_t segmented_only);
 /* position-sensitive 64-bit hash of the own planes' canonical labels: sum over voxels of
  * splitmix64_finalizer((global linear voxel index << 3) | label) mod 2^64.  Additive over z-slabs: the per-rank hashes of a
  * multi-GPU run add up to the hash of the whole label volume (oracle/c_oracle.py computes the same number on the CPU). */
@@ -201,6 +213,9 @@ int vrg_count_nonzero(vrg_handle *h, int64_t *count_out);
 int vrg_download_segmented_map_i64(vrg_handle *h, int64_t *seg_out);
 /* segmented voxel coordinates (z,y,x) of own planes in C order; returns count via n (cap in rows) */
 int vrg_download_segmented(vrg_handle *h, int64_t *coords_out, int64_t cap, int64_t *n);
+/* the same rows compacted on the device into device memory (rows_dev may be NULL: count only); rows beyond cap are not
+ * written; *n = their number.  Synchronises the handle's stream once, for the count. */
+int vrg_segmented_device(vrg_handle *h, int64_t *rows_dev, int64_t cap, int64_t *n);
 int vrg_get_trace(vrg_handle *h, int64_t *rows_out, int64_t cap_rows, int64_t *n_rows); /* (n_flips,n_in,n_out) */
 /* last decision table: in/out normalised Parzen sums per level (VRG:79-82), for parity checks */
 int vrg_get_table(vrg_handle *h, double *pin_out, double *pout_out, int64_t cap);
