@@ -72,6 +72,7 @@ _SIGS = {
     "vrg_enqueue_absorb": [vp],
     "vrg_enqueue_advance": [vp],
     "vrg_poll": [vp, ctypes.POINTER(Result)],
+    "vrg_dense_refresh_sweeps": [vp, ctypes.POINTER(i64)],
     "vrg_apply_flips": [vp, vp, i64, ctypes.POINTER(Result)],
     "vrg_enqueue_table": [vp],
     "vrg_p2p_connect_local": [ctypes.POINTER(vp), ctypes.c_int],

@@ -55,6 +55,7 @@ struct vrg_handle {
     int *d_front = nullptr, *d_dirty = nullptr, *d_stamp = nullptr;
     uint16_t *d_index = nullptr;
     uint32_t *d_S = nullptr, *d_E = nullptr, *d_F = nullptr, *d_C = nullptr;
+    uint32_t *d_Dc = nullptr;  // F64_DENSE: the decision bit-plane of the cached sweeps (vrg_kernels.cuh, dense_refresh)
     double *d_levels = nullptr, *d_pin = nullptr, *d_pout = nullptr, *d_kmat = nullptr;
     uint32_t *d_dbits = nullptr;
     long long *d_lstats = nullptr, *d_gstats = nullptr, *d_ctrl = nullptr, *d_trace = nullptr;
@@ -74,6 +75,7 @@ struct vrg_handle {
     bool slim_sweep = false;  // set while a pipelined batch is enqueued: the dense sweep runs in its 104-register variant
     bool no_ahead = false;  // A/B switch VRG_NO_AHEAD: vrg_run looks at a batch's status before it queues the next one
     bool no_wide = false;  // A/B switch VRG_NO_WIDE: rows of 31 / 32 words stay two 16-word segments in the dense sweep
+    bool no_dcache = false;  // A/B switch VRG_NO_DCACHE: no decision bit-plane, every dense sweep reads the fp64 volume
     bool dense_attr_set = false, force_ldg = false, hist_attr_set = false, attached = false;
     const void *vm_base = nullptr;  // valueMap as indexed by local plane (own uint8 buffer, or attached in its own dtype)
     int vm_dtype = VRG_DTYPE_U8;
@@ -198,6 +200,7 @@ int vrg_create(const vrg_config *cfg, vrg_handle **out) {
     h->grid = h->sms * 8;
     h->force_ldg = getenv("VRG_DENSE_LDG") != nullptr;  // A/B switch: plain loads instead of the TMA rings (sweep, init histogram)
     h->no_wide = getenv("VRG_NO_WIDE") != nullptr;
+    h->no_dcache = getenv("VRG_NO_DCACHE") != nullptr;
     h->no_ahead = getenv("VRG_NO_AHEAD") != nullptr;
     h->graph_ok = getenv("VRG_NO_GRAPH") == nullptr;    // A/B switch: vrg_run stays on plain stream launches
     h->tail_ok = getenv("VRG_NO_FUSED_TAIL") == nullptr;  // A/B switch: the separate kernels behind the sweep
@@ -237,6 +240,7 @@ int vrg_create(const vrg_config *cfg, vrg_handle **out) {
     alloc((void **)&h->d_E, h->plane_bytes);
     alloc((void **)&h->d_F, h->plane_bytes);
     alloc((void **)&h->d_C, h->plane_bytes);
+    if (cfg->intensity_mode == VRG_INTENSITY_F64_DENSE && !h->no_dcache) alloc((void **)&h->d_Dc, h->plane_bytes);
     alloc((void **)&h->d_rowflag, h->rowflag_bytes);
     h->unitmap_bytes = (size_t)p.nzl * ((Y + ROWS_PER_UNIT - 1) / ROWS_PER_UNIT) * p.nseg;
     alloc((void **)&h->d_unitmap, h->unitmap_bytes);
@@ -264,6 +268,7 @@ int vrg_create(const vrg_config *cfg, vrg_handle **out) {
     (void)nvox;  // the input buffers are allocated on the first vrg_upload*; vrg_attach_device needs none
     p.S = h->d_S; p.F = h->d_F; p.Cq = h->d_C; p.rowflag = h->d_rowflag; p.front = h->d_front; p.unitmap = h->d_unitmap; p.dirty = h->d_dirty; p.stamp = h->d_stamp;
     p.data = h->d_data;
+    p.Dc = h->d_Dc;
     p.ctrl = h->d_ctrl; p.trace = h->d_trace;
     *out = h;
     return VRG_OK;
@@ -276,7 +281,7 @@ int vrg_destroy(vrg_handle *h) {
     for (void *big : {(void *)h->d_data, (void *)h->d_vm, (void *)h->d_index, (void *)h->d_labels})
         if (big) cudaFreeAsync(big, h->stream);
     if (h->stream) cudaStreamSynchronize(h->stream);
-    cudaFree(h->d_S); cudaFree(h->d_E); cudaFree(h->d_F); cudaFree(h->d_C); cudaFree(h->d_rowflag); cudaFree(h->d_front); cudaFree(h->d_unitmap); cudaFree(h->d_dirty); cudaFree(h->d_stamp);
+    cudaFree(h->d_S); cudaFree(h->d_E); cudaFree(h->d_F); cudaFree(h->d_C); cudaFree(h->d_Dc); cudaFree(h->d_rowflag); cudaFree(h->d_front); cudaFree(h->d_unitmap); cudaFree(h->d_dirty); cudaFree(h->d_stamp);
     cudaFree(h->d_ctrl); cudaFree(h->d_trace); cudaFree(h->d_hash); cudaFree(h->d_hkeys); cudaFree(h->d_hcount); cudaFree(h->d_gbar); cudaFree(h->d_tail_dbg);
     free_levels(h);
     if (h->cont_alloc) {
@@ -866,6 +871,12 @@ static int enqueue_sweep(vrg_handle *h) {
             else k_sweep_dense<false><<<h->sms, DENSE_WARPS * 32, dsm, h->stream>>>(p);
         } else if (p.lattice) k_sweep_dense_ldg<true><<<h->grid, BLOCK, smem, h->stream>>>(p);
         else k_sweep_dense_ldg<false><<<h->grid, BLOCK, smem, h->stream>>>(p);
+        if (p.Dc != nullptr) {  // every sweep the refresh kernel above returns from at once
+            // 4 blocks of 256 threads x 56 registers per SM: one wave (8 would not all be resident: a second wave behind the
+            // first), half the SM's threads free for the pipelined run's statistics / table kernels
+            k_sweep_dense_cached<<<h->sms * 4, BLOCK, 0, h->stream>>>(p);
+            h->launches++;
+        }
     } else {
         LAUNCH_ML(k_sweep_band, h->grid, BLOCK, smem, p);
     }
@@ -1080,6 +1091,12 @@ int vrg_poll(vrg_handle *h, vrg_result *res) {
     return VRG_OK;
 }
 
+int vrg_dense_refresh_sweeps(vrg_handle *h, int64_t *n) {
+    if (!h || !n) return fail(VRG_ERR_ARG, "null argument");
+    *n = h->inited ? h->h_ctrl[C_REFRESHES] : 0;  // the control block as the last vrg_poll read it
+    return VRG_OK;
+}
+
 // Slab run without label 4: after cancel the iteration forks -- the halo exchange (push, wait, unpack) goes to a
 // second stream while the statistics exchange, the loop bookkeeping and the next decision table stay on the main one;
 // the next sweep is the join.  (With label 4 the absorb step sits between two halo exchanges: everything stays serial.)
@@ -1277,7 +1294,7 @@ static uint64_t run_signature(const vrg_handle *h) {
     };
     mix(&h->p, sizeof(Params));
     if (h->p2p_on) mix(&h->q, sizeof(P2P));
-    const int64_t extra[5] = {h->cfg.intensity_mode, h->p2p_on, h->force_ldg, h->tail_ok, h->pipe_mode};
+    const int64_t extra[6] = {h->cfg.intensity_mode, h->p2p_on, h->force_ldg, h->tail_ok, h->pipe_mode, h->no_dcache};
     mix(extra, sizeof extra);
     return x;
 }

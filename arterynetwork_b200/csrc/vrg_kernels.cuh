@@ -51,6 +51,7 @@ enum { C_STATUS = 0, C_ITER = 1, C_ITER_MAX = 2, C_MAX_SEG = 3, C_APPLY = 4, C_A
        // sweep differs from the one it read`; `the last tail kernel applied its update` (statistics kernels have work)
        C_TABLE_BUF = 14, C_TABLE_NEW = 15, C_TAIL_APPLIED = 16,
        C_REDOS = 17,  // sweeps of the pipelined run that were repeated because the table changed beside them
+       C_REFRESHES = 18,  // dense sweeps that evaluated every decision bit from the intensities (the others read them from Dc)
        C_WORDS = 24 };
 constexpr long long RUNNING = -1;
 
@@ -93,6 +94,9 @@ struct Params {
     const long long *gstats;          // global [2L + ST_EXTRA] (aliases lstats on one GPU)
     long long *ctrl;                  // [C_WORDS]
     long long *trace;                 // [3 * (iter_max + 2)]
+    uint32_t *Dc;                     // F64_DENSE: decision bit-plane (layout of S) written by the last refresh sweep, or nullptr
+                                      // (switch VRG_NO_DCACHE: every dense sweep is a refresh).  Last: in front of `index` it
+                                      // moved the later fields and k_sweep_dense<true> lost 14 registers and 20 % of its speed
 };
 
 __device__ __forceinline__ uint32_t *table_bits(const Params &p) { return p.dbits + (size_t)p.ctrl[C_TABLE_BUF] * p.LW; }
@@ -498,6 +502,20 @@ __device__ __forceinline__ void tma_bulk_load(void *smem_dst, const void *gmem_s
                  : "memory");
 }
 
+// The two kinds of dense sweep.  A voxel's decision bit D = dbits[level(I)] depends on the iteration only through the table, and
+// every change of the table stamps C_FULL_SWEEP, as do the start of a run and caller-chosen flips.  So a REFRESH sweep (the
+// stamp names it) evaluates D from the fp64 intensities and keeps the words in the bit-plane Dc (layout of S); every other sweep
+// of the run is CACHED: it reads D from Dc, and only for the words that hold a band voxel, instead of streaming 8 B per voxel.
+// Both kernels are enqueued for every sweep and one of them returns at once (the choice is on the device: the table is known
+// only there, and the batches are replayed graphs).  Without Dc (VRG_NO_DCACHE) every sweep is a refresh.
+__device__ __forceinline__ bool dense_refresh(const Params &p) {
+    return p.Dc == nullptr || p.ctrl[C_FULL_SWEEP] == p.ctrl[C_SWEEPS] + 1;
+}
+// the refresh sweep's counter (vrg_result.dense_refresh_sweeps); nothing else touches the word while a sweep runs
+__device__ __forceinline__ void count_refresh(const Params &p) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) p.ctrl[C_REFRESHES] += 1;
+}
+
 // Work distribution of the dense sweep.  A work unit = `dense_rows` consecutive rows of one (plane, segment) column; units are
 // numbered so that consecutive units are consecutive in memory.  Every warp starts with two statically assigned units
 // (w, w + nwarps) and then draws further units from a device-wide counter: at any moment the whole machine streams one
@@ -518,7 +536,8 @@ constexpr int WIDE_STAGE_BYTES = 32 * 32 * 8;
 template <bool LATTICE, bool WIDE>
 __device__ __forceinline__ void sweep_dense_body(const Params &p) {
     constexpr int SB = WIDE ? WIDE_STAGE_BYTES : STAGE_BYTES;
-    if (p.ctrl[C_STATUS] != RUNNING) return;
+    if (p.ctrl[C_STATUS] != RUNNING || !dense_refresh(p)) return;
+    count_refresh(p);
     extern __shared__ __align__(128) unsigned char smem_raw[];
     uint32_t *s_dbits = (uint32_t *)smem_raw;
     const int dbits_bytes = (p.LW * 4 + 127) & ~127;
@@ -648,6 +667,7 @@ __device__ __forceinline__ void sweep_dense_body(const Params &p) {
             for (int k = 0; k < BW; ++k) mine |= ((wd[k] >> (l[k] & 31)) & 1u) << (jb + k + (WIDE ? 0 : 1));
         }
         const uint32_t D = transpose32(mine, lane);
+        if (p.Dc != nullptr && st.active) p.Dc[widx] = D;
         __syncwarp();
         if (lane == 0 && pu < nunits) pre_issue(stage);  // the stage is drained (values are in registers): re-arm it for a later row
         if (++stage == DENSE_STAGES) { stage = 0; parity ^= 1u; }
@@ -690,13 +710,10 @@ __global__ void __launch_bounds__(DENSE_WARPS * 32) k_sweep_dense(Params p) { sw
 template <bool LATTICE, bool WIDE = false>
 __global__ void __maxnreg__(96) k_sweep_dense_slim(Params p) { sweep_dense_body<LATTICE, WIDE>(p); }
 
-// Fallback of the dense sweep for odd X (row segments not 16-byte aligned): plain coalesced 8-byte loads.
-template <bool LATTICE>
-__global__ void __launch_bounds__(BLOCK) k_sweep_dense_ldg(Params p) {
-    if (p.ctrl[C_STATUS] != RUNNING) return;
-    extern __shared__ uint32_t s_dbits[];
-    for (int i = threadIdx.x; i < p.LW; i += BLOCK) s_dbits[i] = table_bits(p)[i];
-    __syncthreads();
+// Fallback of the dense sweep for odd X (row segments not 16-byte aligned): plain coalesced 8-byte loads.  CACHED: the same
+// unit loop as the cached sweep, D from Dc (LATTICE and s_dbits unused).
+template <bool LATTICE, bool CACHED>
+__device__ __forceinline__ void sweep_dense_ldg_body(const Params &p, const uint32_t *s_dbits) {
     const int lane = threadIdx.x & 31;
     const int zlo = max(p.valid_lo, p.own_lo - 1), zhi = min(p.valid_hi, p.own_hi + 1);
     const int nyb = (p.Y + ROWS_PER_UNIT - 1) / ROWS_PER_UNIT;
@@ -706,6 +723,8 @@ __global__ void __launch_bounds__(BLOCK) k_sweep_dense_ldg(Params p) {
     Strip st;
     for (long long u = (long long)blockIdx.x * WARPS + (threadIdx.x >> 5); u < nunits; u += nwarps) {
         const Unit un = decode_unit(p, u, zlo, nyb);
+        // cached: a unit with no segmented voxel in or next to it has no band voxel, no flip and no row flag (k_sweep_band)
+        if (CACHED && !unit_near_segmented(p, un.zl, un.y0, un.sg, lane)) continue;
         const int c0 = un.sg * p.segw - 1, c = c0 + lane;
         const bool own = un.zl >= p.own_lo && un.zl < p.own_hi;
         st.begin(p, un.zl, un.y0, c, lane);
@@ -717,22 +736,27 @@ __global__ void __launch_bounds__(BLOCK) k_sweep_dense_ldg(Params p) {
             const uint8_t was = p.rowflag[ridx];
             if (p.E != nullptr && outer) outer &= ~p.E[widx];
             const uint32_t band = inner | outer;
-            const int xlane = (c0 + 1) * 32 + lane;
-            const double *drow = p.data + (long long)un.zl * p.plane_vox + (long long)y * p.X + xlane;
             uint32_t D = 0;
-            constexpr int U = 10;
+            if (CACHED) {
+                if (band) D = p.Dc[widx];  // F = band & (D ^ s) ignores D elsewhere (band = 0 on inactive lanes)
+            } else {
+                const int xlane = (c0 + 1) * 32 + lane;
+                const double *drow = p.data + (long long)un.zl * p.plane_vox + (long long)y * p.X + xlane;
+                constexpr int U = 10;
 #pragma unroll
-            for (int jb = 0; jb < WORDS_PER_WARP; jb += U) {
-                if (jb >= p.segw || c0 + 1 + jb >= p.XW) break;  // warp-uniform
-                double v[U];
+                for (int jb = 0; jb < WORDS_PER_WARP; jb += U) {
+                    if (jb >= p.segw || c0 + 1 + jb >= p.XW) break;  // warp-uniform
+                    double v[U];
 #pragma unroll
-                for (int k = 0; k < U; ++k) v[k] = (xlane + (jb + k) * 32 < p.X) ? drow[(jb + k) * 32] : p.lev0;
+                    for (int k = 0; k < U; ++k) v[k] = (xlane + (jb + k) * 32 < p.X) ? drow[(jb + k) * 32] : p.lev0;
 #pragma unroll
-                for (int k = 0; k < U; ++k) {
-                    const int l = level_of<LATTICE>(p, v[k]);
-                    const unsigned word = __ballot_sync(FULL, (s_dbits[l >> 5] >> (l & 31)) & 1u);
-                    if (lane == jb + k + 1) D = word;
+                    for (int k = 0; k < U; ++k) {
+                        const int l = level_of<LATTICE>(p, v[k]);
+                        const unsigned word = __ballot_sync(FULL, (s_dbits[l >> 5] >> (l & 31)) & 1u);
+                        if (lane == jb + k + 1) D = word;
+                    }
                 }
+                if (p.Dc != nullptr && st.active) p.Dc[widx] = D;
             }
             const uint32_t f = band & (D ^ s);
             store_flips(p, widx, ridx, was, f, st.active, own, lane);
@@ -741,6 +765,22 @@ __global__ void __launch_bounds__(BLOCK) k_sweep_dense_ldg(Params p) {
     }
     flips = warp_sum(flips);
     if (lane == 0 && flips) atomicAdd((unsigned long long *)&p.lstats[2 * p.L + ST_N_FLIPS], (unsigned long long)flips);
+}
+template <bool LATTICE>
+__global__ void __launch_bounds__(BLOCK) k_sweep_dense_ldg(Params p) {
+    if (p.ctrl[C_STATUS] != RUNNING || !dense_refresh(p)) return;
+    count_refresh(p);
+    extern __shared__ uint32_t s_dbits[];
+    for (int i = threadIdx.x; i < p.LW; i += BLOCK) s_dbits[i] = table_bits(p)[i];
+    __syncthreads();
+    sweep_dense_ldg_body<LATTICE, false>(p, s_dbits);
+}
+// The cached sweep, for every shape the refresh kernels serve: streams S (and E, row flags), plus the Dc words under the band.
+// Its blocks leave room on the SMs for the statistics / table kernels of the pipelined run (vrg_tail.cuh): no shared memory,
+// and the register count stays far below k_sweep_dense_slim's 96.
+__global__ void __launch_bounds__(BLOCK, 4) k_sweep_dense_cached(Params p) {
+    if (p.ctrl[C_STATUS] != RUNNING || dense_refresh(p)) return;
+    sweep_dense_ldg_body<false, true>(p, nullptr);
 }
 
 // ---------------------------------------------------------------------------------------------

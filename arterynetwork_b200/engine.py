@@ -122,9 +122,12 @@ class VRGEngine:
         nat.check(self.lib.vrg_poll(self._h, ctypes.byref(r)))
         return self._res(r)
 
-    @staticmethod
-    def _res(r):
-        return {k: int(getattr(r, k)) for k, _ in nat.Result._fields_}
+    def _res(self, r):
+        out = {k: int(getattr(r, k)) for k, _ in nat.Result._fields_}
+        n = nat.i64(0)
+        nat.check(self.lib.vrg_dense_refresh_sweeps(self._h, ctypes.byref(n)))
+        out["dense_refresh_sweeps"] = int(n.value)  # f64_dense: sweeps that read the intensities (the rest read the kept bits)
+        return out
 
     def enqueue_decide(self):
         nat.check(self.lib.vrg_enqueue_decide(self._h))

@@ -141,6 +141,12 @@ int vrg_enqueue_absorb(vrg_handle *h);  /* 4->3 absorption (VRG:167-168,177-179)
 int vrg_enqueue_flip(vrg_handle *h);    /* segmented ^= executed flips (VRG:173,201) */
 int vrg_enqueue_advance(vrg_handle *h); /* exit tests + trace row (VRG:91-117) */
 int vrg_poll(vrg_handle *h, vrg_result *res); /* synchronises the stream */
+/* VRG_INTENSITY_F64_DENSE, as of the last vrg_poll / vrg_run / vrg_apply_flips: sweeps since vrg_init that evaluated every
+ * voxel's decision from its intensity (the first sweep of a run, and each sweep behind a changed decision table or
+ * caller-chosen flips); every other sweep takes the decisions from the bit-plane the last such sweep kept.  With the
+ * environment switch VRG_NO_DCACHE=1 (read by vrg_create) every sweep is one.  0 in the other modes.  (Not a field of
+ * vrg_result: callers allocate that struct, so its size stays as it is.) */
+int vrg_dense_refresh_sweeps(vrg_handle *h, int64_t *n);
 /* One update() call with caller-chosen flips, VRG:124,156-259 (flipedPoints given): coords = n rows of global (z, y, x).
  * Listed voxels that are in neither band are ignored; the band state machine (cancel rule, absorption, region statistics)
  * is applied once and the decision table of the NEW state is computed (vrg_get_table).  Whole-volume handles only. */
