@@ -61,6 +61,7 @@ _SIGS = {
     "vrg_upload_value_map": [vp, vp],
     "vrg_attach_device": [vp, vp, vp],
     "vrg_attach_device_typed": [vp, vp, vp, ctypes.c_int32],
+    "vrg_attach_state_typed": [vp, vp, vp, ctypes.c_int32, vp, ctypes.c_int32],
     "vrg_scan_levels": [vp, ctypes.POINTER(i64)],
     "vrg_get_levels": [vp, vp, i64],
     "vrg_set_levels": [vp, vp, i64],
@@ -74,6 +75,7 @@ _SIGS = {
     "vrg_poll": [vp, ctypes.POINTER(Result)],
     "vrg_dense_refresh_sweeps": [vp, ctypes.POINTER(i64)],
     "vrg_apply_flips": [vp, vp, i64, ctypes.POINTER(Result)],
+    "vrg_apply_flips_device": [vp, vp, i64, ctypes.POINTER(Result)],
     "vrg_enqueue_table": [vp],
     "vrg_p2p_connect_local": [ctypes.POINTER(vp), ctypes.c_int],
     "vrg_labels_hash": [vp, ctypes.POINTER(ctypes.c_uint64)],
@@ -97,6 +99,8 @@ _SIGS = {
     "vrg_labels_device": [vp, vp],
     "vrg_labels_device_typed": [vp, vp, ctypes.c_int32, ctypes.c_int32],
     "vrg_segmented_device": [vp, vp, i64, ctypes.POINTER(i64)],
+    "vrg_band_rows_device": [vp, ctypes.c_int32, vp, i64, ctypes.POINTER(i64)],
+    "vrg_band_sums_device": [vp, vp, vp],
     "vrg_download_segmented": [vp, vp, i64, ctypes.POINTER(i64)],
     "vrg_get_trace": [vp, vp, i64, ctypes.POINTER(i64)],
     "vrg_get_table": [vp, vp, vp, i64],

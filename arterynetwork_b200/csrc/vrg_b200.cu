@@ -444,6 +444,51 @@ int vrg_attach_device_typed(vrg_handle *h, const double *data_dev, const void *v
     h->inited = false;
     return VRG_OK;
 }
+template <typename T>
+static void launch_state(vrg_handle *h, const void *map, long long n, int seg_pass) {
+    const long long off = (long long)h->p.valid_lo * h->p.plane_vox;
+    k_state_from_map<T><<<h->grid, BLOCK, 0, h->stream>>>((const T *)map, h->d_vm + off, n, seg_pass);
+    h->launches++;
+}
+static int state_pass(vrg_handle *h, const void *map, int dtype, int seg_pass) {
+    const long long n = (long long)(h->p.valid_hi - h->p.valid_lo) * h->p.plane_vox;
+    switch (dtype) {
+        case VRG_DTYPE_I8: launch_state<int8_t>(h, map, n, seg_pass); break;
+        case VRG_DTYPE_I16: launch_state<int16_t>(h, map, n, seg_pass); break;
+        case VRG_DTYPE_I32: launch_state<int32_t>(h, map, n, seg_pass); break;
+        case VRG_DTYPE_I64: launch_state<int64_t>(h, map, n, seg_pass); break;
+        case VRG_DTYPE_F32: launch_state<float>(h, map, n, seg_pass); break;
+        case VRG_DTYPE_F64: launch_state<double>(h, map, n, seg_pass); break;
+        default: launch_state<uint8_t>(h, map, n, seg_pass); break;
+    }
+    CK(cudaGetLastError());
+    return VRG_OK;
+}
+// update()'s inputs on the device: the intensities attached zero-copy, the state built into the handle's own uint8 valueMap
+// from segmentedMap (== 1: segmented) and valueMap (== 4: excluded), each read in its own dtype
+int vrg_attach_state_typed(vrg_handle *h, const double *data_dev, const void *seg_dev, int32_t seg_dtype, const void *vm_dev,
+                           int32_t vm_dtype) {
+    if (!h || !data_dev || !seg_dev || !vm_dev) return fail(VRG_ERR_ARG, "null argument");
+    const size_t es = dtype_size(seg_dtype), ev = dtype_size(vm_dtype);
+    if (!es || !ev) return fail(VRG_ERR_ARG, "unknown map dtype %d / %d", (int)seg_dtype, (int)vm_dtype);
+    if ((uintptr_t)seg_dev % es || (uintptr_t)vm_dev % ev) return fail(VRG_ERR_ARG, "map buffer not aligned to its element size");
+    CK(cudaSetDevice(h->cfg.device));
+    Params &p = h->p;
+    if (!h->d_vm) {
+        CK(big_alloc(h, (void **)&h->d_vm, (size_t)p.nzl * p.plane_vox));
+        CK(cudaMemsetAsync(h->d_vm, 3, (size_t)p.nzl * p.plane_vox, h->stream));
+    }
+    { int rc_ = state_pass(h, vm_dev, vm_dtype, 0); if (rc_ != VRG_OK) return rc_; }
+    { int rc_ = state_pass(h, seg_dev, seg_dtype, 1); if (rc_ != VRG_OK) return rc_; }
+    p.data = (const double *)((uintptr_t)data_dev - (uintptr_t)p.valid_lo * p.plane_vox * sizeof(double));
+    h->vm_base = h->d_vm;
+    h->vm_dtype = VRG_DTYPE_U8;
+    h->attached = true;
+    h->have_data = true;
+    h->have_levels = false;
+    h->inited = false;
+    return VRG_OK;
+}
 int vrg_upload_value_map(vrg_handle *h, const uint8_t *vm) {
     if (!vm) return fail(VRG_ERR_ARG, "null buffer");
     int rc = upload_impl(h, nullptr, vm, cudaMemcpyHostToDevice);
@@ -1415,22 +1460,19 @@ int vrg_run(vrg_handle *h, vrg_result *res) {
 }
 
 // ---- update() with caller-chosen flips (VRG:124, flipedPoints given) -----------------------------------------
-int vrg_apply_flips(vrg_handle *h, const int64_t *coords, int64_t n, vrg_result *res) {
-    NEED_INIT();
+static int flips_args(vrg_handle *h, const void *coords, int64_t n) {
     if (n < 0 || (n > 0 && !coords)) return fail(VRG_ERR_ARG, "bad flip list");
     const Params &p = h->p;
     if (h->cfg.intensity_mode == VRG_INTENSITY_CONTINUOUS) return fail(VRG_ERR_ARG, "vrg_apply_flips needs a level-table mode");
     if (h->p2p_on || p.valid_lo != p.own_lo || p.valid_hi != p.own_hi) return fail(VRG_ERR_ARG, "vrg_apply_flips runs on a whole-volume handle");
-    for (int64_t i = 0; i < n; ++i) {
-        const int64_t z = coords[3 * i], y = coords[3 * i + 1], x = coords[3 * i + 2];
-        if (z < h->cfg.z_begin || z >= h->cfg.z_end || y < 0 || y >= p.Y || x < 0 || x >= p.X)
-            return fail(VRG_ERR_ARG, "flip %lld = (%lld, %lld, %lld) lies outside the volume", (long long)i, (long long)z, (long long)y, (long long)x);
-    }
-    long long *d_coords = nullptr;
-    if (n) {
-        CK(cudaMalloc((void **)&d_coords, (size_t)n * 3 * sizeof(long long)));
-        CK(cudaMemcpyAsync(d_coords, coords, (size_t)n * 3 * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
-    }
+    return VRG_OK;
+}
+static int fail_flip_outside(int64_t i, int64_t z, int64_t y, int64_t x) {
+    return fail(VRG_ERR_ARG, "flip %lld = (%lld, %lld, %lld) lies outside the volume", (long long)i, (long long)z, (long long)y, (long long)x);
+}
+// the band state machine on validated device rows (n may be 0)
+static int apply_flips_rows(vrg_handle *h, const long long *d_coords, int64_t n, vrg_result *res) {
+    const Params &p = h->p;
     CK(cudaMemsetAsync(h->d_F, 0, h->plane_bytes, h->stream));
     CK(cudaMemsetAsync(h->d_C, 0, h->plane_bytes, h->stream));
     CK(cudaMemsetAsync(h->d_rowflag, 0, h->rowflag_bytes, h->stream));
@@ -1449,8 +1491,49 @@ int vrg_apply_flips(vrg_handle *h, const int64_t *coords, int64_t n, vrg_result 
         h->launches++;
         rc = vrg_poll(h, res);
     }
+    return rc;
+}
+int vrg_apply_flips(vrg_handle *h, const int64_t *coords, int64_t n, vrg_result *res) {
+    NEED_INIT();
+    { int rc_ = flips_args(h, coords, n); if (rc_ != VRG_OK) return rc_; }
+    const Params &p = h->p;
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t z = coords[3 * i], y = coords[3 * i + 1], x = coords[3 * i + 2];
+        if (z < h->cfg.z_begin || z >= h->cfg.z_end || y < 0 || y >= p.Y || x < 0 || x >= p.X) return fail_flip_outside(i, z, y, x);
+    }
+    long long *d_coords = nullptr;
+    if (n) {
+        CK(cudaMalloc((void **)&d_coords, (size_t)n * 3 * sizeof(long long)));
+        CK(cudaMemcpyAsync(d_coords, coords, (size_t)n * 3 * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
+    }
+    const int rc = apply_flips_rows(h, d_coords, n, res);
     if (d_coords) { cudaStreamSynchronize(h->stream); cudaFree(d_coords); }
     return rc;
+}
+// the same with the rows in device memory: validated on the device (one synchronisation for the verdict) before anything changes
+int vrg_apply_flips_device(vrg_handle *h, const int64_t *rows_dev, int64_t n, vrg_result *res) {
+    NEED_INIT();
+    { int rc_ = flips_args(h, rows_dev, n); if (rc_ != VRG_OK) return rc_; }
+    if ((uintptr_t)rows_dev % sizeof(int64_t)) return fail(VRG_ERR_ARG, "flip rows not aligned to 8 bytes");
+    const long long *d_coords = (const long long *)rows_dev;
+    if (n) {
+        unsigned long long *d_out = (unsigned long long *)h->d_hcount;  // 16 bytes of scratch: count, first row outside
+        CK(cudaMemsetAsync(d_out, 0, sizeof(unsigned long long), h->stream));
+        CK(cudaMemsetAsync(d_out + 1, 0xFF, sizeof(unsigned long long), h->stream));
+        const long long blocks = std::min<long long>(h->grid, (n + BLOCK - 1) / BLOCK);
+        k_check_flips<<<(int)blocks, BLOCK, 0, h->stream>>>(h->p, d_coords, n, h->cfg.z_begin, d_out);
+        h->launches++;
+        CK(cudaGetLastError());
+        unsigned long long v[2];
+        CK(cudaMemcpyAsync(v, d_out, sizeof v, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        if (v[0]) {
+            long long r[3];
+            CK(cudaMemcpy(r, d_coords + 3 * v[1], sizeof r, cudaMemcpyDeviceToHost));
+            return fail_flip_outside((int64_t)v[1], r[0], r[1], r[2]);
+        }
+    }
+    return apply_flips_rows(h, d_coords, n, res);
 }
 
 // FNV-1a over the kernel parameter block: a host that replays captured launches (CUDA graphs) re-captures when it moves
@@ -1701,38 +1784,62 @@ int vrg_download_segmented(vrg_handle *h, int64_t *coords, int64_t cap, int64_t 
     return VRG_OK;
 }
 
-// the same rows compacted on the device: per-row popcounts, an exclusive scan (CUB), a scatter of the triples.  The count
-// travels to the host (the one synchronisation); rows beyond `cap` are not written.
-int vrg_segmented_device(vrg_handle *h, int64_t *rows_dev, int64_t cap, int64_t *n_out) {
+template <int WHICH>
+static cudaError_t launch_rows(vrg_handle *h, long long *counts, const long long *offs, int64_t *rows_dev, int64_t cap) {
+    if (counts) k_seg_count<WHICH><<<h->grid, BLOCK, 0, h->stream>>>(h->p, counts);
+    else k_seg_scatter<WHICH><<<h->grid, BLOCK, 0, h->stream>>>(h->p, offs, (long long *)rows_dev, (long long)cap,
+                                                                  (long long)h->cfg.z_begin);
+    return cudaGetLastError();
+}
+static cudaError_t launch_rows(vrg_handle *h, int which, long long *counts, const long long *offs, int64_t *rows_dev, int64_t cap) {
+    if (which == 1) return launch_rows<1>(h, counts, offs, rows_dev, cap);
+    if (which == 2) return launch_rows<2>(h, counts, offs, rows_dev, cap);
+    return launch_rows<0>(h, counts, offs, rows_dev, cap);
+}
+// the rows of the segmented voxels (which = 0), the inner band (1) or the outer band (2), compacted on the device: popcounts per
+// row segment, an exclusive scan (CUB), a scatter of the triples.  The count travels to the host (the one synchronisation); rows
+// beyond `cap` are not written.
+int vrg_band_rows_device(vrg_handle *h, int32_t which, int64_t *rows_dev, int64_t cap, int64_t *n_out) {
     NEED_INIT();
-    if (!n_out) return fail(VRG_ERR_ARG, "null argument");
+    if (!n_out || which < 0 || which > 2) return fail(VRG_ERR_ARG, "bad argument");
+    if (rows_dev && (uintptr_t)rows_dev % sizeof(int64_t)) return fail(VRG_ERR_ARG, "rows buffer not aligned to 8 bytes");
     const Params &p = h->p;
-    const long long nrows_ll = (long long)h->nz_own * p.Y;
-    if (nrows_ll >= (1LL << 31) - 1) return fail(VRG_ERR_ARG, "too many rows for the device compaction");
-    const int nrows = (int)nrows_ll;
+    const long long nslots_ll = (long long)h->nz_own * p.Y * p.nseg;
+    if (nslots_ll >= (1LL << 31) - 1) return fail(VRG_ERR_ARG, "too many rows for the device compaction");
+    const int nslots = (int)nslots_ll;
     size_t tmp_bytes = 0;
-    CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, (const long long *)nullptr, (long long *)nullptr, nrows + 1, h->stream));
-    const size_t cnt_bytes = ((size_t)(nrows + 1) * sizeof(long long) + 255) & ~(size_t)255;
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, (const long long *)nullptr, (long long *)nullptr, nslots + 1, h->stream));
+    const size_t cnt_bytes = ((size_t)(nslots + 1) * sizeof(long long) + 255) & ~(size_t)255;
     char *buf = nullptr;
     CK(big_alloc(h, (void **)&buf, 2 * cnt_bytes + tmp_bytes));
     long long *counts = (long long *)buf, *offs = (long long *)(buf + cnt_bytes);
-    cudaError_t e = cudaMemsetAsync(counts + nrows, 0, sizeof(long long), h->stream);
-    if (e == cudaSuccess) {
-        k_seg_count<<<h->grid, BLOCK, 0, h->stream>>>(p, counts, nrows);
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cub::DeviceScan::ExclusiveSum(buf + 2 * cnt_bytes, tmp_bytes, counts, offs, nrows + 1, h->stream);
-    if (e == cudaSuccess && rows_dev && cap > 0) {
-        k_seg_scatter<<<h->grid, BLOCK, 0, h->stream>>>(p, offs, nrows, (long long *)rows_dev, (long long)cap, (long long)h->cfg.z_begin);
-        e = cudaGetLastError();
-    }
+    cudaError_t e = cudaMemsetAsync(counts + nslots, 0, sizeof(long long), h->stream);
+    if (e == cudaSuccess) e = launch_rows(h, which, counts, nullptr, nullptr, 0);
+    if (e == cudaSuccess) e = cub::DeviceScan::ExclusiveSum(buf + 2 * cnt_bytes, tmp_bytes, counts, offs, nslots + 1, h->stream);
+    if (e == cudaSuccess && rows_dev && cap > 0) e = launch_rows(h, which, nullptr, offs, rows_dev, cap);
     long long n = 0;
-    if (e == cudaSuccess) e = cudaMemcpyAsync(&n, offs + nrows, sizeof n, cudaMemcpyDeviceToHost, h->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&n, offs + nslots, sizeof n, cudaMemcpyDeviceToHost, h->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
     cudaFreeAsync(buf, h->stream);
-    if (e != cudaSuccess) return fail(VRG_ERR_CUDA, "segmented rows on the device: %s", cudaGetErrorString(e));
+    if (e != cudaSuccess) return fail(VRG_ERR_CUDA, "band rows on the device: %s", cudaGetErrorString(e));
     h->launches += 2 + (rows_dev && cap > 0);
     *n_out = n;
+    return VRG_OK;
+}
+int vrg_segmented_device(vrg_handle *h, int64_t *rows_dev, int64_t cap, int64_t *n_out) {
+    return vrg_band_rows_device(h, 0, rows_dev, cap, n_out);
+}
+
+// update()'s Parzen sum volumes of the current table (k_band_sums_dense), own planes, on the handle's stream (no synchronisation)
+int vrg_band_sums_device(vrg_handle *h, double *pin_dev, double *pout_dev) {
+    NEED_INIT();
+    if (!pin_dev || !pout_dev) return fail(VRG_ERR_ARG, "null buffer");
+    if ((uintptr_t)pin_dev % sizeof(double) || (uintptr_t)pout_dev % sizeof(double)) return fail(VRG_ERR_ARG, "sum buffers not aligned to 8 bytes");
+    if (h->cfg.intensity_mode == VRG_INTENSITY_CONTINUOUS) return fail(VRG_ERR_ARG, "vrg_band_sums_device needs a level-table mode");
+    if (h->p.lattice) k_band_sums_dense<true><<<h->grid, BLOCK, 0, h->stream>>>(h->p, pin_dev, pout_dev);
+    else k_band_sums_dense<false><<<h->grid, BLOCK, 0, h->stream>>>(h->p, pin_dev, pout_dev);
+    h->launches++;
+    CK(cudaGetLastError());
     return VRG_OK;
 }
 

@@ -1737,29 +1737,63 @@ __global__ void __launch_bounds__(BLOCK) k_labels(Params p, T *__restrict__ out,
     }
 }
 
-// segmented rows on the device (vrg_segmented_device): popcount of every own-plane row of S, one warp per row ...
-__global__ void __launch_bounds__(BLOCK) k_seg_count(Params p, long long *__restrict__ counts, int nrows) {
-    const int lane = threadIdx.x & 31;
-    for (int r = blockIdx.x * WARPS + (threadIdx.x >> 5); r < nrows; r += gridDim.x * WARPS) {
-        const uint32_t *row = p.S + (long long)(p.own_lo + r / p.Y) * p.plane_words + (long long)(r % p.Y) * p.WP;
-        long long n = 0;
-        for (int c = lane; c < p.XW; c += 32) n += __popc(row[c]);
-        n = warp_sum(n);
-        if (lane == 0) counts[r] = n;
+// Row compaction on the device (vrg_band_rows_device).  A warp walks a unit (ROWS_PER_UNIT rows of one row segment, the
+// Strip layout: lanes 1..segw hold the segment's words) and takes from each row the word that WHICH selects:
+//   0  S, the segmented voxels                  1  the inner band S & dil26(~S)  (label 1)
+//   2  the outer band ~S & ~E & dil26(S)  (label 2)
+// -- the bands derived as k_labels derives them.  Every lane outside 1..segw, or beyond the row, holds 0.
+template <int WHICH>
+__device__ __forceinline__ uint32_t row_word(const Params &p, Strip &st, int zl, int y, int c, int lane) {
+    if constexpr (WHICH == 0) {
+        const bool active = c >= 0 && c < p.XW && lane >= 1 && lane <= p.segw;
+        return active ? p.S[(long long)zl * p.plane_words + (long long)y * p.WP + c] : 0u;
+    } else {
+        uint32_t s, inner, outer;
+        st.step(p, y, s, inner, outer);
+        if constexpr (WHICH == 1) return inner;
+        const uint32_t e = (p.E && st.active) ? p.E[(long long)zl * p.plane_words + (long long)y * p.WP + c] : 0u;
+        return outer & ~e;
     }
 }
-// ... and, behind an exclusive scan of those counts, the (z, y, x) triples of the row's set bits in C order, z_begin added.
-// A warp takes 32 words of the row at a time; a warp scan of their popcounts gives each lane its first output row.
-__global__ void __launch_bounds__(BLOCK) k_seg_scatter(Params p, const long long *__restrict__ offs, int nrows,
-                                                       long long *__restrict__ rows, long long cap, long long z_begin) {
+// slot of a row segment of the own planes: (row, segment) in C order, so that the scanned counts give C-ordered rows
+__device__ __forceinline__ long long row_slot(const Params &p, int zl, int y, int sg) {
+    return ((long long)(zl - p.own_lo) * p.Y + y) * p.nseg + sg;
+}
+// popcount of every own-plane row segment's selected words ...
+template <int WHICH>
+__global__ void __launch_bounds__(BLOCK) k_seg_count(Params p, long long *__restrict__ counts) {
     const int lane = threadIdx.x & 31;
-    for (int r = blockIdx.x * WARPS + (threadIdx.x >> 5); r < nrows; r += gridDim.x * WARPS) {
-        const int zl = r / p.Y, y = r % p.Y;
-        const uint32_t *row = p.S + (long long)(p.own_lo + zl) * p.plane_words + (long long)y * p.WP;
-        long long base = offs[r];
-        for (int c0 = 0; c0 < p.XW; c0 += 32) {
-            const int c = c0 + lane;
-            uint32_t w = c < p.XW ? row[c] : 0u;
+    const int nyb = (p.Y + ROWS_PER_UNIT - 1) / ROWS_PER_UNIT;
+    const long long nunits = (long long)(p.own_hi - p.own_lo) * nyb * p.nseg;
+    const long long nwarps = (long long)gridDim.x * WARPS;
+    Strip st;
+    for (long long u = (long long)blockIdx.x * WARPS + (threadIdx.x >> 5); u < nunits; u += nwarps) {
+        const Unit un = decode_unit(p, u, p.own_lo, nyb);
+        const int c = un.sg * p.segw - 1 + lane;
+        if (WHICH) st.begin(p, un.zl, un.y0, c, lane);
+        for (int y = un.y0; y < un.y1; ++y) {
+            const long long n = warp_sum(__popc(row_word<WHICH>(p, st, un.zl, y, c, lane)));
+            if (lane == 0) counts[row_slot(p, un.zl, y, un.sg)] = n;
+        }
+    }
+}
+// ... and, behind an exclusive scan of those counts, the (z, y, x) triples of the set bits in C order, z_begin added: a warp
+// scan of the lanes' popcounts gives each lane its first output row.  Rows from `cap` on are not written.
+template <int WHICH>
+__global__ void __launch_bounds__(BLOCK) k_seg_scatter(Params p, const long long *__restrict__ offs, long long *__restrict__ rows,
+                                                       long long cap, long long z_begin) {
+    const int lane = threadIdx.x & 31;
+    const int nyb = (p.Y + ROWS_PER_UNIT - 1) / ROWS_PER_UNIT;
+    const long long nunits = (long long)(p.own_hi - p.own_lo) * nyb * p.nseg;
+    const long long nwarps = (long long)gridDim.x * WARPS;
+    Strip st;
+    for (long long u = (long long)blockIdx.x * WARPS + (threadIdx.x >> 5); u < nunits; u += nwarps) {
+        const Unit un = decode_unit(p, u, p.own_lo, nyb);
+        const int c = un.sg * p.segw - 1 + lane;
+        if (WHICH) st.begin(p, un.zl, un.y0, c, lane);
+        for (int y = un.y0; y < un.y1; ++y) {
+            uint32_t w = row_word<WHICH>(p, st, un.zl, y, c, lane);
+            if (__ballot_sync(FULL, w != 0u) == 0u) continue;
             const int n = __popc(w);
             int incl = n;
 #pragma unroll
@@ -1767,19 +1801,73 @@ __global__ void __launch_bounds__(BLOCK) k_seg_scatter(Params p, const long long
                 const int t = __shfl_up_sync(FULL, incl, o);
                 if (lane >= o) incl += t;
             }
-            long long k = base + incl - n;
+            long long k = offs[row_slot(p, un.zl, y, un.sg)] + incl - n;
             while (w) {
                 const int b = __ffs(w) - 1;
                 w &= w - 1;
                 if (k < cap) {
-                    rows[3 * k] = z_begin + zl;
+                    rows[3 * k] = z_begin + (un.zl - p.own_lo);
                     rows[3 * k + 1] = y;
                     rows[3 * k + 2] = (long long)c * 32 + b;
                 }
                 ++k;
             }
-            base += __shfl_sync(FULL, incl, 31);
         }
+    }
+}
+
+// update()'s two Parzen sum volumes (VRG:132-133,151-155 as the host path writes them), own planes, C order: at every inner /
+// outer band voxel pin * n_in and pout * n_out of its level in the current decision table (one rounding each, as NumPy's
+// pin[idx] * n_in), 0.0 everywhere else.  The level comes from the sweep's lookup (level_of); intensities are read at band
+// voxels only.  A warp writes the 32 voxels of one word per store into each volume (2 x 256 consecutive bytes).
+template <bool LATTICE>
+__global__ void __launch_bounds__(BLOCK) k_band_sums_dense(Params p, double *__restrict__ pin_out, double *__restrict__ pout_out) {
+    const int lane = threadIdx.x & 31;
+    const int nyb = (p.Y + ROWS_PER_UNIT - 1) / ROWS_PER_UNIT;
+    const long long nunits = (long long)(p.own_hi - p.own_lo) * nyb * p.nseg;
+    const long long nwarps = (long long)gridDim.x * WARPS;
+    const double n_in = (double)p.gstats[2 * p.L + ST_N_IN], n_out = (double)p.gstats[2 * p.L + ST_N_OUT];
+    const uint32_t bit = 1u << lane;
+    Strip st;
+    for (long long u = (long long)blockIdx.x * WARPS + (threadIdx.x >> 5); u < nunits; u += nwarps) {
+        const Unit un = decode_unit(p, u, p.own_lo, nyb);
+        const int c0 = un.sg * p.segw - 1, c = c0 + lane;
+        st.begin(p, un.zl, un.y0, c, lane);
+        for (int y = un.y0; y < un.y1; ++y) {
+            uint32_t s, inner, outer;
+            st.step(p, y, s, inner, outer);
+            const uint32_t e = (p.E && st.active) ? p.E[(long long)un.zl * p.plane_words + (long long)y * p.WP + c] : 0u;
+            const uint32_t band = inner | (outer & ~e);
+            const double *rowin = p.data + ((long long)un.zl * p.Y + y) * p.X;
+            const long long rowout = ((long long)(un.zl - p.own_lo) * p.Y + y) * p.X;
+            for (int j = 1; j <= p.segw; ++j) {
+                if (c0 + j >= p.XW) break;
+                const uint32_t bj = __shfl_sync(FULL, band, j);
+                const int x = (c0 + j) * 32 + lane;
+                if (x >= p.X) continue;
+                double a = 0.0, b = 0.0;
+                if (bj & bit) {
+                    const int l = level_of<LATTICE>(p, rowin[x]);
+                    a = p.pin[l] * n_in;
+                    b = p.pout[l] * n_out;
+                }
+                pin_out[rowout + x] = a;
+                pout_out[rowout + x] = b;
+            }
+        }
+    }
+}
+
+// update()'s state from the caller's two maps, each read in its own dtype, into the handle's uint8 valueMap (local planes):
+// the valueMap pass writes 4 where valueMap == 4 and 3 elsewhere, the segmentedMap pass then 0 where segmentedMap == 1
+// (VRG:124: what the host update() reads of its inputs).  vrg_init takes the result as any uint8 map.
+template <typename T>
+__global__ void __launch_bounds__(BLOCK) k_state_from_map(const T *__restrict__ map, uint8_t *__restrict__ vm, long long n,
+                                                          int seg_pass) {
+    for (long long i = (long long)blockIdx.x * BLOCK + threadIdx.x; i < n; i += (long long)gridDim.x * BLOCK) {
+        const T v = map[i];
+        if (!seg_pass) vm[i] = v == T(4) ? 4 : 3;
+        else if (v == T(1)) vm[i] = 0;
     }
 }
 
@@ -1812,6 +1900,21 @@ __global__ void __launch_bounds__(BLOCK) k_expand_i64(const uint8_t *__restrict_
 }
 
 // ---------------------------------------------------------------------------------------------
+// device-resident flip rows (vrg_apply_flips_device): out[0] = how many lie outside the own planes, out[1] = the first of them
+// (the caller sets it to ~0 beforehand)
+__global__ void __launch_bounds__(BLOCK) k_check_flips(Params p, const long long *__restrict__ coords, long long n, long long z_begin,
+                                                       unsigned long long *out) {
+    unsigned long long bad = 0;
+    for (long long i = (long long)blockIdx.x * BLOCK + threadIdx.x; i < n; i += (long long)gridDim.x * BLOCK) {
+        const long long z = coords[3 * i] - z_begin + p.own_lo, y = coords[3 * i + 1], x = coords[3 * i + 2];
+        if (z < p.own_lo || z >= p.own_hi || y < 0 || y >= p.Y || x < 0 || x >= p.X) {
+            ++bad;
+            atomicMin(&out[1], (unsigned long long)i);
+        }
+    }
+    if (bad) atomicAdd(&out[0], bad);
+}
+
 // update() with caller-chosen flips (VRG:124, flipedPoints given): the listed voxels' bits go into F ...
 __global__ void __launch_bounds__(BLOCK) k_set_flips(Params p, const long long *__restrict__ coords, long long n, long long z_begin) {
     for (long long i = (long long)blockIdx.x * BLOCK + threadIdx.x; i < n; i += (long long)gridDim.x * BLOCK) {

@@ -96,6 +96,12 @@ class VRGEngine:
         """Zero-copy like ``attach_device``, the valueMap in its own dtype (``nat.DTYPE_*``): vrg_init reads it as it is."""
         nat.check(self.lib.vrg_attach_device_typed(self._h, nat.vp(data_ptr), nat.vp(value_map_ptr), int(value_map_dtype)))
 
+    def attach_state_typed(self, data_ptr: int, seg_map_ptr: int, seg_map_dtype: int, value_map_ptr: int, value_map_dtype: int):
+        """update()'s inputs on the device: fp64 data attached zero-copy, the state built from segmentedMap (== 1) and valueMap
+        (== 4), each in its own dtype (``nat.DTYPE_*``), into the handle's own map on its stream."""
+        nat.check(self.lib.vrg_attach_state_typed(self._h, nat.vp(data_ptr), nat.vp(seg_map_ptr), int(seg_map_dtype),
+                                                  nat.vp(value_map_ptr), int(value_map_dtype)))
+
     # -- levels -----------------------------------------------------------------------------
     def scan_levels(self) -> np.ndarray:
         n = nat.i64(0)
@@ -152,6 +158,12 @@ class VRGEngine:
         c = np.ascontiguousarray(coords, dtype=np.int64).reshape(-1, 3)
         r = nat.Result()
         nat.check(self.lib.vrg_apply_flips(self._h, c.ctypes.data if c.size else None, c.shape[0], ctypes.byref(r)))
+        return self._res(r)
+
+    def apply_flips_device(self, rows_ptr, n: int) -> dict:
+        """``apply_flips`` with ``n`` int64 rows (z, y, x) in device memory, checked on the device before anything changes."""
+        r = nat.Result()
+        nat.check(self.lib.vrg_apply_flips_device(self._h, nat.vp(rows_ptr or None), int(n), ctypes.byref(r)))
         return self._res(r)
 
     def profile(self, enable=True):
@@ -244,6 +256,17 @@ class VRGEngine:
         n = nat.i64(0)
         nat.check(self.lib.vrg_segmented_device(self._h, nat.vp(rows_ptr or None), int(cap), ctypes.byref(n)))
         return int(n.value)
+
+    def band_rows_device(self, which: int, rows_ptr, cap: int) -> int:
+        """``segmented_device`` for ``which`` = 0 (segmented), 1 (inner band, label 1) or 2 (outer band, label 2)."""
+        n = nat.i64(0)
+        nat.check(self.lib.vrg_band_rows_device(self._h, int(which), nat.vp(rows_ptr or None), int(cap), ctypes.byref(n)))
+        return int(n.value)
+
+    def band_sums_device(self, pin_ptr: int, pout_ptr: int):
+        """update()'s innerProb / outerProb of the current table into two float64 device buffers of the own planes (C order),
+        on the handle's stream (no synchronisation)."""
+        nat.check(self.lib.vrg_band_sums_device(self._h, nat.vp(pin_ptr), nat.vp(pout_ptr)))
 
     def segmented(self, at_most=None) -> np.ndarray:
         """Rows (z, y, x) of the segmented voxels of the own planes, C order.  ``at_most``: an upper bound of their number

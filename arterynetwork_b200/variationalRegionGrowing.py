@@ -15,6 +15,8 @@ caller's axes; stdout, ``LAST_RUN`` and the warning as below.  Nothing of volume
 are used as they are, F-contiguous ones (``torch.from_numpy(nibabel_volume).cuda()``) through their reversed-axes view,
 other strides through a contiguous copy whose labels are copied back; intensities other than float64 are converted once.
 On any error the caller's ``valueMap`` is left bit-unchanged.  ``DEVICES`` and ``LIST_ORDER = True`` take host arrays only.
+``update`` takes CUDA tensors the same way (see its docstring): state, flips, band rows and Parzen sums stay on the device,
+and the results are bit-identical to the call on host arrays.
 
 Module switches (the reference has none; defaults reproduce it):
 
@@ -253,16 +255,56 @@ def _label_dtype_code(torch, dtype):
             torch.int64: nat.DTYPE_I64, torch.float32: nat.DTYPE_F32, torch.float64: nat.DTYPE_F64}.get(dtype)
 
 
+def _tensor_layout(dataArray):
+    """(reversed axes, transposed?) of a CUDA tensor volume: a nibabel-style F-ordered one is used through its reversed-axes
+    view, as _as_zyx does for ndarrays.  The other tensors of the call are viewed the same way."""
+    nd = dataArray.dim()
+    rev = tuple(range(nd - 1, -1, -1))
+    return rev, nd > 1 and not dataArray.is_contiguous() and dataArray.permute(rev).is_contiguous()
+
+
+def _tensor_data3(torch, dataArray, rev, transposed):
+    """The intensities as a C-contiguous float64 (Z, Y, X) tensor: the caller's own when it already is one, otherwise converted
+    once (processed as float64 whatever the input dtype, like the host path)."""
+    d = dataArray.permute(rev) if transposed else dataArray
+    if d.dtype != torch.float64:
+        d = d.to(torch.float64)
+    return d.contiguous().reshape((1,) * (3 - d.dim()) + tuple(d.shape))
+
+
+def _tensor_work(t, rev, transposed):
+    """(``t`` in (Z, Y, X) axis order, a C-contiguous tensor of it for the kernels): that view itself, or for other strides a
+    copy that the caller writes back on success."""
+    v = t.permute(rev) if transposed else t
+    return v, (v if v.is_contiguous() else v.contiguous())
+
+
+def _tensor_user_rows(torch, rows, shape, transposed):
+    """(n, 3) int64 device rows in C order of (Z, Y, X) -> (n, ndim) rows in C order of the caller's axes (``shape``)."""
+    nd = len(shape)
+    r = rows[:, 3 - nd:]
+    if not transposed:
+        return r.contiguous()
+    r = r.flip(1)
+    key = r[:, 0].clone()
+    for ax in range(1, nd):
+        key = key * shape[ax] + r[:, ax]
+    return r[torch.argsort(key)]
+
+
+def _check_tensor(torch, name, t, like):
+    if not isinstance(t, torch.Tensor) or not t.is_cuda:
+        raise TypeError("valueMap is a CUDA tensor: %s must be a CUDA tensor on the same device, got %s" % (name, type(t).__name__))
+    if t.device != like.device:
+        raise ValueError("%s (%s) and valueMap (%s) are on different devices" % (name, t.device, like.device))
+
+
 def _tensor_run(dataArray, valueMap, H, maxSegmentSize):
     """The call on CUDA tensors: inputs attached where they are (the valueMap in its own dtype), labels written back by the
     kernels in that dtype, segmentedMap and the segmented rows built on the device.  Nothing of volume size crosses PCIe."""
     global LAST_RUN
     import torch
-    if not isinstance(dataArray, torch.Tensor) or not dataArray.is_cuda:
-        raise TypeError("valueMap is a CUDA tensor: dataArray must be a CUDA tensor on the same device, got %s"
-                        % type(dataArray).__name__)
-    if dataArray.device != valueMap.device:
-        raise ValueError("dataArray (%s) and valueMap (%s) are on different devices" % (dataArray.device, valueMap.device))
+    _check_tensor(torch, "dataArray", dataArray, valueMap)
     if tuple(dataArray.shape) != tuple(valueMap.shape):
         raise ValueError("dataArray and valueMap must have the same shape")
     if LIST_ORDER:
@@ -287,17 +329,11 @@ def _tensor_run(dataArray, valueMap, H, maxSegmentSize):
         host_seconds[name] = host_seconds.get(name, 0.0) + now - clock[0]
         clock[0] = now
     dev = valueMap.device
-    rev = tuple(range(nd - 1, -1, -1))
-    # nibabel-style F-ordered volume: used through its reversed-axes view, as _as_zyx does for ndarrays
-    transposed = nd > 1 and not dataArray.is_contiguous() and dataArray.permute(rev).is_contiguous()
+    rev, transposed = _tensor_layout(dataArray)
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev)
-        d = dataArray.permute(rev) if transposed else dataArray
-        if d.dtype != torch.float64:
-            d = d.to(torch.float64)  # processed as float64 whatever the input dtype, like the host path
-        d3 = d.contiguous().reshape((1,) * (3 - nd) + tuple(d.shape))  # (Z, Y, X), C order
-        vm_zyx = valueMap.permute(rev) if transposed else valueMap
-        work = vm_zyx if vm_zyx.is_contiguous() else vm_zyx.contiguous()  # other strides: a copy, written back on success
+        d3 = _tensor_data3(torch, dataArray, rev, transposed)  # (Z, Y, X), C order
+        vm_zyx, work = _tensor_work(valueMap, rev, transposed)
         vm3 = work.reshape(d3.shape)
         lap("prepare_inputs")
 
@@ -336,16 +372,10 @@ def _tensor_run(dataArray, valueMap, H, maxSegmentSize):
             res, rows, nonzero, seg3 = run("continuous")
         if work is not vm_zyx:
             vm_zyx.copy_(work)
-        segmented = rows[:, 3 - nd:]
+        segmented = _tensor_user_rows(torch, rows, tuple(dataArray.shape), transposed)
         if transposed:
-            segmented = segmented.flip(1)
-            key = segmented[:, 0].clone()
-            for ax in range(1, nd):
-                key = key * dataArray.shape[ax] + segmented[:, ax]
-            segmented = segmented[torch.argsort(key)]  # C order of the user's axes
-            segmentedMap = seg3.reshape(d.shape).permute(rev).contiguous()
+            segmentedMap = seg3.reshape(d3.shape[3 - nd:]).permute(rev).contiguous()
         else:
-            segmented = segmented.contiguous()
             segmentedMap = seg3.reshape(dataArray.shape)
         lap("user_layout")
     LAST_RUN = dict(res)
@@ -451,6 +481,91 @@ def variationalRegionGrowing(dataArray, valueMap, H=2.25, maxSegmentSize=5000):
     return segmented, segmentedMap, valueMap
 
 
+def _tensor_update(dataArray, segmented, segmentedMap, valueMap, H, flipedPoints, innerProb, outerProb):
+    """update() on CUDA tensors: the state read from the caller's maps where they are, the flips, the band rows and the Parzen
+    sum volumes on the device, on torch's current stream.  Nothing of volume size crosses PCIe."""
+    import torch
+    _check_tensor(torch, "dataArray", dataArray, valueMap)
+    _check_tensor(torch, "segmentedMap", segmentedMap, valueMap)
+    shape = tuple(dataArray.shape)
+    if shape != tuple(valueMap.shape) or shape != tuple(segmentedMap.shape):
+        raise ValueError("dataArray, segmentedMap and valueMap must have the same shape")
+    new_prob = innerProb is None or outerProb is None
+    if not new_prob:
+        for name, t in (("innerProb", innerProb), ("outerProb", outerProb)):
+            _check_tensor(torch, name, t, valueMap)
+            if t.dtype != torch.float64:
+                raise TypeError("%s must be a float64 CUDA tensor, got %s" % (name, t.dtype))
+            if tuple(t.shape) != shape:
+                raise ValueError("%s must have the shape of dataArray" % name)
+    nd = dataArray.dim()
+    if nd > 3 or nd == 0:
+        raise NotImplementedError("update: 1-D to 3-D volumes only, got ndim=%d" % nd)
+    seg_code, vm_code = _label_dtype_code(torch, segmentedMap.dtype), _label_dtype_code(torch, valueMap.dtype)
+    if seg_code is None or vm_code is None:
+        raise TypeError("segmentedMap / valueMap dtype %s / %s: uint8, int8, int16, int32, int64, float32 or float64 only"
+                        % (segmentedMap.dtype, valueMap.dtype))
+    if dataArray.is_complex():
+        raise TypeError("dataArray must hold real intensities, got %s" % dataArray.dtype)
+    dev = valueMap.device
+    rev, transposed = _tensor_layout(dataArray)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev)
+        d3 = _tensor_data3(torch, dataArray, rev, transposed)
+        shape3 = tuple(d3.shape)
+        pairs = [_tensor_work(segmentedMap, rev, transposed), _tensor_work(valueMap, rev, transposed)]
+        seg_w, vm_w = pairs[0][1], pairs[1][1]
+        if flipedPoints is not None:
+            if isinstance(flipedPoints, torch.Tensor) and flipedPoints.is_cuda:
+                if flipedPoints.dtype.is_floating_point or flipedPoints.dtype.is_complex or flipedPoints.dtype == torch.bool:
+                    raise TypeError("flipedPoints must hold integer coordinates, got %s" % flipedPoints.dtype)
+                if flipedPoints.device != dev:
+                    raise ValueError("flipedPoints (%s) and valueMap (%s) are on different devices" % (flipedPoints.device, dev))
+                pts = flipedPoints.reshape(-1, nd).to(torch.int64)
+            else:  # a host list of points is small: copied to the device once
+                pts = torch.from_numpy(np.asarray(flipedPoints, dtype=np.int64).reshape(-1, nd)).to(dev)
+            if transposed:
+                pts = pts.flip(1)
+            flips = torch.cat([pts.new_zeros((pts.shape[0], 3 - nd)), pts], dim=1).contiguous()  # (z, y, x) rows
+        with VRGEngine(shape3, H=H, max_segment_size=2 ** 62, iter_max=ITER_MAX, device=dev.index, intensity="f64_band") as eng:
+            eng.set_stream(stream.cuda_stream)
+            eng.attach_state_typed(d3.data_ptr(), seg_w.data_ptr(), seg_code, vm_w.data_ptr(), vm_code)
+            eng.init()
+            if flipedPoints is None:
+                eng.enqueue_table()
+                res = eng.poll()
+            else:  # rows outside the volume raise here, before anything of the caller's is written
+                res = eng.apply_flips_device(flips.data_ptr() if len(flips) else None, len(flips))
+
+            def rows(which, cap):
+                out = torch.empty((cap, 3), dtype=torch.int64, device=dev)
+                n = eng.band_rows_device(which, out.data_ptr() if cap else None, cap)
+                if n > cap:
+                    out = torch.empty((n, 3), dtype=torch.int64, device=dev)
+                    eng.band_rows_device(which, out.data_ptr(), n)
+                return _tensor_user_rows(torch, out[:n], shape, transposed)
+            innerBnd = rows(1, res["n_in"])  # the inner band is part of the segmented set
+            outerBnd = rows(2, 0)  # counted first
+            segmentedOut = segmented if flipedPoints is None else rows(0, res["n_in"])
+            if new_prob:  # VRG:132-133
+                pin3 = torch.empty(shape3, dtype=torch.float64, device=dev)
+                pout3 = torch.empty(shape3, dtype=torch.float64, device=dev)
+            else:
+                pairs += [_tensor_work(innerProb, rev, transposed), _tensor_work(outerProb, rev, transposed)]
+                pin3, pout3 = pairs[2][1], pairs[3][1]
+            eng.band_sums_device(pin3.data_ptr(), pout3.data_ptr())
+            eng.labels_device_typed(seg_w.data_ptr(), seg_code, segmented_only=True)
+            eng.labels_device_typed(vm_w.data_ptr(), vm_code)
+        for view, work in pairs:
+            if work is not view:
+                view.copy_(work)
+        if new_prob:
+            zyx_shape = shape3[3 - nd:]
+            innerProb, outerProb = ((t.reshape(zyx_shape).permute(rev).contiguous() if transposed else t.reshape(shape))
+                                    for t in (pin3, pout3))
+    return segmentedOut, segmentedMap, valueMap, innerBnd, outerBnd, innerProb, outerProb
+
+
 def update(dataArray, segmented, segmentedMap, valueMap, H, flipedPoints=None, innerBnd=None, outerBnd=None,
            innerProb=None, outerProb=None):
     """One call of the reference's ``update`` (VRG:124-261) on the GPU: the init branch (``flipedPoints is None``,
@@ -464,7 +579,24 @@ def update(dataArray, segmented, segmentedMap, valueMap, H, flipedPoints=None, i
     reference's where its incremental sums have not drifted).  ``valueMap`` and ``segmentedMap`` are updated in place
     and returned as the same objects, like the reference does; listed voxels that are in neither band are ignored.
     Level-table data only (at most 65536 distinct intensities), one GPU (``DEVICE``).
+
+    CUDA tensors: when ``valueMap`` is a CUDA tensor the call runs on its device and torch's current stream, and nothing of
+    volume size crosses PCIe.  ``dataArray`` and ``segmentedMap`` must be CUDA tensors on that device (mixing host arrays and
+    tensors raises ``TypeError``); intensities of any real dtype are converted to float64 once, the two maps are read in
+    their own dtypes (uint8, int8, int16, int32, int64, float32, float64): ``segmentedMap == 1`` is segmented, ``valueMap ==
+    4`` excluded.  ``flipedPoints`` may be a CUDA integer tensor ``(F, ndim)`` or anything ``np.asarray`` takes (copied to the
+    device once); a point outside the volume raises ``ValueError`` before anything is modified.  ``valueMap`` and
+    ``segmentedMap`` are updated in place in their dtypes; ``innerBnd`` / ``outerBnd`` come back as int64 CUDA tensors
+    ``(n, ndim)`` in C order of the caller's axes, ``segmented`` too (the caller's object on the init branch);
+    ``innerProb`` / ``outerProb`` must then be float64 CUDA tensors (``TypeError`` otherwise) and are updated in place, or
+    are returned as new C-contiguous ones when either is None.  Layouts as in ``variationalRegionGrowing``; on any error
+    the four caller tensors are bit-unchanged.  Results are bit-identical to the call on host arrays.
     """
+    torch = sys.modules.get("torch")  # a tensor can only come from an imported torch
+    if torch is not None and isinstance(valueMap, torch.Tensor) and valueMap.is_cuda:
+        return _tensor_update(dataArray, segmented, segmentedMap, valueMap, H, flipedPoints, innerProb, outerProb)
+    if torch is not None and any(isinstance(a, torch.Tensor) and a.is_cuda for a in (dataArray, segmentedMap, innerProb, outerProb)):
+        raise TypeError("update: valueMap is not a CUDA tensor, so dataArray, segmentedMap, innerProb and outerProb may not be")
     dataArray = np.asarray(dataArray)
     if not isinstance(valueMap, np.ndarray) or not isinstance(segmentedMap, np.ndarray):
         raise TypeError("valueMap and segmentedMap must be ndarrays (they are updated in place, as in the reference)")

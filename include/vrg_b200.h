@@ -121,6 +121,11 @@ typedef enum {
  * pass); anything but an integral value in 0..4 (negative, fractional, NaN, above 4) makes vrg_init return VRG_ERR_LABEL.
  * The valueMap pointer must be aligned to its element size (any storage offset of a tensor view is). */
 int vrg_attach_device_typed(vrg_handle *h, const double *data_dev, const void *value_map_dev, int32_t value_map_dtype);
+/* the inputs of update() (VRG:124) on the device: data attached zero-copy like vrg_attach_device; the state built on the handle's
+ * stream into the handle's own uint8 valueMap from the caller's segmentedMap (== 1: segmented) and valueMap (== 4: excluded),
+ * each in its own vrg_dtype and read only by this call (every other value: outside).  Map pointers aligned to their element size. */
+int vrg_attach_state_typed(vrg_handle *h, const double *data_dev, const void *seg_map_dev, int32_t seg_map_dtype,
+                           const void *value_map_dev, int32_t value_map_dtype);
 
 /* distinct intensity levels (the decision table's domain) ------------------- */
 int vrg_scan_levels(vrg_handle *h, int64_t *n_levels);             /* local slab */
@@ -151,6 +156,9 @@ int vrg_dense_refresh_sweeps(vrg_handle *h, int64_t *n);
  * Listed voxels that are in neither band are ignored; the band state machine (cancel rule, absorption, region statistics)
  * is applied once and the decision table of the NEW state is computed (vrg_get_table).  Whole-volume handles only. */
 int vrg_apply_flips(vrg_handle *h, const int64_t *coords_host, int64_t n, vrg_result *res);
+/* the same with the n rows in device memory (int64, 8-byte aligned): checked on the device first, one synchronisation for the
+ * verdict; a row outside the volume returns VRG_ERR_ARG naming the first such row, and nothing has changed */
+int vrg_apply_flips_device(vrg_handle *h, const int64_t *rows_dev, int64_t n, vrg_result *res);
 /* decision table of the current state without a sweep (after vrg_init: the sums the reference's init branch stores) */
 int vrg_enqueue_table(vrg_handle *h);
 
@@ -222,6 +230,13 @@ int vrg_download_segmented(vrg_handle *h, int64_t *coords_out, int64_t cap, int6
 /* the same rows compacted on the device into device memory (rows_dev may be NULL: count only); rows beyond cap are not
  * written; *n = their number.  Synchronises the handle's stream once, for the count. */
 int vrg_segmented_device(vrg_handle *h, int64_t *rows_dev, int64_t cap, int64_t *n);
+/* the same for which = 0 (segmented, == vrg_segmented_device), 1 (inner band, label 1) or 2 (outer band, label 2): rows (z,y,x)
+ * of the own planes in C order, compacted on the device; one synchronisation, for the count */
+int vrg_band_rows_device(vrg_handle *h, int32_t which, int64_t *rows_dev, int64_t cap, int64_t *n);
+/* update()'s innerProb / outerProb (VRG:132-133,151-155) of the current decision table (after vrg_init + vrg_enqueue_table, or
+ * vrg_apply_flips*): own planes, C order, float64 device buffers; pin * n_in and pout * n_out (vrg_get_table, one rounding each) at
+ * every inner / outer band voxel, 0.0 elsewhere.  Enqueued on the handle's stream, no synchronisation.  Level-table modes only. */
+int vrg_band_sums_device(vrg_handle *h, double *pin_dev, double *pout_dev);
 int vrg_get_trace(vrg_handle *h, int64_t *rows_out, int64_t cap_rows, int64_t *n_rows); /* (n_flips,n_in,n_out) */
 /* last decision table: in/out normalised Parzen sums per level (VRG:79-82), for parity checks */
 int vrg_get_table(vrg_handle *h, double *pin_out, double *pout_out, int64_t cap);
