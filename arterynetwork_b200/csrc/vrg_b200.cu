@@ -72,11 +72,8 @@ struct vrg_handle {
     bool have_data = false, have_levels = false, inited = false, separate_gstats = false;
     int64_t launches = 0;
     int grid = 148 * 8;
-    bool slim_sweep = false;  // set while a pipelined batch is enqueued: the dense sweep runs in its 104-register variant
-    bool no_ahead = false;  // A/B switch VRG_NO_AHEAD: vrg_run looks at a batch's status before it queues the next one
-    bool no_wide = false;  // A/B switch VRG_NO_WIDE: rows of 31 / 32 words stay two 16-word segments in the dense sweep
     bool no_dcache = false;  // A/B switch VRG_NO_DCACHE: no decision bit-plane, every dense sweep reads the fp64 volume
-    bool dense_attr_set = false, force_ldg = false, hist_attr_set = false, attached = false;
+    bool dense_attr_set = false, hist_attr_set = false, attached = false;
     const void *vm_base = nullptr;  // valueMap as indexed by local plane (own uint8 buffer, or attached in its own dtype)
     int vm_dtype = VRG_DTYPE_U8;
     // optional per-kernel timing (CUDA events on the launch stream), see vrg_profile
@@ -94,10 +91,9 @@ struct vrg_handle {
     long long *d_slots = nullptr;
     std::vector<void *> ipc_opened;
     long long epoch = 0;
-    // second stream of a slab run: the halo exchange runs beside the statistics exchange + decision table
-    cudaStream_t halo_stream = nullptr;
+    // second stream of the pipelined run: the statistics exchange + next decision table beside the next sweep
+    cudaStream_t side_stream = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    bool halo_pending = false, p2p_overlap = true;
     // continuous-intensity mode (vrg_parzen.cuh)
     Cont cq;
     bool cont_alloc = false;
@@ -141,9 +137,8 @@ static size_t dense_smem_bytes(const Params &p, bool wide = false) {
            (size_t)DENSE_WARPS * DENSE_STAGES * (wide ? WIDE_STAGE_BYTES : STAGE_BYTES);
 }
 // rows of 31 / 32 words (two 16-word segments): one warp per whole row in the dense sweep, if its 8 KB stages fit
-static bool dense_wide(const vrg_handle *h) {
-    const Params &p = h->p;
-    return p.nseg == 2 && p.segw == 16 && dense_smem_bytes(p, true) <= 227 * 1024 && !h->no_wide;
+static bool dense_wide(const Params &p) {
+    return p.nseg == 2 && p.segw == 16 && dense_smem_bytes(p, true) <= 227 * 1024;
 }
 
 static cudaEvent_t prof_event(vrg_handle *h) {
@@ -198,11 +193,7 @@ int vrg_create(const vrg_config *cfg, vrg_handle **out) {
     CK(cudaGetDeviceProperties(&prop, cfg->device));
     h->sms = prop.multiProcessorCount;
     h->grid = h->sms * 8;
-    h->force_ldg = getenv("VRG_DENSE_LDG") != nullptr;  // A/B switch: plain loads instead of the TMA rings (sweep, init histogram)
-    h->no_wide = getenv("VRG_NO_WIDE") != nullptr;
     h->no_dcache = getenv("VRG_NO_DCACHE") != nullptr;
-    h->no_ahead = getenv("VRG_NO_AHEAD") != nullptr;
-    h->graph_ok = getenv("VRG_NO_GRAPH") == nullptr;    // A/B switch: vrg_run stays on plain stream launches
     h->tail_ok = getenv("VRG_NO_FUSED_TAIL") == nullptr;  // A/B switch: the separate kernels behind the sweep
     if (const char *e = getenv("VRG_PIPELINE")) h->pipe_mode = atoi(e) != 0;  // A/B switch (default: pipelined on slabs only)
     CK(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
@@ -229,7 +220,6 @@ int vrg_create(const vrg_config *cfg, vrg_handle **out) {
     {   // rows per work unit of the dense sweep: long units on large volumes (fewer window restarts), short ones on thin slabs
         const long long rows_per_warp = (long long)(h->nz_own + 2) * Y * (p.nseg == 2 && p.segw == 16 ? 1 : p.nseg) / ((long long)h->sms * DENSE_WARPS);
         p.dense_rows = rows_per_warp >= 96 ? 8 : 4;  // measured: profiles/README.md (r2b, r2c)
-        if (const char *e = getenv("VRG_DENSE_ROWS")) p.dense_rows = std::max(1, atoi(e));  // A/B switch
     }
     h->plane_bytes = (size_t)p.nzl * p.plane_words * sizeof(uint32_t);
     h->rowflag_bytes = (size_t)p.nzl * Y * p.nseg;
@@ -289,7 +279,7 @@ int vrg_destroy(vrg_handle *h) {
         cudaFree(h->cq.rowlist); cudaFree(h->cq.count); cudaFree(h->cq.partial); cudaFree(h->cq.abrowlist); cudaFree(h->cq.AB);
     }
     if (h->gexec) cudaGraphExecDestroy(h->gexec);
-    if (h->halo_stream) { cudaStreamSynchronize(h->halo_stream); cudaStreamDestroy(h->halo_stream); }
+    if (h->side_stream) { cudaStreamSynchronize(h->side_stream); cudaStreamDestroy(h->side_stream); }
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     if (h->ev_join) cudaEventDestroy(h->ev_join);
     for (void *o : h->ipc_opened) cudaIpcCloseMemHandle(o);
@@ -310,7 +300,7 @@ int vrg_set_stream(vrg_handle *h, void *s) {
     CK(cudaStreamSynchronize(h->stream));
     if (h->own_stream) { cudaStreamDestroy(h->stream); h->own_stream = false; }
     h->stream = (cudaStream_t)s;
-    h->graph_ok = getenv("VRG_NO_GRAPH") == nullptr;
+    h->graph_ok = true;  // a new stream may be capturable where the last one was not
     return VRG_OK;
 }
 
@@ -639,39 +629,27 @@ static int launch_init_hist(vrg_handle *h) {
         CK(cudaFuncSetAttribute(k_init_hist_private<MODE_INDEX, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         CK(cudaFuncSetAttribute(k_init_hist_private<MODE_F64_BAND, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         CK(cudaFuncSetAttribute(k_init_hist_private<MODE_F64_BAND, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        CK(cudaFuncSetAttribute(k_init_hist_tma<MODE_INDEX, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        CK(cudaFuncSetAttribute(k_init_hist_tma<MODE_INDEX, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        CK(cudaFuncSetAttribute(k_init_hist_tma<MODE_F64_BAND, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        CK(cudaFuncSetAttribute(k_init_hist_tma<MODE_F64_BAND, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         CK(cudaFuncSetAttribute(k_init_hist_shared<MODE_INDEX, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         CK(cudaFuncSetAttribute(k_init_hist_shared<MODE_INDEX, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         CK(cudaFuncSetAttribute(k_init_hist_shared<MODE_F64_BAND, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         CK(cudaFuncSetAttribute(k_init_hist_shared<MODE_F64_BAND, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         h->hist_attr_set = true;
     }
-    // TMA-staged variant: the level source streams through a per-warp ring (16-byte aligned row segments only)
+    // TMA-staged: the level source streams through a per-warp ring (16-byte aligned row segments only), one shared-memory
+    // histogram per warp (atomics), many warps per SM
     const size_t elem = h->cfg.intensity_mode == VRG_INTENSITY_INDEX ? sizeof(uint16_t) : sizeof(double);
     const uintptr_t src_base = h->cfg.intensity_mode == VRG_INTENSITY_INDEX ? (uintptr_t)p.index : (uintptr_t)p.data;
-    if (((size_t)p.X * elem) % 16 == 0 && (src_base & 15) == 0 && !h->force_ldg) {
+    if (((size_t)p.X * elem) % 16 == 0 && (src_base & 15) == 0) {
         const size_t stage_bytes = ((size_t)p.segw * 32 * elem + 127) & ~(size_t)127;
-        {   // one shared-memory histogram per warp (atomics): many warps per SM
-            const size_t per_w = (size_t)((p.L + 1) & ~1) * sizeof(unsigned int);
-            const size_t per = per_w + HIST_STAGES * stage_bytes + HIST_STAGES * 8;
-            // the kernel evaluates whole batches of 10 words: on a short row the last batch reads (and ignores) up to 2560 bytes
-            // behind its stage, which must still be shared memory of this block
-            const size_t slack = 10 * 32 * sizeof(double);
-            const int hw = (int)std::min<size_t>(16, (227 * 1024 - 256 - slack) / per);
-            if (hw >= 8 && getenv("VRG_HIST_PRIVATE") == nullptr) {
-                const size_t smem = (((size_t)hw * HIST_STAGES * 8 + 127) & ~(size_t)127) + (size_t)hw * HIST_STAGES * stage_bytes + hw * per_w + slack;
-                LAUNCH_ML(k_init_hist_shared, h->sms, hw * 32, smem, p, hw, (int)stage_bytes);
-                return VRG_OK;
-            }
-        }
-        const size_t per = per_warp + HIST_STAGES * stage_bytes + HIST_STAGES * 8;
-        const int hw = (int)std::min<size_t>(16, (227 * 1024 - 256) / per);
-        if (hw >= 3) {
-            const size_t smem = (((size_t)hw * HIST_STAGES * 8 + 127) & ~(size_t)127) + (size_t)hw * HIST_STAGES * stage_bytes + hw * per_warp;
-            LAUNCH_ML(k_init_hist_tma, h->sms, hw * 32, smem, p, hw, (int)stage_bytes);
+        const size_t per_w = (size_t)((p.L + 1) & ~1) * sizeof(unsigned int);
+        const size_t per = per_w + HIST_STAGES * stage_bytes + HIST_STAGES * 8;
+        // the kernel evaluates whole batches of 10 words: on a short row the last batch reads (and ignores) up to 2560 bytes
+        // behind its stage, which must still be shared memory of this block
+        const size_t slack = 10 * 32 * sizeof(double);
+        const int hw = (int)std::min<size_t>(16, (227 * 1024 - 256 - slack) / per);
+        if (hw >= 8) {
+            const size_t smem = (((size_t)hw * HIST_STAGES * 8 + 127) & ~(size_t)127) + (size_t)hw * HIST_STAGES * stage_bytes + hw * per_w + slack;
+            LAUNCH_ML(k_init_hist_shared, h->sms, hw * 32, smem, p, hw, (int)stage_bytes);
             return VRG_OK;
         }
     }
@@ -886,14 +864,15 @@ int vrg_init(vrg_handle *h) {
     if (!h || !h->inited) return fail(VRG_ERR_ARG, "init first"); \
     CK(cudaSetDevice(h->cfg.device))
 
-static int enqueue_sweep(vrg_handle *h) {
+// slim: the pipelined run's sweep, which leaves room for the statistics / table kernels beside it (vrg_tail.cuh)
+static int enqueue_sweep(vrg_handle *h, bool slim = false) {
     const Params &p = h->p;
     const size_t smem = (size_t)p.LW * sizeof(uint32_t);
     if (h->prof) cudaEventRecord(prof_event(h), h->stream);
     if (h->cfg.intensity_mode == VRG_INTENSITY_F64_DENSE) {
-        const bool wide = dense_wide(h);
+        const bool wide = dense_wide(p);
         const size_t dsm = dense_smem_bytes(p, wide);
-        if ((p.X & 1) == 0 && (((uintptr_t)p.data) & 15) == 0 && dsm <= 227 * 1024 && !h->force_ldg) {  // TMA ring: 16-byte aligned row segments
+        if ((p.X & 1) == 0 && (((uintptr_t)p.data) & 15) == 0 && dsm <= 227 * 1024) {  // TMA ring: 16-byte aligned row segments
             if (!h->dense_attr_set) {
                 CK(cudaFuncSetAttribute(k_sweep_dense<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
                 CK(cudaFuncSetAttribute(k_sweep_dense<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
@@ -905,7 +884,7 @@ static int enqueue_sweep(vrg_handle *h) {
                 CK(cudaFuncSetAttribute(k_sweep_dense_slim<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
                 h->dense_attr_set = true;
             }
-            if (h->slim_sweep) {  // pipelined run: leave room for the statistics / table kernels beside the sweep
+            if (slim) {
                 if (wide && p.lattice) k_sweep_dense_slim<true, true><<<h->sms, DENSE_WARPS * 32, dsm, h->stream>>>(p);
                 else if (wide) k_sweep_dense_slim<false, true><<<h->sms, DENSE_WARPS * 32, dsm, h->stream>>>(p);
                 else if (p.lattice) k_sweep_dense_slim<true><<<h->sms, DENSE_WARPS * 32, dsm, h->stream>>>(p);
@@ -983,23 +962,20 @@ int vrg_enqueue_advance(vrg_handle *h) {
 
 // ---- peer-memory transport ---------------------------------------------------------------------------
 // phase 0: executed flips (and cancelled flips when label 4 is present) after cancel; phase 1: excluded plane after flip
-static int enqueue_p2p_halo_on(vrg_handle *h, int phase, cudaStream_t st) {
+int vrg_enqueue_p2p_halo(vrg_handle *h, int phase) {
+    NEED_INIT();
+    if (!h->p2p_on) return fail(VRG_ERR_ARG, "p2p transport not connected");
     const int kinds = phase == 0 ? ((1 << PK_F) | (h->p.E ? (1 << PK_C) : 0)) : (h->p.E ? (1 << PK_E) : 0);
     if (!kinds) return VRG_OK;
-    k_p2p_push_halo<<<h->sms, BLOCK, 0, st>>>(h->p, h->q, kinds, 0);
-    k_p2p_wait_unpack_halo<<<h->sms, BLOCK, 0, st>>>(h->p, h->q, kinds, 0, phase == 0);
+    k_p2p_push_halo<<<h->sms, BLOCK, 0, h->stream>>>(h->p, h->q, kinds, 0);
+    k_p2p_wait_unpack_halo<<<h->sms, BLOCK, 0, h->stream>>>(h->p, h->q, kinds, 0, phase == 0);
     h->launches += 2;
     if (phase == 0) {
-        k_quirks<<<h->grid, BLOCK, 0, st>>>(h->p);
+        k_quirks<<<h->grid, BLOCK, 0, h->stream>>>(h->p);
         h->launches++;
     }
     CK(cudaGetLastError());
     return VRG_OK;
-}
-int vrg_enqueue_p2p_halo(vrg_handle *h, int phase) {
-    NEED_INIT();
-    if (!h->p2p_on) return fail(VRG_ERR_ARG, "p2p transport not connected");
-    return enqueue_p2p_halo_on(h, phase, h->stream);
 }
 int vrg_enqueue_p2p_stats(vrg_handle *h) {
     NEED_INIT();
@@ -1060,12 +1036,6 @@ int vrg_p2p_connect(vrg_handle *h, int rank, int world, const void *all_handles)
             q.peer_recv[r == rank - 1 ? 0 : 1] = (uint32_t *)pr;
         }
     }
-    if (!h->halo_stream) {
-        CK(cudaStreamCreateWithFlags(&h->halo_stream, cudaStreamNonBlocking));
-        CK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
-    }
-    h->p2p_overlap = getenv("VRG_P2P_SERIAL") == nullptr;  // A/B switch: everything on one stream, in program order
     h->p2p_on = true;
     h->inited = false;
     return VRG_OK;
@@ -1103,12 +1073,6 @@ int vrg_p2p_connect_local(vrg_handle **hs, int world) {
         for (int o = 0; o < world; ++o) { q.peer_flags[o] = hs[o]->d_flags; q.peer_slots[o] = hs[o]->d_slots; }
         q.peer_recv[0] = r > 0 ? hs[r - 1]->d_recv : nullptr;
         q.peer_recv[1] = r + 1 < world ? hs[r + 1]->d_recv : nullptr;
-        if (!h->halo_stream) {
-            CK(cudaStreamCreateWithFlags(&h->halo_stream, cudaStreamNonBlocking));
-            CK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-            CK(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
-        }
-        h->p2p_overlap = getenv("VRG_P2P_SERIAL") == nullptr;
         h->p2p_on = true;
         h->inited = false;
     }
@@ -1139,17 +1103,6 @@ int vrg_poll(vrg_handle *h, vrg_result *res) {
 int vrg_dense_refresh_sweeps(vrg_handle *h, int64_t *n) {
     if (!h || !n) return fail(VRG_ERR_ARG, "null argument");
     *n = h->inited ? h->h_ctrl[C_REFRESHES] : 0;  // the control block as the last vrg_poll read it
-    return VRG_OK;
-}
-
-// Slab run without label 4: after cancel the iteration forks -- the halo exchange (push, wait, unpack) goes to a
-// second stream while the statistics exchange, the loop bookkeeping and the next decision table stay on the main one;
-// the next sweep is the join.  (With label 4 the absorb step sits between two halo exchanges: everything stays serial.)
-static int join_halo(vrg_handle *h) {
-    if (h->halo_pending) {
-        CK(cudaStreamWaitEvent(h->stream, h->ev_join, 0));
-        h->halo_pending = false;
-    }
     return VRG_OK;
 }
 
@@ -1212,10 +1165,10 @@ static int enqueue_tail(vrg_handle *h) {
     return VRG_OK;
 }
 
-// second stream + events of the pipelined run (the slab transport creates them when it connects)
+// second stream + events of the pipelined run
 static int ensure_side_stream(vrg_handle *h) {
-    if (!h->halo_stream) {
-        CK(cudaStreamCreateWithFlags(&h->halo_stream, cudaStreamNonBlocking));
+    if (!h->side_stream) {
+        CK(cudaStreamCreateWithFlags(&h->side_stream, cudaStreamNonBlocking));
         CK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
         CK(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
     }
@@ -1254,19 +1207,19 @@ static int enqueue_tail_pipe(vrg_handle *h) {
 // this update are forked to the second stream.
 static int enqueue_pipelined(vrg_handle *h) {
     int rc;
-    if ((rc = enqueue_sweep(h)) != VRG_OK) return rc;
+    if ((rc = enqueue_sweep(h, true)) != VRG_OK) return rc;
     if (h->async_pending) {
         CK(cudaStreamWaitEvent(h->stream, h->ev_join, 0));
         h->async_pending = false;
     }
     if ((rc = enqueue_tail_pipe(h)) != VRG_OK) return rc;
     CK(cudaEventRecord(h->ev_fork, h->stream));
-    CK(cudaStreamWaitEvent(h->halo_stream, h->ev_fork, 0));
-    k_async_stats<<<1, ASYNC_BLOCK, 0, h->halo_stream>>>(h->p, h->q, h->d_gstats, h->p2p_on ? 1 : 0);
-    k_async_table<<<h->p.LW, ASYNC_BLOCK, 0, h->halo_stream>>>(h->p);
+    CK(cudaStreamWaitEvent(h->side_stream, h->ev_fork, 0));
+    k_async_stats<<<1, ASYNC_BLOCK, 0, h->side_stream>>>(h->p, h->q, h->d_gstats, h->p2p_on ? 1 : 0);
+    k_async_table<<<h->p.LW, ASYNC_BLOCK, 0, h->side_stream>>>(h->p);
     h->launches += 2;
     CK(cudaGetLastError());
-    CK(cudaEventRecord(h->ev_join, h->halo_stream));
+    CK(cudaEventRecord(h->ev_join, h->side_stream));
     h->async_pending = true;
     return VRG_OK;
 }
@@ -1290,29 +1243,12 @@ static int enqueue_batch(vrg_handle *h, int n) {
             continue;
         }
         if (piped) {
-            h->slim_sweep = getenv("VRG_NO_SLIM") == nullptr;
-            rc = enqueue_pipelined(h);
-            h->slim_sweep = false;
-            if (rc != VRG_OK) return rc;
+            if ((rc = enqueue_pipelined(h)) != VRG_OK) return rc;
             continue;
         }
         if (fused) {  // the table of this sweep was computed by the previous tail (the first one: vrg_run)
             if ((rc = enqueue_sweep(h)) != VRG_OK) return rc;
             if ((rc = enqueue_tail(h)) != VRG_OK) return rc;
-            continue;
-        }
-        const bool overlap = h->p2p_on && h->p2p_overlap && h->p.E == nullptr && h->halo_stream != nullptr;
-        if (overlap) {
-            if ((rc = enqueue_table(h)) != VRG_OK) return rc;
-            if ((rc = join_halo(h)) != VRG_OK) return rc;          // the sweep reads the halo planes of S
-            if ((rc = enqueue_sweep(h)) != VRG_OK) return rc;
-            if ((rc = vrg_enqueue_cancel(h)) != VRG_OK) return rc;
-            CK(cudaEventRecord(h->ev_fork, h->stream));
-            CK(cudaStreamWaitEvent(h->halo_stream, h->ev_fork, 0));
-            if ((rc = enqueue_p2p_halo_on(h, 0, h->halo_stream)) != VRG_OK) return rc;
-            CK(cudaEventRecord(h->ev_join, h->halo_stream));
-            h->halo_pending = true;
-            if ((rc = vrg_enqueue_p2p_stats(h)) != VRG_OK) return rc;
             continue;
         }
         if ((rc = vrg_enqueue_decide(h)) != VRG_OK) return rc;
@@ -1327,8 +1263,7 @@ static int enqueue_batch(vrg_handle *h, int n) {
             if ((rc = vrg_enqueue_advance(h)) != VRG_OK) return rc;
         }
     }
-    { int rc_ = join_async(h); if (rc_ != VRG_OK) return rc_; }
-    return join_halo(h);  // a batch ends joined: it may be a captured graph, and the host polls the main stream
+    return join_async(h);  // a batch ends joined: it may be a captured graph, and the host polls the main stream
 }
 
 static uint64_t run_signature(const vrg_handle *h) {
@@ -1339,7 +1274,7 @@ static uint64_t run_signature(const vrg_handle *h) {
     };
     mix(&h->p, sizeof(Params));
     if (h->p2p_on) mix(&h->q, sizeof(P2P));
-    const int64_t extra[6] = {h->cfg.intensity_mode, h->p2p_on, h->force_ldg, h->tail_ok, h->pipe_mode, h->no_dcache};
+    const int64_t extra[5] = {h->cfg.intensity_mode, h->p2p_on, h->tail_ok, h->pipe_mode, h->no_dcache};
     mix(extra, sizeof extra);
     return x;
 }
@@ -1404,7 +1339,7 @@ int vrg_run(vrg_handle *h, vrg_result *res) {
         CK(cudaMemcpyAsync(h->h_poll + slot * C_WORDS, h->d_ctrl, C_WORDS * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
         CK(cudaEventRecord(h->ev_poll[slot], h->stream));
         ++nbatch;
-        const bool ahead = use_graph && h->gexec != nullptr && !h->no_ahead;
+        const bool ahead = use_graph && h->gexec != nullptr;
         if (ahead && nbatch < 2) continue;  // nothing older to look at yet
         const int look = ahead ? (int)((nbatch - 2) & 1) : slot;
         CK(cudaEventSynchronize(h->ev_poll[look]));

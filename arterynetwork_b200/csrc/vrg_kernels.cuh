@@ -622,7 +622,6 @@ __device__ __forceinline__ void sweep_dense_body(const Params &p) {
             st.template begin<WIDE>(p, czl, y, c0 + lane, lane);
             fresh = false;
         }
-#ifndef VRG_NO_NEXT_WINDOW
         if (y + 1 >= cy1) {  // last row of the unit: lane 0 announced the next one when it issued this row
             nu = myring[ctail & (UNIT_RING - 1)];
             if (nu < nunits) {
@@ -630,7 +629,6 @@ __device__ __forceinline__ void sweep_dense_body(const Params &p) {
                 nx.template begin<WIDE>(p, nzl, ny, (WIDE ? 0 : nsg * p.segw - 1) + lane, lane);
             }
         }
-#endif
         uint32_t s, inner, outer;
         st.template step<WIDE>(p, y, s, inner, outer, lane);
         const long long widx = (long long)czl * p.plane_words + (long long)y * p.WP + c0 + lane;
@@ -676,22 +674,11 @@ __device__ __forceinline__ void sweep_dense_body(const Params &p) {
         else store_flips(p, widx, ridx, was, f, st.active, own, lane);
         if (own) flips += __popc(f);
         if (++cy >= cy1) {  // on to the next unit of this warp's sequence: its window is under way
-#ifndef VRG_NO_NEXT_WINDOW
             ++ctail;
             cu = nu; czl = nzl; csg = nsg; cy = ny; cy1 = ny1;
             st = nx;
             c0 = WIDE ? 0 : csg * p.segw - 1;
             own = czl >= p.own_lo && czl < p.own_hi;
-#else
-            __syncwarp();
-            cu = myring[ctail++ & (UNIT_RING - 1)];
-            if (cu < nunits) {
-                decode(cu, czl, csg, cy, cy1);
-                c0 = WIDE ? 0 : csg * p.segw - 1;
-                own = czl >= p.own_lo && czl < p.own_hi;
-                st.template begin<WIDE>(p, czl, cy, c0 + lane, lane);
-            }
-#endif
         }
     }
     flips = warp_sum(flips);
@@ -928,8 +915,8 @@ template <int MODE, bool LATTICE>
 __global__ void __launch_bounds__(BLOCK) k_cancel(Params p) {
     const bool go = p.ctrl[C_STATUS] == RUNNING && p.ctrl[C_APPLY];
     if (blockIdx.x == 0 && threadIdx.x == 0) {
-        // snapshot for the slab halo exchange that follows (vrg_p2p.cuh): it may run beside the statistics exchange,
-        // whose bookkeeping advances C_SWEEPS / C_STATUS.  Sequence number = (run epoch << 32) | (sweep + 1).
+        // snapshot for the slab halo exchange and k_quirks that follow (vrg_p2p.cuh): they read this iteration from it, not
+        // from C_SWEEPS / C_STATUS, which the statistics exchange advances.  Sequence number = (run epoch << 32) | (sweep + 1).
         p.ctrl[C_HALO_GO] = go;
         p.ctrl[C_HALO_SEQ] = (long long)(((unsigned long long)p.ctrl[C_EPOCH] << 32) | (unsigned long long)(p.ctrl[C_SWEEPS] + 1));
     }
@@ -1376,135 +1363,14 @@ __global__ void k_init_hist_private(Params p, int hw) {
     }
 }
 
-// k_init_hist_tma: k_init_hist_private with the level source (fp64 intensities, or the uint16 index volume) streamed
-// through a per-warp ring of TMA bulk-copy stages, exactly like the dense sweep: one stage = one row segment.  With the
-// loads off the warps' dependency chains, the few warps that fit beside their private histograms (5 at 468 levels)
-// keep enough bytes in flight to run at HBM speed.  Needs 16-byte aligned row segments (host checks).
-constexpr int HIST_STAGES = 2;
-template <int MODE, bool LATTICE>
-__global__ void k_init_hist_tma(Params p, int hw, int stage_bytes) {
-    using T = typename std::conditional<MODE == MODE_INDEX, uint16_t, double>::type;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int LP = (p.L + 1) & ~1;
-    uint64_t *bars = (uint64_t *)smem_raw;                                                  // [hw][HIST_STAGES]
-    unsigned char *stages = smem_raw + ((hw * HIST_STAGES * 8 + 127) & ~127);                // [hw][HIST_STAGES][stage_bytes]
-    uint16_t *s_hp = (uint16_t *)(stages + (size_t)hw * HIST_STAGES * stage_bytes);         // [hw][LP][32]
-    for (int i = threadIdx.x; i < hw * LP * 32; i += blockDim.x) s_hp[i] = 0;
-    uint64_t *mybar = bars + warp * HIST_STAGES;
-    unsigned char *mystage = stages + (size_t)warp * HIST_STAGES * stage_bytes;
-    if (lane == 0) {
-#pragma unroll
-        for (int s = 0; s < HIST_STAGES; ++s) mbar_init(mybar + s, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    uint16_t *mine = s_hp + (size_t)warp * LP * 32 + lane * 2;
-    unsigned long long *hin = (unsigned long long *)p.lstats, *hout = hin + p.L;
-    const long long nrows = (long long)(p.own_hi - p.own_lo) * p.Y * p.nseg;
-    const long long stride = (long long)gridDim.x * hw;
-    auto decode = [&](long long r, int &zl, int &y, int &sg) {
-        sg = (int)(r % p.nseg);
-        const long long t = r / p.nseg;
-        y = (int)(t % p.Y);
-        zl = p.own_lo + (int)(t / p.Y);
-    };
-    auto issue = [&](long long r, int s) {  // lane 0 only
-        int zl, y, sg;
-        decode(r, zl, y, sg);
-        const int x0 = sg * p.segw * 32;
-        const uint32_t bytes = (uint32_t)min(p.segw * 32, p.X - x0) * (uint32_t)sizeof(T);
-        const long long vox = (long long)zl * p.plane_vox + (long long)y * p.X + x0;
-        const void *src = MODE == MODE_INDEX ? (const void *)(p.index + vox) : (const void *)(p.data + vox);
-        mbar_expect_tx(mybar + s, bytes);
-        tma_bulk_load(mystage + (size_t)s * stage_bytes, src, bytes, mybar + s);
-    };
-    long long pre = (long long)blockIdx.x * hw + warp, cur = pre;
-#pragma unroll
-    for (int s = 0; s < HIST_STAGES; ++s) {
-        if (pre < nrows) {
-            if (lane == 0) issue(pre, s);
-            pre += stride;
-        }
-    }
-    long long n_in = 0, n_out = 0, n_ex = 0;
-    int pending = 0, stage = 0;
-    uint32_t parity = 0;
-    auto flush = [&]() {
-        __syncwarp();
-        for (int l = 0; l < p.L; ++l) {
-            unsigned int v = mine[(l >> 1) * 64 + (l & 1)];
-            mine[(l >> 1) * 64 + (l & 1)] = 0;
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(FULL, v, o);
-            if (lane == 0 && v) atomicAdd(&hout[l], (unsigned long long)v);
-        }
-        pending = 0;
-    };
-    for (; cur < nrows; cur += stride) {
-        int zl, y, sg;
-        decode(cur, zl, y, sg);
-        const int cfirst = sg * p.segw, nw = min(p.segw, p.XW - cfirst);
-        const long long wbase = (long long)zl * p.plane_words + (long long)y * p.WP + cfirst;
-        // lane j holds word j of the segment: region sizes by popcount, per-voxel work below only for the histogram
-        const uint32_t vrow = lane < nw ? valid_mask(p, cfirst + lane) : 0u;
-        const uint32_t srow = lane < nw ? p.S[wbase + lane] & vrow : 0u;
-        const uint32_t erow = (p.E && lane < nw) ? p.E[wbase + lane] & vrow & ~srow : 0u;
-        const uint32_t orow = vrow & ~srow & ~erow;  // outside region: the histogram this kernel keeps in shared memory
-        n_in += __popc(srow); n_ex += __popc(erow); n_out += __popc(orow);
-        const T *sv = (const T *)(mystage + (size_t)stage * stage_bytes) + lane;
-        mbar_wait(mybar + stage, parity);
-        constexpr int BW = 10;
-#pragma unroll
-        for (int jb = 0; jb < WORDS_PER_WARP; jb += BW) {
-            if (jb >= nw) break;  // warp-uniform
-            int lv[BW];
-#pragma unroll
-            for (int k = 0; k < BW; ++k) {
-                if (MODE == MODE_INDEX) lv[k] = (int)sv[(jb + k) * 32];
-                else lv[k] = level_of<LATTICE>(p, (double)sv[(jb + k) * 32]);
-            }
-            // branch-free: every lane does its load / add / store, adding 0 where the voxel is not an outside voxel
-            // (words past the row end hold stale bytes: their level is forced to 0, their increment is 0)
-            uint32_t segbits = 0;
-#pragma unroll
-            for (int k = 0; k < BW; ++k) {
-                const uint32_t ow = __shfl_sync(FULL, orow, (jb + k) & 31), sw = __shfl_sync(FULL, srow, (jb + k) & 31);
-                const uint32_t inc = (ow >> lane) & 1u, seg = (sw >> lane) & 1u;
-                const int l = (inc | seg) ? lv[k] : 0;
-                lv[k] = l;
-                segbits |= seg << k;
-                uint16_t *slot = mine + (l >> 1) * 64 + (l & 1);
-                *slot = (uint16_t)(*slot + inc);
-            }
-            if (__any_sync(FULL, segbits != 0u)) {  // the (tiny) inside region goes through global atomics
-#pragma unroll
-                for (int k = 0; k < BW; ++k)
-                    if (segbits & (1u << k)) atomicAdd(&hin[lv[k]], 1ull);
-            }
-        }
-        __syncwarp();
-        if (pre < nrows) {  // the stage is drained: re-arm it for a later row
-            if (lane == 0) issue(pre, stage);
-            pre += stride;
-        }
-        if (++stage == HIST_STAGES) { stage = 0; parity ^= 1u; }
-        pending += nw;
-        if (pending > 60000) flush();
-    }
-    flush();
-    n_in = warp_sum(n_in); n_out = warp_sum(n_out); n_ex = warp_sum(n_ex);
-    if (lane == 0) {
-        if (n_in) atomicAdd((unsigned long long *)&p.lstats[2 * p.L + ST_N_IN], (unsigned long long)n_in);
-        if (n_out) atomicAdd((unsigned long long *)&p.lstats[2 * p.L + ST_N_OUT], (unsigned long long)n_out);
-        if (n_ex) atomicAdd((unsigned long long *)&p.lstats[2 * p.L + ST_N_EXCL], (unsigned long long)n_ex);
-    }
-}
-
-// k_init_hist_shared: the same stream, but ONE histogram per warp updated by shared-memory atomics instead of 32 lane-private
-// ones: 4 bytes per level and warp instead of 64, so 12 warps fit beside their TMA rings where the lane-private layout left 5
-// (k_init_hist_tma ran at 22 % issue utilisation with 25 % of the DRAM bandwidth: too few warps to hide its own latency).
+// k_init_hist_shared: the result of k_init_hist, with the level source (fp64 intensities, or the uint16 index volume) streamed
+// through a per-warp ring of TMA bulk-copy stages, exactly like the dense sweep: one stage = one row segment.  Needs 16-byte
+// aligned row segments (host checks; k_init_hist_private and k_init_hist serve the rest).  ONE histogram per warp, updated
+// by shared-memory atomics: 4 bytes per level and warp instead of the 64 of k_init_hist_private's 32 lane-private ones, so
+// 12 warps fit beside their TMA rings where the lane-private layout beside the same rings left 5 (that variant ran at 22 %
+// issue utilisation with 25 % of the DRAM bandwidth: too few warps to hide its own latency).
 // Lanes of a warp that meet in a bin are serialised by the hardware; the outside region's levels spread over tens of bins.
+constexpr int HIST_STAGES = 2;
 template <int MODE, bool LATTICE>
 __global__ void k_init_hist_shared(Params p, int hw, int stage_bytes) {
     using T = typename std::conditional<MODE == MODE_INDEX, uint16_t, double>::type;

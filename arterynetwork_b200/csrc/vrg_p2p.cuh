@@ -95,8 +95,8 @@ __device__ __forceinline__ bool p2p_last_block(unsigned long long *counter) {
 // ---- halo --------------------------------------------------------------------------------------------------------
 // kinds: bit mask over PK_*.  `running_only`: loop exchanges obey the run status; the one after init does not.
 // Loop exchanges take their sequence number and their go / no-go from the snapshot k_cancel left in the control block
-// (C_HALO_SEQ, C_HALO_GO): the halo exchange may run on a second stream beside the statistics exchange, whose
-// bookkeeping moves C_SWEEPS / C_STATUS on.  The receive buffer is double-buffered by sequence parity, because a
+// (C_HALO_SEQ, C_HALO_GO), which holds the iteration k_cancel applied until the next k_cancel; C_SWEEPS / C_STATUS move on
+// with the statistics exchange's bookkeeping.  The receive buffer is double-buffered by sequence parity, because a
 // neighbour that is one iteration ahead may push its next planes while this rank still unpacks the current ones.
 __device__ __forceinline__ bool p2p_halo_seq(const Params &p, int seq_zero, unsigned long long &seq) {
     if (seq_zero) { seq = (unsigned long long)p.ctrl[C_EPOCH] << 32; return true; }

@@ -547,10 +547,7 @@ __global__ void __launch_bounds__(TAIL_BLOCK, 1) k_tail_pipe(Params p, P2P q, un
 
 // k_async_stats (second stream, one small block beside the running sweep): the statistics all-reduce of the update the tail
 // kernel just applied (slabs), then the exit tests of VRG:91-104,118 and the loop bookkeeping of VRG:113-117.
-#ifndef VRG_ASYNC_BLOCK
-#define VRG_ASYNC_BLOCK 256
-#endif
-constexpr int ASYNC_BLOCK = VRG_ASYNC_BLOCK;  // these blocks have to find room on SMs the sweep's blocks occupy: see k_sweep_dense_slim
+constexpr int ASYNC_BLOCK = 256;  // these blocks have to find room on SMs the sweep's blocks occupy: see k_sweep_dense_slim
 __global__ void __launch_bounds__(ASYNC_BLOCK) k_async_stats(Params p, P2P q, long long *gstats, int p2p) {
     __shared__ int s_ok;
     if (p.ctrl[C_STATUS] != RUNNING || !p.ctrl[C_TAIL_APPLIED]) return;

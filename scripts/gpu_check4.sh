@@ -1,8 +1,9 @@
 #!/bin/bash
 set -x
-mkdir -p gpurun_out
+OUT=${OUT:-out}  # output directory (git-ignored)
+mkdir -p "$OUT"
 TAG=${1:-r2d}
-timeout 900 python -m pytest tests -m gpu -q -x -rs 2>&1 | tail -8 > gpurun_out/${TAG}_pytest_gpu.txt
-cat gpurun_out/${TAG}_pytest_gpu.txt
-VRG_VERBOSE=1 timeout 300 python scripts/sweep_time.py 82x880x880:10 640x880x880:10 > gpurun_out/${TAG}_sweep_time.jsonl 2> gpurun_out/${TAG}_sweep_time.err
-cat gpurun_out/${TAG}_sweep_time.jsonl; tail -n 5 gpurun_out/${TAG}_sweep_time.err
+timeout 900 python -m pytest tests -m gpu -q -x -rs 2>&1 | tail -8 > $OUT/${TAG}_pytest_gpu.txt
+cat $OUT/${TAG}_pytest_gpu.txt
+VRG_VERBOSE=1 timeout 300 python scripts/sweep_time.py 82x880x880 640x880x880 > $OUT/${TAG}_sweep_time.jsonl 2> $OUT/${TAG}_sweep_time.err
+cat $OUT/${TAG}_sweep_time.jsonl; tail -n 5 $OUT/${TAG}_sweep_time.err

@@ -1,7 +1,7 @@
 #!/bin/bash
 # gpurun --gpus N -- bash scripts/gpu_multi_ab.sh N [TAG] : multi-GPU parity tests, then the N-GPU bench on the production path
 # (pipelined: statistics + table beside the next sweep) and, for comparison, in order (VRG_PIPELINE=0: fused tail kernel) and
-# on the separate kernels (VRG_NO_FUSED_TAIL=1: halo exchange on a second stream)
+# on the separate kernels (VRG_NO_FUSED_TAIL=1: cancel, halo exchange, statistics exchange and table in program order)
 N=${1:-2}
 TAG=${2:-r2}
 set -x

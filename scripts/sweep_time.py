@@ -1,10 +1,10 @@
 #!/usr/bin/env python
-"""A/B timings of the dense sweep on arbitrary volume shapes (one process, several configurations):
+"""Timings of the dense sweep on arbitrary volume shapes (one process, several shapes):
 
-    python scripts/sweep_time.py 640x880x880:7,10 82x880x880:7,10 128x2048x2048:8,10
+    python scripts/sweep_time.py 640x880x880 82x880x880 128x2048x2048
 
-Each item is ZxYxX:bw[,bw...]; bw = VRG_DENSE_BW (words per batch of the decision evaluation).  Prints one JSON line per
-run: mean k_sweep_dense time (CUDA events on the launch stream), whole-run time with CUDA graphs, iterations."""
+Each item is ZxYxX.  Prints one JSON line per shape: mean k_sweep_dense time (CUDA events on the launch stream), whole-run
+time with CUDA graphs, iterations."""
 import json
 import os
 import sys
@@ -20,44 +20,41 @@ def main():
     stream = torch.cuda.Stream()
     torch.cuda.set_stream(stream)
     for item in sys.argv[1:]:
-        shp, _, bws = item.partition(":")
-        shape = tuple(int(t) for t in shp.split("x"))
+        shape = tuple(int(t) for t in item.split("x"))
         d, v = bench.device_phantom(shape, 0, 0, shape[0], 0)
         torch.cuda.synchronize()
         nvox = shape[0] * shape[1] * shape[2]
-        for bw in (bws.split(",") if bws else ["0"]):
-            os.environ["VRG_DENSE_BW"] = bw
-            with VRGEngine(shape, max_segment_size=10 ** 15, intensity="f64_dense") as eng:
-                eng.set_stream(stream.cuda_stream)
+        with VRGEngine(shape, max_segment_size=10 ** 15, intensity="f64_dense") as eng:
+            eng.set_stream(stream.cuda_stream)
 
-                def step():
-                    eng.attach_device(d.data_ptr(), v.data_ptr())
-                    eng.init()
-                    return eng.run()
-                step(); step()
-                s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                torch.cuda.synchronize()
-                s.record()
-                res = step()
-                e.record()
-                torch.cuda.synchronize()
-                ms_graph = s.elapsed_time(e)
-                eng.profile(True)
-                s.record()
-                res = step()
-                e.record()
-                torch.cuda.synchronize()
-                ms_eager = s.elapsed_time(e)
-                prof = eng.get_profile()
-                tail = eng.get_tail_profile()
-                eng.profile(False)
-            per = prof["decide_ms"] / max(1, prof["decide_launches"])
-            print(json.dumps({"shape": shape, "bw": bw, "sweeps": res["sweeps"], "sweep_ms": per,
-                              "sweep_10B_GBps": 10.0 * nvox / (per * 1e-3) / 1e9, "real_8B_GBps": 8.13 * nvox / (per * 1e-3) / 1e9,
-                              "cancel_ms": prof["cancel_ms"] / max(1, prof["cancel_launches"]), "tail_phases_us": tail,
-                              "run_ms_graph": ms_graph, "run_ms_eager_profiled": ms_eager,
-                              "Gvox_s_graph": nvox * res["sweeps"] / ms_graph / 1e6,
-                              "per_iter_us_graph": 1e3 * ms_graph / res["sweeps"]}), flush=True)
+            def step():
+                eng.attach_device(d.data_ptr(), v.data_ptr())
+                eng.init()
+                return eng.run()
+            step(); step()
+            s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            torch.cuda.synchronize()
+            s.record()
+            res = step()
+            e.record()
+            torch.cuda.synchronize()
+            ms_graph = s.elapsed_time(e)
+            eng.profile(True)
+            s.record()
+            res = step()
+            e.record()
+            torch.cuda.synchronize()
+            ms_eager = s.elapsed_time(e)
+            prof = eng.get_profile()
+            tail = eng.get_tail_profile()
+            eng.profile(False)
+        per = prof["decide_ms"] / max(1, prof["decide_launches"])
+        print(json.dumps({"shape": shape, "sweeps": res["sweeps"], "sweep_ms": per,
+                          "sweep_10B_GBps": 10.0 * nvox / (per * 1e-3) / 1e9, "real_8B_GBps": 8.13 * nvox / (per * 1e-3) / 1e9,
+                          "cancel_ms": prof["cancel_ms"] / max(1, prof["cancel_launches"]), "tail_phases_us": tail,
+                          "run_ms_graph": ms_graph, "run_ms_eager_profiled": ms_eager,
+                          "Gvox_s_graph": nvox * res["sweeps"] / ms_graph / 1e6,
+                          "per_iter_us_graph": 1e3 * ms_graph / res["sweeps"]}), flush=True)
         del d, v
         torch.cuda.empty_cache()
 

@@ -19,8 +19,10 @@ COUNTERS = ("iterations", "exit_reason", "n_in", "n_out", "n_excluded", "sweeps"
             "q_remove_to_outside", "q_cancel_repromoted")
 
 
-def run_dense(data, vm, H, max_seg, monkeypatch, env=(), iter_max=200):
-    """One f64_dense run on a fresh handle with the environment switches `env` set while the handle is created."""
+def run_dense(data, vm, H, max_seg, monkeypatch, env=(), iter_max=200, unaligned=False):
+    """One f64_dense run on a fresh handle with the environment switches `env` set while the handle is created.
+    `unaligned`: attach the intensities zero-copy from a CUDA buffer that is only 8-byte aligned, as a tensor view with an
+    odd storage offset is, instead of uploading a copy."""
     from arterynetwork_b200.engine import VRGEngine
     for k in env:
         monkeypatch.setenv(k, "1")
@@ -30,7 +32,15 @@ def run_dense(data, vm, H, max_seg, monkeypatch, env=(), iter_max=200):
         for k in env:
             monkeypatch.delenv(k)
     with eng:
-        eng.upload(np.asarray(data, dtype=np.float64), np.asarray(vm, dtype=np.uint8))
+        if unaligned:
+            import torch
+            d = torch.empty(data.size + 1, dtype=torch.float64, device="cuda")[1:]
+            assert d.data_ptr() % 16 == 8
+            d.copy_(torch.from_numpy(np.ascontiguousarray(data, dtype=np.float64).ravel()))
+            v = torch.from_numpy(np.ascontiguousarray(vm, dtype=np.uint8)).cuda()
+            eng.attach_device(d.data_ptr(), v.data_ptr())
+        else:
+            eng.upload(np.asarray(data, dtype=np.float64), np.asarray(vm, dtype=np.uint8))
         eng.init()
         out = dict(eng.run())
         out["labels"] = eng.labels()
@@ -134,12 +144,11 @@ def _phantom(shape, kw):
     return data, vm
 
 
-@pytest.mark.parametrize("case", ["odd_x", "wide_1024", "dense_ldg", "label4"])
+@pytest.mark.parametrize("case", ["odd_x", "wide_1024", "unaligned", "label4"])
 def test_every_sweep_variant_keeps_and_reads_the_plane(case, monkeypatch):
-    """The refresh kernels other than the TMA ring of the bench shape: the plain-load kernel (odd X, and VRG_DENSE_LDG=1),
-    a whole row per warp (X = 1024), and a label-4 input (excluded mask, separate kernels behind the sweep).  Default equals
-    VRG_NO_DCACHE=1 equals the oracle, and the cache is used."""
-    env = ()
+    """The refresh kernels other than the TMA ring of the bench shape: the plain-load kernel (odd X, and an even X attached
+    from an 8-byte aligned buffer), a whole row per warp (X = 1024), and a label-4 input (excluded mask, separate kernels
+    behind the sweep).  Default equals VRG_NO_DCACHE=1 equals the oracle, and the cache is used."""
     if case == "odd_x":
         from random_cases import table_shift_case
         data, vm = table_shift_case()
@@ -153,12 +162,18 @@ def test_every_sweep_variant_keeps_and_reads_the_plane(case, monkeypatch):
         ref = vrg_oracle_c(data, vm, max_segment_size=10 ** 12)
         H, ms = 2.25, 10 ** 12
     else:
-        g = load_golden("forest40" if case == "dense_ldg" else "excl32")
+        g = load_golden("forest40" if case == "unaligned" else "excl32")
         data, vm, H, ms = g["data"], g["value_map_in"], g["H"], g["max_segment_size"]
         ref = {"iterations": g["iterations"], "trace": g["trace"], "labels": g["labels"]}
-        env = ("VRG_DENSE_LDG",) if case == "dense_ldg" else ()
-    a = run_dense(data, vm, H, ms, monkeypatch, env=env)
-    b = run_dense(data, vm, H, ms, monkeypatch, env=env + ("VRG_NO_DCACHE",))
+    unaligned = case == "unaligned"
+    if unaligned:  # the refresh must be the plain-load kernel, not the TMA ring it would take on aligned data
+        from torch.profiler import ProfilerActivity, profile
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            a = run_dense(data, vm, H, ms, monkeypatch, unaligned=True)
+        assert any("k_sweep_dense_ldg" in e.name for e in prof.events())
+    else:
+        a = run_dense(data, vm, H, ms, monkeypatch)
+    b = run_dense(data, vm, H, ms, monkeypatch, env=("VRG_NO_DCACHE",), unaligned=unaligned)
     assert_same_run(a, b)
     assert a["iterations"] == ref["iterations"] > 3
     assert np.array_equal(a["trace"], ref["trace"]) and np.array_equal(a["labels"], ref["labels"])
