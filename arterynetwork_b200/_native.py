@@ -108,6 +108,8 @@ _SIGS = {
     "vrg_get_band_sums": [vp, vp, vp, vp, i64, ctypes.POINTER(i64)],
     "vrg_edt": [ctypes.c_int, vp, vp, vp],
     "vrg_edt_device": [ctypes.c_int, vp, vp, vp, vp],
+    "vrg_edt_ft": [ctypes.c_int, vp, vp, vp, vp, vp],
+    "vrg_edt_ft_device": [ctypes.c_int, vp, vp, vp, vp, vp, vp],
     "vrg_release_scratch": [ctypes.c_int],
     "vrg_label_components": [ctypes.c_int, vp, vp, vp, ctypes.POINTER(i64), vp, i64],
     "vrg_label_components_device": [ctypes.c_int, vp, vp, vp, ctypes.POINTER(i64), vp, i64, vp],

@@ -18,6 +18,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 
 void vrg_set_error_internal(const char *msg);  // vrg_b200.cu: text behind vrg_last_error()
 
@@ -370,6 +371,298 @@ int bad_args(const char *what) {
     return VRG_ERR_ARG;
 }
 
+// ---- Feature transform: scipy.ndimage.distance_transform_edt(mask, sampling=..., return_indices=...) ----
+// SciPy computes the feature transform (the nearest zero voxel of every voxel) with Maurer's algorithm, one line at a
+// time, axis 0 (z) first, then y, then x, and the distances afterwards from the features in NumPy.  Which of two equally
+// near zero voxels a voxel gets is decided by the order of the passes, by the tie rule of the query (the earlier site
+// keeps a tie) and, with sampling, by the rounding of every fp64 step.  The passes below therefore restate SciPy's loop
+// decision for decision: a site is a voxel that has a feature, the build pops with SciPy's test, the query walks the
+// stack with SciPy's comparison, and every fp64 operation is a separately rounded __dmul_rn / __dadd_rn / __dsub_rn in
+// SciPy's order of evaluation (nvcc would contract a*b - c into an FMA and change decisions).  Unit spacing is spacing
+// 1.0: multiplying by 1.0 is exact, so the decisions are those of SciPy's path without sampling.
+// Features travel packed: after pass z a voxel's feature differs from the voxel only in z (uint16), after pass y only in
+// z and y (uint32, z | y << 16).  FT_NONE in the z field: no feature yet (a line without a zero voxel so far).
+constexpr uint32_t FT_NONE = 0xFFFFu;
+
+__device__ __forceinline__ double ft_t(int f, int c, double s) { return __dmul_rn((double)(f - c), s); }  // SciPy's t, sampled
+__device__ __forceinline__ double ft_sq(double t) { return __dmul_rn(t, t); }
+
+// SciPy's pop test for the two top sites u, v of the stack and the new site w along the pass axis (positions pu, pv, pw;
+// uR, vR, wR = their squared distances over the other axes): c*vR - b*uR - a*wR - a*b*c > 0, left to right
+__device__ __forceinline__ bool ft_pop(int pu, int pv, int pw, double uR, double vR, double wR, double s) {
+    const double a = ft_t(pv, pu, s), b = ft_t(pw, pv, s), c = __dadd_rn(a, b);
+    const double e = __dsub_rn(__dsub_rn(__dsub_rn(__dmul_rn(c, vR), __dmul_rn(b, uR)), __dmul_rn(a, wR)), __dmul_rn(__dmul_rn(a, b), c));
+    return !(e <= 0.0);
+}
+
+// pass z: the sites of a line are its zero voxels.  With no other axis yet uR = vR = wR = 0, SciPy's test reads
+// -a*b*c <= 0 and never pops, so the stack is every zero voxel of the line in order; the query walks it with SciPy's
+// comparison (advance while strictly nearer), finding the next site by scanning the mask ahead.  One thread per (y, x)
+// line, neighbouring lanes on neighbouring x.
+__global__ void __launch_bounds__(256) k_ft_z(const uint8_t *__restrict__ mask, uint16_t *__restrict__ fz, long long nlines, int Z,
+                                              double s0) {
+    for (long long line = (long long)blockIdx.x * blockDim.x + threadIdx.x; line < nlines; line += (long long)gridDim.x * blockDim.x) {
+        const uint8_t *m = mask + line;
+        uint16_t *o = fz + line;
+        int cur = 0;
+        while (cur < Z && m[(long long)cur * nlines] != 0) ++cur;
+        if (cur == Z) {
+            for (int i = 0; i < Z; ++i) o[(long long)i * nlines] = (uint16_t)FT_NONE;
+            continue;
+        }
+        int nxt = cur + 1;
+        while (nxt < Z && m[(long long)nxt * nlines] != 0) ++nxt;
+        for (int i = 0; i < Z; ++i) {
+            double d1 = ft_sq(ft_t(cur, i, s0));
+            while (nxt < Z) {
+                const double d2 = ft_sq(ft_t(nxt, i, s0));
+                if (d1 <= d2) break;
+                d1 = d2;
+                cur = nxt++;
+                while (nxt < Z && m[(long long)nxt * nlines] != 0) ++nxt;
+            }
+            o[(long long)i * nlines] = (uint16_t)cur;
+        }
+    }
+}
+
+// pass y: one thread per (z, x) line, lanes on neighbouring x.  A site carries (its feature's z, y).  The stack lives in
+// scratch laid out like the volume (entry q of line (z, x) at (z, q, x): lanes at the same depth touch one row segment);
+// the two top entries and their squared z-distances stay in registers.  Inputs are fetched eight steps ahead, stack
+// entries of the query four at a time.
+__global__ void __launch_bounds__(128) k_ft_y(const uint16_t *__restrict__ fz, uint32_t *__restrict__ fy, uint32_t *__restrict__ stack,
+                                              int Z, int Y, int X, double s0, double s1) {
+    const long long nlines = (long long)Z * X;
+    for (long long line = (long long)blockIdx.x * blockDim.x + threadIdx.x; line < nlines; line += (long long)gridDim.x * blockDim.x) {
+        const int z = (int)(line / X), x = (int)(line % X);
+        const long long base = (long long)z * Y * X + x;
+        const uint16_t *in = fz + base;
+        uint32_t *st = stack + base, *out = fy + base;
+        int q = -1;  // depth - 1
+        int uy = 0, uz = 0, vy = 0, vz = 0;
+        double uR = 0.0, vR = 0.0;
+        constexpr int PF = 8;
+        for (int i0 = 0; i0 < Y; i0 += PF) {
+            uint16_t pre[PF];
+#pragma unroll
+            for (int k = 0; k < PF; ++k) pre[k] = i0 + k < Y ? in[(long long)(i0 + k) * X] : (uint16_t)FT_NONE;
+#pragma unroll
+            for (int k = 0; k < PF; ++k) {
+                const int f0 = pre[k], i = i0 + k;
+                if (f0 == (int)FT_NONE) continue;  // also every step beyond the line's end
+                const double wR = ft_sq(ft_t(f0, z, s0));
+                while (q >= 1 && ft_pop(uy, vy, i, uR, vR, wR, s1)) {
+                    --q;
+                    vy = uy; vz = uz; vR = uR;
+                    if (q >= 1) {
+                        const uint32_t e = st[(long long)(q - 1) * X];
+                        uy = (int)(e & 0xFFFFu); uz = (int)(e >> 16); uR = ft_sq(ft_t(uz, z, s0));
+                    }
+                }
+                ++q;
+                st[(long long)q * X] = (uint32_t)i | ((uint32_t)f0 << 16);
+                uy = vy; uz = vz; uR = vR;
+                vy = i; vz = f0; vR = wR;
+            }
+        }
+        if (q < 0) {  // no site on this line: SciPy leaves it without features
+            for (int i = 0; i < Y; ++i) out[(long long)i * X] = FT_NONE;
+            continue;
+        }
+        const int maxl = q;
+        constexpr int PB = 4;
+        uint32_t pe[PB];  // entries l+1 .. l+have
+        int have = 0, l = 0;
+        int cy = (int)(st[0] & 0xFFFFu), cz = (int)(st[0] >> 16);
+        double cR = ft_sq(ft_t(cz, z, s0));
+        for (int i = 0; i < Y; ++i) {
+            double d1 = __dadd_rn(cR, ft_sq(ft_t(cy, i, s1)));
+            while (l < maxl) {
+                if (have == 0) {
+#pragma unroll
+                    for (int j = 0; j < PB; ++j) pe[j] = st[(long long)min(l + 1 + j, maxl) * X];
+                    have = min(PB, maxl - l);
+                }
+                const int ny = (int)(pe[0] & 0xFFFFu), nz = (int)(pe[0] >> 16);
+                const double nR = ft_sq(ft_t(nz, z, s0));
+                const double d2 = __dadd_rn(nR, ft_sq(ft_t(ny, i, s1)));
+                if (d1 <= d2) break;
+                d1 = d2; ++l; --have;
+                cy = ny; cz = nz; cR = nR;
+#pragma unroll
+                for (int j = 0; j + 1 < PB; ++j) pe[j] = pe[j + 1];
+            }
+            out[(long long)i * X] = (uint32_t)cz | ((uint32_t)cy << 16);
+        }
+    }
+}
+
+// pass x, the last pass: the lines are the contiguous rows.  One warp owns 32 consecutive rows, one lane per row; the
+// rows pass through shared memory in tiles of 32 x 32 voxels, so every global access is a coalesced row segment while
+// each lane walks its own row.  Build: tiles of pass-y features in, pushes onto the lane's stack (scratch, entry q of
+// lane at [q][lane] of the warp's region: x | z << 16 | y << 32).  Query: features of a tile out to shared memory, then
+// written row by row as SciPy's outputs: int32 indices[3][Z][Y][X] when `idx` is set, and when `dist` is set the float64
+// distance in NumPy's order, sqrt(((dz*s0)^2 + (dy*s1)^2) + (dx*s2)^2).  A row without any site means the mask has no
+// zero voxel: *flag is raised.
+constexpr int FT_WARPS = 4;
+__global__ void __launch_bounds__(32 * FT_WARPS) k_ft_x(const uint32_t *__restrict__ fy, unsigned long long *__restrict__ stack,
+                                                        int32_t *__restrict__ idx, double *__restrict__ dist, long long nrows, int Y,
+                                                        int X, double s0, double s1, double s2, int *flag) {
+    __shared__ unsigned long long tile[FT_WARPS][32 * 33];  // +1 column: lane r at row r of the tile hits its own bank
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    unsigned long long *to = tile[wib];
+    uint32_t *ti = (uint32_t *)to;
+    const long long n = nrows * X, nw = (nrows + 31) / 32;
+    for (long long w = (long long)blockIdx.x * FT_WARPS + wib; w < nw; w += (long long)gridDim.x * FT_WARPS) {
+        const long long r0 = w * 32, row = r0 + lane;
+        const bool active = row < nrows;
+        const int z = active ? (int)(row / Y) : 0, y = active ? (int)(row % Y) : 0;
+        const int nr = (int)min(32LL, nrows - r0);
+        unsigned long long *st = stack + r0 * X + lane;
+        int q = -1;
+        int ux = 0, vx = 0;
+        double uR = 0.0, vR = 0.0;
+        for (int c0 = 0; c0 < X; c0 += 32) {
+            const int nc = min(32, X - c0);
+            __syncwarp();
+            if (lane < nc)
+                for (int r = 0; r < nr; ++r) ti[r * 33 + lane] = fy[(r0 + r) * X + c0 + lane];
+            __syncwarp();
+            if (!active) continue;
+            for (int k = 0; k < nc; ++k) {
+                const uint32_t f = ti[lane * 33 + k];
+                const int f0 = (int)(f & 0xFFFFu), f1 = (int)(f >> 16), i = c0 + k;
+                if (f0 == (int)FT_NONE) continue;
+                const double wR = __dadd_rn(ft_sq(ft_t(f0, z, s0)), ft_sq(ft_t(f1, y, s1)));
+                while (q >= 1 && ft_pop(ux, vx, i, uR, vR, wR, s2)) {
+                    --q;
+                    vx = ux; vR = uR;
+                    if (q >= 1) {
+                        const unsigned long long e = st[(long long)(q - 1) * 32];
+                        ux = (int)(e & 0xFFFFu);
+                        uR = __dadd_rn(ft_sq(ft_t((int)((e >> 16) & 0xFFFFu), z, s0)), ft_sq(ft_t((int)(e >> 32), y, s1)));
+                    }
+                }
+                ++q;
+                st[(long long)q * 32] = (unsigned long long)i | ((unsigned long long)f0 << 16) | ((unsigned long long)f1 << 32);
+                ux = vx; uR = vR;
+                vx = i; vR = wR;
+            }
+        }
+        const unsigned rows_ok = __ballot_sync(FULLMASK, active && q >= 0);
+        if (active && q < 0) *flag = 1;
+        const int maxl = q;
+        constexpr int PB = 4;
+        unsigned long long pe[PB], cur = 0ull;
+        int have = 0, l = 0;
+        double cR = 0.0;
+        if (maxl >= 0) {
+            cur = st[0];
+            cR = __dadd_rn(ft_sq(ft_t((int)((cur >> 16) & 0xFFFFu), z, s0)), ft_sq(ft_t((int)(cur >> 32), y, s1)));
+        }
+        for (int c0 = 0; c0 < X; c0 += 32) {
+            const int nc = min(32, X - c0);
+            __syncwarp();
+            if (maxl >= 0) {
+                for (int k = 0; k < nc; ++k) {
+                    const int i = c0 + k;
+                    double d1 = __dadd_rn(cR, ft_sq(ft_t((int)(cur & 0xFFFFu), i, s2)));
+                    while (l < maxl) {
+                        if (have == 0) {
+#pragma unroll
+                            for (int j = 0; j < PB; ++j) pe[j] = st[(long long)min(l + 1 + j, maxl) * 32];
+                            have = min(PB, maxl - l);
+                        }
+                        const double nR = __dadd_rn(ft_sq(ft_t((int)((pe[0] >> 16) & 0xFFFFu), z, s0)), ft_sq(ft_t((int)(pe[0] >> 32), y, s1)));
+                        const double d2 = __dadd_rn(nR, ft_sq(ft_t((int)(pe[0] & 0xFFFFu), i, s2)));
+                        if (d1 <= d2) break;
+                        d1 = d2; ++l; --have;
+                        cur = pe[0]; cR = nR;
+#pragma unroll
+                        for (int j = 0; j + 1 < PB; ++j) pe[j] = pe[j + 1];
+                    }
+                    to[lane * 33 + k] = cur;
+                }
+            }
+            __syncwarp();
+            if (lane >= nc) continue;
+            const int x = c0 + lane;
+            for (int r = 0; r < nr; ++r) {
+                if (!((rows_ok >> r) & 1u)) continue;
+                const unsigned long long e = to[r * 33 + lane];
+                const int fx = (int)(e & 0xFFFFu), fzv = (int)((e >> 16) & 0xFFFFu), fyv = (int)(e >> 32);
+                const long long p = (r0 + r) * X + x;
+                if (idx) { idx[p] = fzv; idx[n + p] = fyv; idx[2 * n + p] = fx; }
+                if (dist) {
+                    const long long rr = r0 + r;
+                    const double tz = ft_t(fzv, (int)(rr / Y), s0), ty = ft_t(fyv, (int)(rr % Y), s1), tx = ft_t(fx, x, s2);
+                    dist[p] = __dsqrt_rn(__dadd_rn(__dadd_rn(ft_sq(tz), ft_sq(ty)), ft_sq(tx)));
+                }
+            }
+        }
+    }
+}
+
+// The three feature-transform passes.  Scratch: uint16 pass-z features, uint32 pass-y features, 8-byte stack slots
+// (shared by the y and x passes): 14 bytes per voxel.  *flag raised when the mask has no zero voxel.  Asynchronous.
+int ft_passes(const uint8_t *d_mask, const int64_t *shape, const double *s, double *dist, int32_t *idx, int *flag, cudaStream_t stream) {
+    const long long Z = shape[0], Y = shape[1], X = shape[2], n = Z * Y * X, nrows = Z * Y;
+    Buf fz, fy, st;
+    cudaError_t e = fz.alloc(n * sizeof(uint16_t), stream);
+    if (e == cudaSuccess) e = fy.alloc(n * sizeof(uint32_t), stream);
+    if (e == cudaSuccess) e = st.alloc((size_t)((nrows + 31) / 32) * 32 * X * sizeof(unsigned long long), stream);
+    if (e == cudaSuccess) {
+        const int gz = (int)std::min<long long>((Y * X + 255) / 256, 148 * 16);
+        const int gy = (int)std::min<long long>((Z * X + 127) / 128, 148 * 16);
+        const int gx = (int)std::min<long long>(((nrows + 31) / 32 + FT_WARPS - 1) / FT_WARPS, 148 * 16);
+        k_ft_z<<<gz, 256, 0, stream>>>(d_mask, fz.as<uint16_t>(), Y * X, (int)Z, s[0]);
+        k_ft_y<<<gy, 128, 0, stream>>>(fz.as<uint16_t>(), fy.as<uint32_t>(), st.as<uint32_t>(), (int)Z, (int)Y, (int)X, s[0], s[1]);
+        k_ft_x<<<gx, 32 * FT_WARPS, 0, stream>>>(fy.as<uint32_t>(), st.as<unsigned long long>(), idx, dist, nrows, (int)Y, (int)X,
+                                                 s[0], s[1], s[2], flag);
+        e = cudaGetLastError();
+    }
+    if (e != cudaSuccess) {
+        vrg_set_error_internal(cudaGetErrorString(e));
+        return e == cudaErrorMemoryAllocation ? VRG_ERR_NOMEM : VRG_ERR_CUDA;
+    }
+    return VRG_OK;
+}
+
+int ft_device(const uint8_t *d_mask, const int64_t *shape, const double *s, double *dist, int32_t *idx, cudaStream_t stream) {
+    Buf flag;
+    cudaError_t e = flag.alloc(sizeof(int), stream);
+    int rc = VRG_OK;
+    if (e == cudaSuccess) e = cudaMemsetAsync(flag.p, 0, sizeof(int), stream);
+    if (e == cudaSuccess) {
+        rc = ft_passes(d_mask, shape, s, dist, idx, flag.as<int>(), stream);
+        if (rc == VRG_OK) {
+            int h_flag = 0;
+            e = cudaMemcpyAsync(&h_flag, flag.p, sizeof(int), cudaMemcpyDeviceToHost, stream);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+            if (e == cudaSuccess && h_flag) {
+                vrg_set_error_internal("distance transform: the mask has no zero voxel");
+                rc = VRG_ERR_ARG;
+            }
+        }
+    }
+    if (e != cudaSuccess) {
+        vrg_set_error_internal(cudaGetErrorString(e));
+        rc = e == cudaErrorMemoryAllocation ? VRG_ERR_NOMEM : VRG_ERR_CUDA;
+    }
+    return rc;
+}
+
+// checks the arguments of both feature-transform entry points and fills s with the spacings (1.0 without sampling)
+int ft_check(const uint8_t *mask, const int64_t *shape, const double *sampling, const double *dist, const int32_t *idx, double *s) {
+    if (!mask || edt_check(shape) != VRG_OK) return bad_args("feature transform: null mask or bad shape (axes 1..16384)");
+    if (!dist && !idx) return bad_args("feature transform: at least one of dist / indices must be requested");
+    for (int d = 0; d < 3; ++d) {
+        s[d] = sampling ? sampling[d] : 1.0;
+        if (!(s[d] > 0.0) || !std::isfinite(s[d])) return bad_args("feature transform: sampling must be positive and finite");
+    }
+    return VRG_OK;
+}
+
 }  // namespace
 
 // shared with vrg_mask.cu: the x pass alone -- uint16 distance to the nearest zero voxel of the same row at every FOREGROUND
@@ -408,6 +701,43 @@ extern "C" int vrg_edt(int device, const uint8_t *mask_host, const int64_t *shap
     if (e == cudaSuccess) {
         rc = edt_device(d_mask.as<uint8_t>(), shape, d_out.as<double>(), nullptr);
         if (rc == VRG_OK) e = cudaMemcpy(dist_host, d_out.p, n * sizeof(double), cudaMemcpyDeviceToHost);
+    }
+    if (e != cudaSuccess) {
+        vrg_set_error_internal(cudaGetErrorString(e));
+        rc = e == cudaErrorMemoryAllocation ? VRG_ERR_NOMEM : VRG_ERR_CUDA;
+    }
+    return rc;
+}
+
+// mask / dist / indices live on the device; sampling (3 doubles or NULL) on the host
+extern "C" int vrg_edt_ft_device(int device, const uint8_t *mask_dev, const int64_t *shape, const double *sampling, double *dist_dev,
+                                 int32_t *indices_dev, void *cuda_stream) {
+    double s[3];
+    const int rc = ft_check(mask_dev, shape, sampling, dist_dev, indices_dev, s);
+    if (rc != VRG_OK) return rc;
+    if (cudaSetDevice(device) != cudaSuccess) return VRG_ERR_CUDA;
+    vrg_scratch::pool_setup(device);
+    return ft_device(mask_dev, shape, s, dist_dev, indices_dev, (cudaStream_t)cuda_stream);
+}
+
+// host buffers: mask uint8 (Z, Y, X), dist float64 (Z, Y, X), indices int32 (3, Z, Y, X), all C order
+extern "C" int vrg_edt_ft(int device, const uint8_t *mask_host, const int64_t *shape, const double *sampling, double *dist_host,
+                          int32_t *indices_host) {
+    double s[3];
+    int rc = ft_check(mask_host, shape, sampling, dist_host, indices_host, s);
+    if (rc != VRG_OK) return rc;
+    if (cudaSetDevice(device) != cudaSuccess) return VRG_ERR_CUDA;
+    vrg_scratch::pool_setup(device);
+    const size_t n = (size_t)shape[0] * shape[1] * shape[2];
+    Buf d_mask, d_dist, d_idx;
+    cudaError_t e = d_mask.alloc(n, nullptr);
+    if (e == cudaSuccess && dist_host) e = d_dist.alloc(n * sizeof(double), nullptr);
+    if (e == cudaSuccess && indices_host) e = d_idx.alloc(3 * n * sizeof(int32_t), nullptr);
+    if (e == cudaSuccess) e = cudaMemcpy(d_mask.p, mask_host, n, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) {
+        rc = ft_device(d_mask.as<uint8_t>(), shape, s, d_dist.as<double>(), d_idx.as<int32_t>(), nullptr);
+        if (rc == VRG_OK && dist_host) e = cudaMemcpy(dist_host, d_dist.p, n * sizeof(double), cudaMemcpyDeviceToHost);
+        if (rc == VRG_OK && e == cudaSuccess && indices_host) e = cudaMemcpy(indices_host, d_idx.p, 3 * n * sizeof(int32_t), cudaMemcpyDeviceToHost);
     }
     if (e != cudaSuccess) {
         vrg_set_error_internal(cudaGetErrorString(e));

@@ -3,8 +3,8 @@ distance transform ``Code/manualCorrectionGUI.py:248`` runs on the VRG output --
 
 Same names, arguments and return conventions as the reference where it has a function (``labelVolume``,
 ``maskVolume``); the threshold / component-filter rule that the reference writes inline in ``main()`` (GVV:183-200) is
-``vesselnessToVesselMask``; ``distance_transform_edt`` stands in for the SciPy call of the same name with default
-arguments.  NIfTI I/O (``loadVolume`` / ``saveVolume``) is out of scope: nibabel is the reference's storage layer.
+``vesselnessToVesselMask``; ``distance_transform_edt`` stands in for the SciPy call of the same name, with SciPy's
+signature (``sampling``, ``return_indices``, in-place outputs) for 3-D volumes.  NIfTI I/O (``loadVolume`` / ``saveVolume``) is out of scope: nibabel is the reference's storage layer.
 
 Everything runs through the C-ABI of ``include/vrg_b200.h`` on the GPU; there is no CPU fallback.  NumPy arrays are
 copied to the device and back; CUDA tensors stay where they are (``*_device`` entry points, on the tensor's device and
@@ -65,10 +65,20 @@ def _stream(torch, t):
     return ctypes.c_void_p(torch.cuda.current_stream(t.device).cuda_stream or None)
 
 
-def distance_transform_edt(input, device: int = 0):
-    """``scipy.ndimage.distance_transform_edt(input)`` with default arguments (GVV:183, manualCorrectionGUI.py:248):
-    float64 Euclidean distance of every non-zero voxel to the nearest zero voxel.  A CUDA tensor in, a CUDA tensor out (on
-    its device; ``device`` is then not used)."""
+def distance_transform_edt(input, sampling=None, return_distances=True, return_indices=False, distances=None, indices=None,
+                           device: int = 0):
+    """``scipy.ndimage.distance_transform_edt`` (GVV:183, manualCorrectionGUI.py:248) for 3-D volumes: float64 Euclidean
+    distance of every non-zero voxel to the nearest zero voxel and, with ``return_indices``, the feature transform: int32
+    ``(3, Z, Y, X)`` coordinates of that zero voxel.
+
+    Arguments, return values (``dt``, ``ft``, a tuple of both, or ``None`` when every requested output was written in
+    place into ``distances`` / ``indices``) and argument errors are SciPy's, and so is every output value, ties between
+    equally near zero voxels and the rounding of anisotropic ``sampling`` (a scalar or one spacing per axis, positive and
+    finite) included.  A CUDA tensor in gives CUDA tensors out (on its device and torch's current stream; ``device`` is
+    then not used), and ``distances`` / ``indices`` may then be CUDA tensors on that device.  The call with default
+    arguments runs the plain distance transform; any other runs SciPy's feature transform on the caller's axes."""
+    if sampling is not None or not return_distances or return_indices or distances is not None or indices is not None:
+        return _edt_ft(input, sampling, return_distances, return_indices, distances, indices, device)
     torch = _cuda_torch(input)
     if torch is not None:
         m, transposed = _tensor_view(torch, input != 0, torch.uint8)
@@ -83,6 +93,100 @@ def distance_transform_edt(input, device: int = 0):
     shp = _shape3(m)  # kept alive across the call
     nat.check(nat.load().vrg_edt(device, m.ctypes.data, ctypes.addressof(shp), out.ctypes.data))
     return out.T if transposed else out
+
+
+def _sampling3(sampling):
+    """SciPy's normalisation of ``sampling`` (a scalar for every axis, or one value per axis) as 3 C doubles, or None."""
+    if sampling is None:
+        return None
+    if not isinstance(sampling, str) and np.iterable(sampling):
+        s = list(sampling)
+        if len(s) != 3:
+            raise RuntimeError("sequence argument must have length equal to input rank")
+    else:
+        s = [sampling] * 3
+    s = np.asarray(s, dtype=np.float64)
+    if not (np.isfinite(s).all() and (s > 0).all()):
+        raise ValueError("distance_transform_edt: sampling must be positive and finite, got %r" % (s.tolist(),))
+    return (ctypes.c_double * 3)(*s)
+
+
+def _edt_ft(input, sampling, return_distances, return_indices, distances, indices, device):
+    """distance_transform_edt through SciPy's feature transform (``vrg_edt_ft`` / ``vrg_edt_ft_device``).  The input is
+    taken in C order on the caller's axes: a transposed view would run the passes in the other order and break ties
+    differently from SciPy."""
+    torch = _cuda_torch(input)
+    out_type = torch.Tensor if torch is not None else np.ndarray  # SciPy writes in place into arrays only
+    dt_inplace, ft_inplace = isinstance(distances, out_type), isinstance(indices, out_type)
+    errors = []  # SciPy's _distance_transform_arg_check
+    if not return_distances and not return_indices:
+        errors.append("at least one of return_distances/return_indices must be True")
+    if dt_inplace and not return_distances:
+        errors.append("return_distances must be True if distances is supplied")
+    if ft_inplace and not return_indices:
+        errors.append("return_indices must be True if indices is supplied")
+    if errors:
+        raise RuntimeError(", ".join(errors))
+    if torch is not None:
+        if input.dim() != 3:
+            raise ValueError("3-D volumes only, got shape %r" % (tuple(input.shape),))
+        shape = tuple(input.shape)
+        f64, i32 = torch.float64, torch.int32
+    else:
+        input = np.asarray(input)
+        if input.ndim != 3:
+            raise ValueError("3-D volumes only, got shape %r" % (input.shape,))
+        shape = input.shape
+        f64, i32 = np.float64, np.int32
+    s = _sampling3(sampling)
+    for out, inplace, want_shape, want_dtype, name, dtname in (
+            (indices, ft_inplace, (3,) + shape, i32, "indices", "int32"),
+            (distances, dt_inplace, shape, f64, "distances", "float64")):
+        if not inplace:
+            continue
+        if tuple(out.shape) != want_shape:
+            raise RuntimeError("%s array has wrong shape" % name)
+        if out.dtype != want_dtype:
+            raise RuntimeError("%s array must be %s" % (name, dtname))
+        if torch is not None and out.device != input.device:
+            raise RuntimeError("%s must be on %s, the input's device" % (name, input.device))
+    lib = nat.load()
+    shp = (nat.i64 * 3)(*shape)  # kept alive across the call
+    m = (input != 0).to(torch.uint8).contiguous() if torch is not None else np.ascontiguousarray(input != 0, dtype=np.uint8)
+
+    def target(out, inplace, sh, dtype):
+        """where the kernel writes an output: the caller's array when it is C-contiguous, else a new one (copied over)"""
+        if torch is not None:
+            return out if inplace and out.is_contiguous() else torch.empty(sh, dtype=dtype, device=m.device)
+        return out if inplace and out.flags.c_contiguous and out.flags.writeable else np.empty(sh, dtype=dtype)
+
+    dt = target(distances, dt_inplace, shape, f64) if return_distances else None
+    ft = target(indices, ft_inplace, (3,) + shape, i32) if return_indices else None
+    sp = None if s is None else ctypes.addressof(s)
+    if torch is not None:
+        with torch.cuda.device(m.device):
+            nat.check(lib.vrg_edt_ft_device(m.device.index, m.data_ptr(), ctypes.addressof(shp), sp,
+                                            None if dt is None else dt.data_ptr(), None if ft is None else ft.data_ptr(),
+                                            _stream(torch, m)))
+    else:
+        nat.check(lib.vrg_edt_ft(device, m.ctypes.data, ctypes.addressof(shp), sp,
+                                 None if dt is None else dt.ctypes.data, None if ft is None else ft.ctypes.data))
+    result = []
+    if return_distances:
+        if dt_inplace:
+            if dt is not distances:
+                distances[...] = dt
+        else:
+            result.append(dt)
+    if return_indices:
+        if ft_inplace:
+            if ft is not indices:
+                indices[...] = ft
+        else:
+            result.append(ft)
+    if len(result) == 2:
+        return tuple(result)
+    return result[0] if result else None
 
 
 def labelVolume(volume, minSize=1, maxHop=3, device: int = 0):

@@ -295,6 +295,15 @@ int vrg_phantom_device(int device, const int64_t *shape, int64_t z0, int64_t nz,
  * VRG_ERR_ARG when the mask has no zero voxel. */
 int vrg_edt(int device, const uint8_t *mask_host, const int64_t *shape, double *dist_host);
 int vrg_edt_device(int device, const uint8_t *mask_dev, const int64_t *shape, double *dist_dev, void *cuda_stream);
+/* scipy.ndimage.distance_transform_edt(mask, sampling=..., return_indices=...): SciPy's feature transform (Maurer's
+ * algorithm, axis 0 first, SciPy's tie rule and fp64 order of evaluation) and the distances SciPy derives from it.
+ * sampling: 3 positive finite voxel spacings (z, y, x) in host memory, or NULL for unit spacing.  dist: float64 (Z, Y, X)
+ * distance to the nearest zero voxel, NULL = not requested; indices: int32 (3, Z, Y, X), the coordinates of that voxel,
+ * NULL = not requested; at least one of the two.  VRG_ERR_ARG when the mask has no zero voxel. */
+int vrg_edt_ft(int device, const uint8_t *mask_host, const int64_t *shape, const double *sampling, double *dist_host,
+               int32_t *indices_host);
+int vrg_edt_ft_device(int device, const uint8_t *mask_dev, const int64_t *shape, const double *sampling, double *dist_dev,
+                      int32_t *indices_dev, void *cuda_stream);
 /* these entry points take their scratch memory from the device's stream-ordered pool and keep it cached between calls;
  * this hands it back to the driver */
 int vrg_release_scratch(int device);
