@@ -55,7 +55,7 @@ struct vrg_handle {
     int *d_front = nullptr, *d_dirty = nullptr, *d_stamp = nullptr;
     uint16_t *d_index = nullptr;
     uint32_t *d_S = nullptr, *d_E = nullptr, *d_F = nullptr, *d_C = nullptr;
-    uint32_t *d_Dc = nullptr;  // F64_DENSE: the decision bit-plane of the cached sweeps (vrg_kernels.cuh, dense_refresh)
+    uint32_t *d_Dc = nullptr;  // F64_DENSE: the decision bit-plane of the sweeps between refreshes (vrg_kernels.cuh, dense_refresh)
     double *d_levels = nullptr, *d_pin = nullptr, *d_pout = nullptr, *d_kmat = nullptr;
     uint32_t *d_dbits = nullptr;
     long long *d_lstats = nullptr, *d_gstats = nullptr, *d_ctrl = nullptr, *d_trace = nullptr;
@@ -216,7 +216,8 @@ int vrg_create(const vrg_config *cfg, vrg_handle **out) {
     p.plane_words = (long long)Y * p.WP;
     p.plane_vox = (long long)Y * X;
     p.mhH = -0.5 * cfg->H;
-    p.dirty_lists = cfg->intensity_mode == VRG_INTENSITY_F64_BAND || cfg->intensity_mode == VRG_INTENSITY_INDEX;
+    p.dirty_lists = cfg->intensity_mode == VRG_INTENSITY_F64_BAND || cfg->intensity_mode == VRG_INTENSITY_INDEX ||
+                    (cfg->intensity_mode == VRG_INTENSITY_F64_DENSE && !h->no_dcache);  // without Dc every dense sweep is a refresh
     {   // rows per work unit of the dense sweep: long units on large volumes (fewer window restarts), short ones on thin slabs
         const long long rows_per_warp = (long long)(h->nz_own + 2) * Y * (p.nseg == 2 && p.segw == 16 ? 1 : p.nseg) / ((long long)h->sms * DENSE_WARPS);
         p.dense_rows = rows_per_warp >= 96 ? 8 : 4;  // measured: profiles/README.md (r2b, r2c)
@@ -895,10 +896,10 @@ static int enqueue_sweep(vrg_handle *h, bool slim = false) {
             else k_sweep_dense<false><<<h->sms, DENSE_WARPS * 32, dsm, h->stream>>>(p);
         } else if (p.lattice) k_sweep_dense_ldg<true><<<h->grid, BLOCK, smem, h->stream>>>(p);
         else k_sweep_dense_ldg<false><<<h->grid, BLOCK, smem, h->stream>>>(p);
-        if (p.Dc != nullptr) {  // every sweep the refresh kernel above returns from at once
-            // 4 blocks of 256 threads x 56 registers per SM: one wave (8 would not all be resident: a second wave behind the
+        if (p.Dc != nullptr) {  // every sweep the refresh kernel above returns from at once: D from Dc, no shared memory
+            // 4 blocks of 256 threads x 48 registers per SM: one wave (8 would not all be resident: a second wave behind the
             // first), half the SM's threads free for the pipelined run's statistics / table kernels
-            k_sweep_dense_cached<<<h->sms * 4, BLOCK, 0, h->stream>>>(p);
+            k_sweep_band<MODE_F64_DENSE, false><<<h->sms * 4, BLOCK, 0, h->stream>>>(p);
             h->launches++;
         }
     } else {

@@ -62,7 +62,7 @@ struct Params {
     int Y, X, XW, WP, nseg, segw;    // rows, voxels/row, words/row, word pitch, warp segments per row, words per segment (<= 30)
     int nzl;                          // local planes incl. halos
     int dense_rows;                   // rows per work unit of the dense sweep (8 on large volumes, 4 on thin slabs)
-    int dirty_lists;                  // 1: the band / index sweeps' incremental pass wants the dirty-row lists (k_cancel builds them)
+    int dirty_lists;                  // 1: k_sweep_band's incremental pass wants the dirty-row lists (k_cancel builds them)
     int own_lo, own_hi;               // local plane range owned
     int valid_lo, valid_hi;           // local planes that lie inside the global volume
     uint32_t tail_mask;               // valid bits of word XW-1
@@ -386,8 +386,20 @@ __device__ __forceinline__ void store_flips_wide(const Params &p, long long widx
     }
 }
 
-// Decision + flip word of one row segment of the BAND / INDEX modes: the decision bit D is looked up only for the
-// 32-voxel words that hold a band voxel (four gathers in flight); a band voxel flips iff D != S (VRG:87).
+// The two kinds of dense sweep.  A voxel's decision bit D = dbits[level(I)] depends on the iteration only through the table, and
+// every change of the table stamps C_FULL_SWEEP, as do the start of a run and caller-chosen flips.  So a REFRESH sweep (the
+// stamp names it) evaluates D from the fp64 intensities and keeps the words in the bit-plane Dc (layout of S); every other sweep
+// of the run is k_sweep_band<MODE_F64_DENSE>: the band sweep with D read from Dc, and only for the words that hold a band voxel,
+// instead of streaming 8 B per voxel.  Both kernels are enqueued for every sweep and one of them returns at once (the choice is
+// on the device: the table is known only there, and the batches are replayed graphs).  Without Dc (VRG_NO_DCACHE) every sweep
+// is a refresh.
+__device__ __forceinline__ bool dense_refresh(const Params &p) {
+    return p.Dc == nullptr || p.ctrl[C_FULL_SWEEP] == p.ctrl[C_SWEEPS] + 1;
+}
+
+// Decision + flip word of one row segment of the band sweep: the decision bit D is looked up only for the 32-voxel words
+// that hold a band voxel -- BAND / INDEX: gathered through the level and the table (four gathers in flight); F64_DENSE: the
+// word of Dc, one load per lane.  A band voxel flips iff D != S (VRG:87).
 template <int MODE, bool LATTICE>
 __device__ __forceinline__ int band_row(const Params &p, const uint32_t *s_dbits, int zl, int y, int sg, uint32_t s,
                                         uint32_t inner, uint32_t outer, bool active, bool own, int lane) {
@@ -397,28 +409,32 @@ __device__ __forceinline__ int band_row(const Params &p, const uint32_t *s_dbits
     const uint8_t was = p.rowflag[ridx];
     if (p.E != nullptr && outer) outer &= ~p.E[widx];
     const uint32_t band = inner | outer;
-    unsigned m = __ballot_sync(FULL, band != 0u);
     uint32_t D = 0;
-    const long long rowvox = (long long)zl * p.plane_vox + (long long)y * p.X + lane;
-    while (m) {  // warp-uniform: only words that hold a band voxel, four at a time
-        int js[4], lv[4];
+    if constexpr (MODE == MODE_F64_DENSE) {
+        if (band) D = p.Dc[widx];  // F = band & (D ^ s) ignores D elsewhere (band = 0 on inactive lanes)
+    } else {
+        unsigned m = __ballot_sync(FULL, band != 0u);
+        const long long rowvox = (long long)zl * p.plane_vox + (long long)y * p.X + lane;
+        while (m) {  // warp-uniform: only words that hold a band voxel, four at a time
+            int js[4], lv[4];
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            js[k] = -1; lv[k] = -1;
-            if (m) {
-                js[k] = __ffs(m) - 1;
-                m &= m - 1;
-                const int x = (c0 + js[k]) * 32 + lane;
-                if (x < p.X) lv[k] = level_at<MODE, LATTICE>(p, rowvox + (long long)(c0 + js[k]) * 32);
+            for (int k = 0; k < 4; ++k) {
+                js[k] = -1; lv[k] = -1;
+                if (m) {
+                    js[k] = __ffs(m) - 1;
+                    m &= m - 1;
+                    const int x = (c0 + js[k]) * 32 + lane;
+                    if (x < p.X) lv[k] = level_at<MODE, LATTICE>(p, rowvox + (long long)(c0 + js[k]) * 32);
+                }
             }
-        }
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            if (js[k] < 0) break;
-            const int l = lv[k];
-            const uint32_t bit = l >= 0 ? (s_dbits[l >> 5] >> (l & 31)) & 1u : 0u;
-            const unsigned word = __ballot_sync(FULL, bit);
-            if (lane == js[k]) D = word;
+            for (int k = 0; k < 4; ++k) {
+                if (js[k] < 0) break;
+                const int l = lv[k];
+                const uint32_t bit = l >= 0 ? (s_dbits[l >> 5] >> (l & 31)) & 1u : 0u;
+                const unsigned word = __ballot_sync(FULL, bit);
+                if (lane == js[k]) D = word;
+            }
         }
     }
     const uint32_t f = band & (D ^ s);  // inner band leaves iff in < out, outer band enters iff in >= out
@@ -426,7 +442,7 @@ __device__ __forceinline__ int band_row(const Params &p, const uint32_t *s_dbits
     return own ? __popc(f) : 0;
 }
 
-// k_sweep_band: the stencil sweep of the BAND / INDEX modes.  Bands:
+// k_sweep_band: the stencil sweep of the BAND / INDEX modes, and every sweep but the refreshes of the F64_DENSE mode.  Bands:
 //   inner = S & dil26(~S in volume)      (segmented with an unsegmented in-bounds neighbour, VRG:139-142)
 //   outer = ~S & ~E & dil26(S)           (unsegmented, not excluded, with a segmented neighbour, VRG:143-145)
 // Full pass: a warp owns a strip of ROWS_PER_UNIT rows x 30 words of one plane and slides down it, over the units
@@ -435,12 +451,17 @@ __device__ __forceinline__ int band_row(const Params &p, const uint32_t *s_dbits
 // from last time only if a voxel of its 26-neighbourhood flipped, so only the rows within one row / plane /
 // segment of last sweep's front rows are re-evaluated (each claimed once through `stamp`); every other row keeps
 // its all-zero flip word.  The work is then proportional to the moving front, like the reference's narrow band.
+// F64_DENSE: the sweep behind a refresh is incremental too, so the refresh kernels leave F, the row flags and the front
+// list as the full pass would.  No shared memory: D comes from Dc, not from the table.
 template <int MODE, bool LATTICE>
 __global__ void __launch_bounds__(BLOCK) k_sweep_band(Params p) {
     if (p.ctrl[C_STATUS] != RUNNING) return;
+    if (MODE == MODE_F64_DENSE && dense_refresh(p)) return;
     extern __shared__ uint32_t s_dbits[];
-    for (int i = threadIdx.x; i < p.LW; i += BLOCK) s_dbits[i] = table_bits(p)[i];
-    __syncthreads();
+    if (MODE != MODE_F64_DENSE) {
+        for (int i = threadIdx.x; i < p.LW; i += BLOCK) s_dbits[i] = table_bits(p)[i];
+        __syncthreads();
+    }
     const int lane = threadIdx.x & 31;
     const int zlo = max(p.valid_lo, p.own_lo - 1), zhi = min(p.valid_hi, p.own_hi + 1);
     const int nyb = (p.Y + ROWS_PER_UNIT - 1) / ROWS_PER_UNIT;
@@ -502,15 +523,6 @@ __device__ __forceinline__ void tma_bulk_load(void *smem_dst, const void *gmem_s
                  : "memory");
 }
 
-// The two kinds of dense sweep.  A voxel's decision bit D = dbits[level(I)] depends on the iteration only through the table, and
-// every change of the table stamps C_FULL_SWEEP, as do the start of a run and caller-chosen flips.  So a REFRESH sweep (the
-// stamp names it) evaluates D from the fp64 intensities and keeps the words in the bit-plane Dc (layout of S); every other sweep
-// of the run is CACHED: it reads D from Dc, and only for the words that hold a band voxel, instead of streaming 8 B per voxel.
-// Both kernels are enqueued for every sweep and one of them returns at once (the choice is on the device: the table is known
-// only there, and the batches are replayed graphs).  Without Dc (VRG_NO_DCACHE) every sweep is a refresh.
-__device__ __forceinline__ bool dense_refresh(const Params &p) {
-    return p.Dc == nullptr || p.ctrl[C_FULL_SWEEP] == p.ctrl[C_SWEEPS] + 1;
-}
 // the refresh sweep's counter (vrg_result.dense_refresh_sweeps); nothing else touches the word while a sweep runs
 __device__ __forceinline__ void count_refresh(const Params &p) {
     if (blockIdx.x == 0 && threadIdx.x == 0) p.ctrl[C_REFRESHES] += 1;
@@ -697,10 +709,14 @@ __global__ void __launch_bounds__(DENSE_WARPS * 32) k_sweep_dense(Params p) { sw
 template <bool LATTICE, bool WIDE = false>
 __global__ void __maxnreg__(96) k_sweep_dense_slim(Params p) { sweep_dense_body<LATTICE, WIDE>(p); }
 
-// Fallback of the dense sweep for odd X (row segments not 16-byte aligned): plain coalesced 8-byte loads.  CACHED: the same
-// unit loop as the cached sweep, D from Dc (LATTICE and s_dbits unused).
-template <bool LATTICE, bool CACHED>
-__device__ __forceinline__ void sweep_dense_ldg_body(const Params &p, const uint32_t *s_dbits) {
+// Fallback of the dense sweep for odd X (row segments not 16-byte aligned): plain coalesced 8-byte loads.
+template <bool LATTICE>
+__global__ void __launch_bounds__(BLOCK) k_sweep_dense_ldg(Params p) {
+    if (p.ctrl[C_STATUS] != RUNNING || !dense_refresh(p)) return;
+    count_refresh(p);
+    extern __shared__ uint32_t s_dbits[];
+    for (int i = threadIdx.x; i < p.LW; i += BLOCK) s_dbits[i] = table_bits(p)[i];
+    __syncthreads();
     const int lane = threadIdx.x & 31;
     const int zlo = max(p.valid_lo, p.own_lo - 1), zhi = min(p.valid_hi, p.own_hi + 1);
     const int nyb = (p.Y + ROWS_PER_UNIT - 1) / ROWS_PER_UNIT;
@@ -710,8 +726,6 @@ __device__ __forceinline__ void sweep_dense_ldg_body(const Params &p, const uint
     Strip st;
     for (long long u = (long long)blockIdx.x * WARPS + (threadIdx.x >> 5); u < nunits; u += nwarps) {
         const Unit un = decode_unit(p, u, zlo, nyb);
-        // cached: a unit with no segmented voxel in or next to it has no band voxel, no flip and no row flag (k_sweep_band)
-        if (CACHED && !unit_near_segmented(p, un.zl, un.y0, un.sg, lane)) continue;
         const int c0 = un.sg * p.segw - 1, c = c0 + lane;
         const bool own = un.zl >= p.own_lo && un.zl < p.own_hi;
         st.begin(p, un.zl, un.y0, c, lane);
@@ -724,27 +738,23 @@ __device__ __forceinline__ void sweep_dense_ldg_body(const Params &p, const uint
             if (p.E != nullptr && outer) outer &= ~p.E[widx];
             const uint32_t band = inner | outer;
             uint32_t D = 0;
-            if (CACHED) {
-                if (band) D = p.Dc[widx];  // F = band & (D ^ s) ignores D elsewhere (band = 0 on inactive lanes)
-            } else {
-                const int xlane = (c0 + 1) * 32 + lane;
-                const double *drow = p.data + (long long)un.zl * p.plane_vox + (long long)y * p.X + xlane;
-                constexpr int U = 10;
+            const int xlane = (c0 + 1) * 32 + lane;
+            const double *drow = p.data + (long long)un.zl * p.plane_vox + (long long)y * p.X + xlane;
+            constexpr int U = 10;
 #pragma unroll
-                for (int jb = 0; jb < WORDS_PER_WARP; jb += U) {
-                    if (jb >= p.segw || c0 + 1 + jb >= p.XW) break;  // warp-uniform
-                    double v[U];
+            for (int jb = 0; jb < WORDS_PER_WARP; jb += U) {
+                if (jb >= p.segw || c0 + 1 + jb >= p.XW) break;  // warp-uniform
+                double v[U];
 #pragma unroll
-                    for (int k = 0; k < U; ++k) v[k] = (xlane + (jb + k) * 32 < p.X) ? drow[(jb + k) * 32] : p.lev0;
+                for (int k = 0; k < U; ++k) v[k] = (xlane + (jb + k) * 32 < p.X) ? drow[(jb + k) * 32] : p.lev0;
 #pragma unroll
-                    for (int k = 0; k < U; ++k) {
-                        const int l = level_of<LATTICE>(p, v[k]);
-                        const unsigned word = __ballot_sync(FULL, (s_dbits[l >> 5] >> (l & 31)) & 1u);
-                        if (lane == jb + k + 1) D = word;
-                    }
+                for (int k = 0; k < U; ++k) {
+                    const int l = level_of<LATTICE>(p, v[k]);
+                    const unsigned word = __ballot_sync(FULL, (s_dbits[l >> 5] >> (l & 31)) & 1u);
+                    if (lane == jb + k + 1) D = word;
                 }
-                if (p.Dc != nullptr && st.active) p.Dc[widx] = D;
             }
+            if (p.Dc != nullptr && st.active) p.Dc[widx] = D;
             const uint32_t f = band & (D ^ s);
             store_flips(p, widx, ridx, was, f, st.active, own, lane);
             if (own) flips += __popc(f);
@@ -752,22 +762,6 @@ __device__ __forceinline__ void sweep_dense_ldg_body(const Params &p, const uint
     }
     flips = warp_sum(flips);
     if (lane == 0 && flips) atomicAdd((unsigned long long *)&p.lstats[2 * p.L + ST_N_FLIPS], (unsigned long long)flips);
-}
-template <bool LATTICE>
-__global__ void __launch_bounds__(BLOCK) k_sweep_dense_ldg(Params p) {
-    if (p.ctrl[C_STATUS] != RUNNING || !dense_refresh(p)) return;
-    count_refresh(p);
-    extern __shared__ uint32_t s_dbits[];
-    for (int i = threadIdx.x; i < p.LW; i += BLOCK) s_dbits[i] = table_bits(p)[i];
-    __syncthreads();
-    sweep_dense_ldg_body<LATTICE, false>(p, s_dbits);
-}
-// The cached sweep, for every shape the refresh kernels serve: streams S (and E, row flags), plus the Dc words under the band.
-// Its blocks leave room on the SMs for the statistics / table kernels of the pipelined run (vrg_tail.cuh): no shared memory,
-// and the register count stays far below k_sweep_dense_slim's 96.
-__global__ void __launch_bounds__(BLOCK, 4) k_sweep_dense_cached(Params p) {
-    if (p.ctrl[C_STATUS] != RUNNING || dense_refresh(p)) return;
-    sweep_dense_ldg_body<false, true>(p, nullptr);
 }
 
 // ---------------------------------------------------------------------------------------------
